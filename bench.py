@@ -579,7 +579,25 @@ def sharded_measure(nside, lmax, steps, warmup):
     return None
 
 
+DUMP_BYTES = 60_000_000   # --dump-outputs writes at most this many bytes of data (with the .npy headers, under 64 MB)
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as dirname/<name>.npy in float64.  When together they exceed DUMP_BYTES, every array larger than its
+    share of that budget is cut to the entries at sorted positions drawn with numpy seed 0: the same positions for the same
+    arguments, so the files of two builds compare entry for entry."""
+    arrays = {k: np.asarray(v, dtype=np.float64).ravel() for k, v in arrays.items()}
+    share = DUMP_BYTES // 8 // len(arrays)
+    over = sum(a.size for a in arrays.values()) * 8 > DUMP_BYTES
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if over and a.size > share:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def main():
+    sys.dont_write_bytecode = True   # the tree may be read-only: nothing imported from it is cached there
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=3)
@@ -602,7 +620,14 @@ def main():
     ap.add_argument("--mode", default="chains", choices=["chains", "sharded"],
                     help="chains: one independent chain per GPU (weak scaling, the default and the driver's contract); "
                          "sharded: ONE chain whose SHTs are m-sharded over the GPUs (BASELINE config #4, strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned to the caller (rank 0's chain) as DIR/<name>.npy: "
+                         "alm_EE/BB (constrained realization), binned_dl_EE/BB, accept_EE/BB (Metropolis blocks, pncp), pcg_iterations")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "chains"):
+        ap.error("--dump-outputs writes the outputs of the default path (--impl b200 --mode chains)")
     global MASK_KIND
     MASK_KIND = args.mask
     if args.impl == "reference":
@@ -681,6 +706,7 @@ def main():
             b = state["binned"]
             sky, _ = cr.sample_mask(unfold(b))
             pcg_its.append(cr.last_pcg_iterations)
+            state["sky"] = sky
             if not pncp:
                 state["binned"] = cls.sample(sky)
                 return
@@ -688,7 +714,7 @@ def main():
             mixed = cr.to_mixed(sky, unfold(b))
             b, acc = cls.sample_high_l(mixed, b)
             accepts.append((sum(acc["EE"]) + sum(acc["BB"])) / max(1, len(acc["EE"]) + len(acc["BB"])))
-            state["binned"] = b
+            state["binned"], state["accept"] = b, acc
         return step
     step_device = make_step(cr, cls, state, pcg_its, accepts)
 
@@ -741,6 +767,13 @@ def main():
     clocks.start()
     pcg_its.clear()
     ms_total = timed(step_device, args.warmup, args.steps)
+    if args.dump_outputs and rank == 0:   # now: the passes below run the same sampler again
+        last = {"alm_" + p: state["sky"][p].cpu() for p in ("EE", "BB")}
+        last.update({"binned_dl_" + p: state["binned"][p].cpu() for p in ("EE", "BB")})
+        if pncp:
+            last.update({"accept_" + p: state["accept"][p] for p in ("EE", "BB")})
+        last["pcg_iterations"] = [pcg_its[-1]]
+        dump_outputs(args.dump_outputs, last)
     launches = counted["launches"]
     its_timed = pcg_its[args.warmup:]
     clocks.stop_flag = True

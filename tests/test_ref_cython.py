@@ -1,5 +1,6 @@
-"""The reference's own compiled Cython kernels (oracle/_ref, built from /root/reference/variance_expension.pyx
-by oracle/build_ref.py) against the oracle restatement (CPU) and the sm_100a kernels (GPU): index work bit-exact."""
+"""The reference's own compiled Cython kernels (oracle/_ref, built from variance_expension.pyx of a reference checkout
+by oracle/build_ref.py) against the oracle restatement (CPU) and the sm_100a kernels (GPU): index work bit-exact.
+The repository holds no reference source: without oracle/_ref these tests skip."""
 import os
 import sys
 
@@ -13,7 +14,7 @@ REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 
 
 def ref_module():
     if not os.path.isdir(REF):
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref not built (python oracle/build_ref.py <reference checkout>)")
     if REF not in sys.path:
         sys.path.insert(0, REF)
     try:
