@@ -48,31 +48,10 @@
 #else
 #define LEG_SYNTH_BOUNDS __launch_bounds__(LEG_NT)
 #endif
-#ifndef LEG_SMEMRED
-#define LEG_SMEMRED 0   // spin-2 analysis fast loop: the WHOLE sum over the 32 lanes goes through shared memory (no shuffles in the loop)
-#endif
-#if LEG_SMEMRED
-#define LEG_FOLD2 0
-#define LEG_FOLD3 0
-#endif
-#ifndef LEG_FOLD2
-#define LEG_FOLD2 1  // spin-2 analysis: lane-permuted inputs so that the warp reduce-scatter needs one select stage instead of three
-#endif
-#ifndef LEG_FOLD3
-#define LEG_FOLD3 1  // spin-2 analysis fast loop: the last three stages of the reduce-scatter are deferred, FOLD3_NB pairs of l
-#endif               // at a time, to a sum through shared memory (needs LEG_FOLD2)
-#define FOLD3_NB 8
-#ifndef LEG_SPLITACC
-#define LEG_SPLITACC 0   // spin-2 analysis fast loop: two half-length accumulation chains per value (experiment, see the loop)
-#endif
+#define FOLD3_NB 8   // spin-2 analysis fast loop: pairs of l whose last three reduce-scatter stages are summed at once in shared memory
 #define FULL 0xffffffffu
 #ifndef LEG_CHK
 #define LEG_CHK 4     // pairs of l between two looks at which ring groups of a warp have come alive (transition phase)
-#endif
-#ifdef LEG_XNOBAR      // EXPERIMENT ONLY (wrong results): tile-loop barriers of the synthesis / analysis kernels become warp barriers,
-#define TILE_SYNC() __syncwarp()   // to measure what the CTA-wide barriers cost
-#else
-#define TILE_SYNC() __syncthreads()
 #endif
 constexpr int kUnrollA = LEG_UA;
 
@@ -510,7 +489,7 @@ leg_synth_kernel(PlanDev P, const double* __restrict__ almE, const double* __res
                 sRb[cur ^ 1][u * LEG_NT + tid] = nr[u];
             }
         }
-        TILE_SYNC();
+        __syncthreads();
     }
 
     // spin 0: north = S + A, south = +-(S - A); spin 2: combine the lambda^+- sums; the south sign follows the
@@ -738,82 +717,36 @@ struct AnalIn {
 // contributions of one ring pair at one l: spin 0 -> (re, im); spin 2 -> (Y1..Y4) with
 //   Y1 = l+ k1n + s l- k1s, Y2 = l- k2n + s l+ k2s, Y3 = l+ k3n + s l- k3s, Y4 = l- k4n + s l+ k4s
 // (E.re = Y1+Y2, E.im = Y3+Y4, B.re = Y3-Y4, B.im = Y2-Y1 are formed once per (l,m) in the finish kernel)
-template <int SPIN, bool FIRST, bool INIT>
-__device__ __forceinline__ void anal_acc(double* o, const AnalIn<SPIN>& G, double pc, double mc)
-{
-    if (SPIN == 0) {
-        const double gr = FIRST ? G.q1r : G.q2r, gi = FIRST ? G.q1i : G.q2i;
-        o[0] = INIT ? gr * pc : fma(gr, pc, o[0]);
-        o[1] = INIT ? gi * pc : fma(gi, pc, o[1]);
-    } else {
-        if (INIT) { o[0] = pc * G.q1r; o[1] = mc * G.q1i; o[2] = pc * G.q2r; o[3] = mc * G.q2i; }
-        else { o[0] = fma(pc, G.q1r, o[0]); o[1] = fma(mc, G.q1i, o[1]); o[2] = fma(pc, G.q2r, o[2]); o[3] = fma(mc, G.q2i, o[3]); }
-        if (FIRST) {
-            o[0] = fma(mc, G.u1r, o[0]); o[1] = fma(pc, G.u1i, o[1]); o[2] = fma(mc, G.u2r, o[2]); o[3] = fma(pc, G.u2i, o[3]);
-        } else {
-            o[0] = fma(-mc, G.u1r, o[0]); o[1] = fma(-pc, G.u1i, o[1]); o[2] = fma(-mc, G.u2r, o[2]); o[3] = fma(-pc, G.u2i, o[3]);
-        }
-    }
-}
-
-#if LEG_FOLD2
-// Spin 2, lane-permuted form.  With X = (k1n, k2s, k3n, k4s) (multiplied by lam^+) and Y = (k1s, k2n, k3s, k4n) (by lam^-),
+// Spin 2 is accumulated in a lane-permuted form.  With X = (k1n, k2s, k3n, k4s) (multiplied by lam^+) and
+// Y = (k1s, k2n, k3s, k4n) (by lam^-),
 //   first-parity l:  Y_c = lam^+ X_c + lam^- Y_c,   other parity:  Y_c = s_c (lam^+ X_c - lam^- Y_c),  s = (+,-,+,-),
 // every slot has the same instruction pattern, so a lane may hold value c = slot ^ pi in slot `slot` for any lane constant pi
 // by permuting its X, Y once.  pi = (lane bit 4, lane bit 3) makes the first two exchange stages of the reduce-scatter
 // (which move half and a quarter of the values) select-free: every lane keeps the low slots and sends the high ones.
-// The sign s_c is applied by the lane that ends up owning the value (anal_sign).
-template <bool FIRST, bool INIT>
-__device__ __forceinline__ void anal_acc2(double* o, const AnalIn<2>& G, double pc, double mc)
+// The sign s_c is applied by the lane that ends up owning the value (flipmask in leg_anal_kernel).
+template <int SPIN, bool FIRST, bool INIT>
+__device__ __forceinline__ void anal_acc(double* o, const AnalIn<SPIN>& G, double pc, double mc)
 {
-    if (INIT) { o[0] = pc * G.q1r; o[1] = pc * G.q1i; o[2] = pc * G.q2r; o[3] = pc * G.q2i; }
-    else { o[0] = fma(pc, G.q1r, o[0]); o[1] = fma(pc, G.q1i, o[1]); o[2] = fma(pc, G.q2r, o[2]); o[3] = fma(pc, G.q2i, o[3]); }
-    if (FIRST) { o[0] = fma(mc, G.u1r, o[0]); o[1] = fma(mc, G.u1i, o[1]); o[2] = fma(mc, G.u2r, o[2]); o[3] = fma(mc, G.u2i, o[3]); }
-    else { o[0] = fma(-mc, G.u1r, o[0]); o[1] = fma(-mc, G.u1i, o[1]); o[2] = fma(-mc, G.u2r, o[2]); o[3] = fma(-mc, G.u2i, o[3]); }
+    if constexpr (SPIN == 0) {
+        const double gr = FIRST ? G.q1r : G.q2r, gi = FIRST ? G.q1i : G.q2i;
+        o[0] = INIT ? gr * pc : fma(gr, pc, o[0]);
+        o[1] = INIT ? gi * pc : fma(gi, pc, o[1]);
+    } else {
+        if (INIT) { o[0] = pc * G.q1r; o[1] = pc * G.q1i; o[2] = pc * G.q2r; o[3] = pc * G.q2i; }
+        else { o[0] = fma(pc, G.q1r, o[0]); o[1] = fma(pc, G.q1i, o[1]); o[2] = fma(pc, G.q2r, o[2]); o[3] = fma(pc, G.q2i, o[3]); }
+        if (FIRST) { o[0] = fma(mc, G.u1r, o[0]); o[1] = fma(mc, G.u1i, o[1]); o[2] = fma(mc, G.u2r, o[2]); o[3] = fma(mc, G.u2i, o[3]); }
+        else { o[0] = fma(-mc, G.u1r, o[0]); o[1] = fma(-mc, G.u1i, o[1]); o[2] = fma(-mc, G.u2r, o[2]); o[3] = fma(-mc, G.u2i, o[3]); }
+    }
 }
 
-// v[0..3]: slots of the first l, v[4..7]: of the second.  Returns the full sum of value (h, c) = (lane bit 2, pi) in every
-// lane: 9 SHFL.64, 9 DADD, one select pair.
-__device__ __forceinline__ double warp_fold2(double* v, int lane)
-{
-    v[0] += __shfl_xor_sync(FULL, v[2], 16); v[1] += __shfl_xor_sync(FULL, v[3], 16);
-    v[4] += __shfl_xor_sync(FULL, v[6], 16); v[5] += __shfl_xor_sync(FULL, v[7], 16);
-    v[0] += __shfl_xor_sync(FULL, v[1], 8);
-    v[4] += __shfl_xor_sync(FULL, v[5], 8);
-    const bool h = lane & 4;
-    const double keep = h ? v[4] : v[0], send = h ? v[0] : v[4];
-    double r = keep + __shfl_xor_sync(FULL, send, 4);
-    r += __shfl_xor_sync(FULL, r, 2);
-    r += __shfl_xor_sync(FULL, r, 1);
-    return r;
-}
-#endif
-
-// reduce-scatter of NVAL values over the warp: afterwards lane holds the full sum of value
-// index lane >> (5 - log2(NVAL)); all lanes sharing that index hold the same number.
-template <int NVAL>
+// reduce-scatter over the warp of the values of a pair of l.
+// spin 0, 4 values: afterwards lane holds the full sum of value lane >> 3.
+// spin 2, v[0..3]: slots of the first l, v[4..7]: of the second.  Returns the full sum of value (h, c) = (lane bit 2, pi) in
+// every lane: 9 SHFL.64, 9 DADD, one select pair.
+template <int SPIN>
 __device__ __forceinline__ double warp_fold(double* v, int lane)
 {
-    if (NVAL == 8) {
-        const bool h4 = lane & 16;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const double keep = h4 ? v[i + 4] : v[i], send = h4 ? v[i] : v[i + 4];
-            v[i] = keep + __shfl_xor_sync(FULL, send, 16);
-        }
-        const bool h3 = lane & 8;
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-            const double keep = h3 ? v[i + 2] : v[i], send = h3 ? v[i] : v[i + 2];
-            v[i] = keep + __shfl_xor_sync(FULL, send, 8);
-        }
-        const bool h2 = lane & 4;
-        const double keep = h2 ? v[1] : v[0], send = h2 ? v[0] : v[1];
-        double r = keep + __shfl_xor_sync(FULL, send, 4);
-        r += __shfl_xor_sync(FULL, r, 2);
-        r += __shfl_xor_sync(FULL, r, 1);
-        return r;
-    } else {  // 4 values
+    if constexpr (SPIN == 0) {
         const bool h4 = lane & 16;
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
@@ -827,27 +760,19 @@ __device__ __forceinline__ double warp_fold(double* v, int lane)
         r += __shfl_xor_sync(FULL, r, 2);
         r += __shfl_xor_sync(FULL, r, 1);
         return r;
+    } else {
+        v[0] += __shfl_xor_sync(FULL, v[2], 16); v[1] += __shfl_xor_sync(FULL, v[3], 16);
+        v[4] += __shfl_xor_sync(FULL, v[6], 16); v[5] += __shfl_xor_sync(FULL, v[7], 16);
+        v[0] += __shfl_xor_sync(FULL, v[1], 8);
+        v[4] += __shfl_xor_sync(FULL, v[5], 8);
+        const bool h = lane & 4;
+        const double keep = h ? v[4] : v[0], send = h ? v[0] : v[4];
+        double r = keep + __shfl_xor_sync(FULL, send, 4);
+        r += __shfl_xor_sync(FULL, r, 2);
+        r += __shfl_xor_sync(FULL, r, 1);
+        return r;
     }
 }
-
-template <int SPIN, bool FIRST, bool INIT>
-__device__ __forceinline__ void anal_acc_sel(double* o, const AnalIn<SPIN>& G, double pc, double mc)
-{
-#if LEG_FOLD2
-    if constexpr (SPIN == 2) { anal_acc2<FIRST, INIT>(o, G, pc, mc); return; }
-#endif
-    anal_acc<SPIN, FIRST, INIT>(o, G, pc, mc);
-}
-template <int SPIN, int NVAL>
-__device__ __forceinline__ double anal_fold_sel(double* v, int lane)
-{
-#if LEG_FOLD2
-    if constexpr (SPIN == 2) return warp_fold2(v, lane);
-#endif
-    return warp_fold<NVAL>(v, lane);
-}
-#define ANAL_ACC(FIRST, INIT, o, G, pc, mc) anal_acc_sel<SPIN, FIRST, INIT>(o, G, pc, mc)
-#define ANAL_FOLD(v, lane) anal_fold_sel<SPIN, NVAL>(v, lane)
 
 #ifndef LEG_MINB_A
 #define LEG_MINB_A 3   // 3 CTAs per SM: caps the unrolled fast loop at 168 registers
@@ -860,8 +785,7 @@ template <int SPIN, int NC>
 constexpr size_t leg_anal_smem()
 {
     return sizeof(double2) * LEG_TL + sizeof(double) * LEG_NW * NC * LEG_TL * (SPIN ? 4 : 2)
-           + ((SPIN && LEG_FOLD2 && LEG_FOLD3) ? sizeof(double2) * LEG_NW * NC * FOLD3_NB * 32 : 0)
-           + ((SPIN && LEG_SMEMRED) ? sizeof(double2) * LEG_NW * NC * (NC == 1 ? 4 : 2) * 4 * 32 : 0);
+           + (SPIN ? sizeof(double2) * LEG_NW * NC * FOLD3_NB * 32 : 0);
 }
 // NC > 1: chain batch (see leg_synth_kernel): spectra of chain c at Fm + c fm_stride, partial sums at partial + c part_stride;
 // the recurrence of a (ring pair, m) thread is shared, the reduce-scatter runs once per chain.
@@ -885,21 +809,12 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
     double2* sR = leg_dyn;                                                  // [LEG_TL]
     double* sPartAll = reinterpret_cast<double*>(leg_dyn + LEG_TL);         // [LEG_NW][NC][LEG_TL * NV]
     auto sPart = [&](int ww, int c) { return sPartAll + ((size_t)(ww * NC + c)) * (LEG_TL * NV); };
-#if LEG_FOLD2 && LEG_FOLD3
     // After the two select-free exchange stages a lane holds, for each of the two l of a pair, the sum over 4 lanes of the
     // value c = (lane bit 4, lane bit 3); what remains is a sum over the 8 lanes that differ in bits 2..0.  Instead of three
     // more dependent shuffle stages per pair of l, the fast loop parks those two numbers in shared memory and sums FOLD3_NB
     // pairs of l at a time (8 independent loads per output, no selects).  Slot of lane L for local pair q:
     // L ^ c(L) ^ ((q & 1) << 2): stores are conflict free and the 32 outputs read in one step hit 16 distinct 8-byte banks.
     double2* sFoldAll = reinterpret_cast<double2*>(sPartAll + (size_t)LEG_NW * NC * LEG_TL * NV);   // [LEG_NW][NC][FOLD3_NB * 32] (spin 2)
-#endif
-#if LEG_SMEMRED
-    // Every lane parks its 8 values of a pair of l as 4 double2 rows [pair][value pair][lane]; NBQ pairs at a time a lane sums half
-    // a row (16 lanes, rotated start: conflict free) with LDS.128, the two halves meet in one shuffle.  No shuffle, select or
-    // lane-dependent slot in the accumulation loop; fixed summation order.
-    constexpr int NBQ = NC == 1 ? 4 : 2;
-    double2* sRedAll = reinterpret_cast<double2*>(sPartAll + (size_t)LEG_NW * NC * LEG_TL * NV);   // [LEG_NW][NC][NBQ * 4 * 32] (spin 2)
-#endif
     const int l0 = m > SPIN ? m : SPIN;
     const int64_t base = (int64_t)m * (2 * L + 1 - m) / 2;
     // first entry (l = lt) of this block's partial sums is pbase + lt
@@ -945,7 +860,6 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
                     g.q1r = qn.x - un.y; g.q1i = qn.x + un.y; g.q2r = qn.y + un.x; g.q2i = qn.y - un.x;
                     g.u1r = sg * (qs.x - us.y); g.u1i = sg * (qs.x + us.y);
                     g.u2r = sg * (qs.y + us.x); g.u2i = sg * (qs.y - us.x);
-#if LEG_FOLD2
                     {   // (q1r,q1i,q2r,q2i) <- X = (k1n, k2s, k3n, k4s), (u1r,u1i,u2r,u2i) <- Y = (k1s, k2n, k3s, k4n), then slot = c ^ pi
                         double t = g.q1i; g.q1i = g.u1i; g.u1i = t;
                         t = g.q2i; g.q2i = g.u2i; g.u2i = t;
@@ -958,7 +872,6 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
                             t = g.u1r; g.u1r = g.u1i; g.u1i = t;  t = g.u2r; g.u2r = g.u2i; g.u2i = t;
                         }
                     }
-#endif
                 }
             }
         }
@@ -968,25 +881,20 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
 #pragma unroll
     for (int j = 0; j < R; ++j) if (__any_sync(FULL, (myact >> j) & 1u)) gact |= 1u << j;
     bool all_live = false;      // see leg_synth_kernel
-#if LEG_FOLD2
     // spin 2: the lane ends up owning (h, c) = (bit 2, (bit 4, bit 3)); odd c of the second l carries a minus sign
     const int vidx = SPIN ? ((lane & 4) | ((lane >> 3) & 3)) : lane >> 3;
     const int flipmask = (SPIN && (lane & 4) && (lane & 8)) ? (int)0x80000000 : 0;   // sign flip as an integer XOR (no FP64 op)
-#else
-    const int vidx = lane >> (SPIN ? 2 : 3);           // value index this lane ends up owning
-    const int flipmask = 0;
-#endif
     const bool writer = (lane & (SPIN ? 3 : 7)) == 0;
 
     for (int lt = l0; lt <= L; lt += LEG_TL) {
-        TILE_SYNC();
+        __syncthreads();
         for (int i = tid; i < LEG_TL; i += LEG_NT) {
             const int l = lt + i;
             double2 r = make_double2(0.0, 0.0);
             if (l <= L) { if (SPIN) r = P.rec2[base + l]; else r.x = P.rec0[base + l]; }
             sR[i] = r;
         }
-        TILE_SYNC();
+        __syncthreads();
         const int ni = min(LEG_TL, L - lt + 1);
         const int npr = (ni + 1) >> 1;
         int ip = 0;
@@ -1014,8 +922,13 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
                         const double pc = st[j].sc ? 0.0 : st[j].pc, mc = st[j].sc ? 0.0 : st[j].mc;
 #pragma unroll
                         for (int c = 0; c < NC; ++c) {
-                            if (h == 0) { if (j == 0) ANAL_ACC(true, true, v[c], G[j][c], pc, mc); else ANAL_ACC(true, false, v[c], G[j][c], pc, mc); }
-                            else { if (j == 0) ANAL_ACC(false, true, v[c] + NV, G[j][c], pc, mc); else ANAL_ACC(false, false, v[c] + NV, G[j][c], pc, mc); }
+                            if (h == 0) {
+                                if (j == 0) anal_acc<SPIN, true, true>(v[c], G[j][c], pc, mc);
+                                else anal_acc<SPIN, true, false>(v[c], G[j][c], pc, mc);
+                            } else {
+                                if (j == 0) anal_acc<SPIN, false, true>(v[c] + NV, G[j][c], pc, mc);
+                                else anal_acc<SPIN, false, false>(v[c] + NV, G[j][c], pc, mc);
+                            }
                         }
                         rec_step<SPIN>(st[j], r.x, r.y);
                         rescale_check<SPIN>(st[j]);
@@ -1023,7 +936,7 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
                 }
 #pragma unroll
                 for (int c = 0; c < NC; ++c) {
-                    const double s = ANAL_FOLD(v[c], lane);
+                    const double s = warp_fold<SPIN>(v[c], lane);
                     if (writer) sPart(w, c)[ip * NVAL + vidx] = __hiloint2double(__double2hiint(s) ^ flipmask, __double2loint(s));
                 }
                 ++ip;
@@ -1045,16 +958,16 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
                         if (j >= J0) {
 #pragma unroll
                             for (int c = 0; c < NC; ++c) {
-                                if (j == J0) ANAL_ACC(true, true, v[c], G[j][c], st[j].pc, st[j].mc);
-                                else ANAL_ACC(true, false, v[c], G[j][c], st[j].pc, st[j].mc);
+                                if (j == J0) anal_acc<SPIN, true, true>(v[c], G[j][c], st[j].pc, st[j].mc);
+                                else anal_acc<SPIN, true, false>(v[c], G[j][c], st[j].pc, st[j].mc);
                             }
                         }
                         rec_step<SPIN>(st[j], r0.x, r0.y);
                         if (j >= J0) {
 #pragma unroll
                             for (int c = 0; c < NC; ++c) {
-                                if (j == J0) ANAL_ACC(false, true, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
-                                else ANAL_ACC(false, false, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
+                                if (j == J0) anal_acc<SPIN, false, true>(v[c] + NV, G[j][c], st[j].pc, st[j].mc);
+                                else anal_acc<SPIN, false, false>(v[c] + NV, G[j][c], st[j].pc, st[j].mc);
                             }
                         }
                         rec_step<SPIN>(st[j], r1.x, r1.y);
@@ -1067,7 +980,7 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
                     } else {
 #pragma unroll
                         for (int c = 0; c < NC; ++c) {
-                            const double s = ANAL_FOLD(v[c], lane);
+                            const double s = warp_fold<SPIN>(v[c], lane);
                             if (writer) sPart(w, c)[ip * NVAL + vidx] = __hiloint2double(__double2hiint(s) ^ flipmask, __double2loint(s));
                         }
                     }
@@ -1078,8 +991,7 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
             else if (R >= 2 && jlo == 1) run(std::integral_constant<int, (R >= 2 ? 1 : R)>());
             else run(std::integral_constant<int, R>());
         }
-#if LEG_FOLD2 && LEG_FOLD3
-        if (SPIN == 2) {
+        if constexpr (SPIN == 2) {
             const int cperm = ((lane >> 4) & 1) << 1 | ((lane >> 3) & 1);
             int ipb = ip;   // first pair of l of the batch parked in the fold buffers
             // sums the parked pairs [ipb, ipb + n) over the 8 lanes of each value and writes them to the warp's partial sums
@@ -1110,99 +1022,36 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
             for (; ip < npr; ++ip) {  // (C)
                 double v[NC][NVAL];
                 const double2 r0 = sR[2 * ip], r1 = sR[2 * ip + 1];
-#if LEG_SPLITACC
-                // two half-length accumulation chains per value (rings j < R/2 and j >= R/2), joined by one add: the sums over
-                // the R rings of a thread are dependent DFMA chains of depth 2 R, the longest ones in the loop
-                double v2[NC][NVAL];
 #pragma unroll
                 for (int j = 0; j < R; ++j) {
 #pragma unroll
                     for (int c = 0; c < NC; ++c) {
-                        double* t = (R >= 4 && j >= R / 2) ? v2[c] : v[c];
-                        if (j == 0 || (R >= 4 && j == R / 2)) ANAL_ACC(true, true, t, G[j][c], st[j].pc, st[j].mc);
-                        else ANAL_ACC(true, false, t, G[j][c], st[j].pc, st[j].mc);
+                        if (j == 0) anal_acc<SPIN, true, true>(v[c], G[j][c], st[j].pc, st[j].mc);
+                        else anal_acc<SPIN, true, false>(v[c], G[j][c], st[j].pc, st[j].mc);
                     }
                     rec_step<SPIN>(st[j], r0.x, r0.y);
 #pragma unroll
                     for (int c = 0; c < NC; ++c) {
-                        double* t = (R >= 4 && j >= R / 2) ? v2[c] : v[c];
-                        if (j == 0 || (R >= 4 && j == R / 2)) ANAL_ACC(false, true, t + NV, G[j][c], st[j].pc, st[j].mc);
-                        else ANAL_ACC(false, false, t + NV, G[j][c], st[j].pc, st[j].mc);
+                        if (j == 0) anal_acc<SPIN, false, true>(v[c] + NV, G[j][c], st[j].pc, st[j].mc);
+                        else anal_acc<SPIN, false, false>(v[c] + NV, G[j][c], st[j].pc, st[j].mc);
                     }
                     rec_step<SPIN>(st[j], r1.x, r1.y);
                 }
-                if (R >= 4) {
-#pragma unroll
-                    for (int c = 0; c < NC; ++c)
-#pragma unroll
-                        for (int qq = 0; qq < NVAL; ++qq) v[c][qq] += v2[c][qq];
-                }
-#else
-#pragma unroll
-                for (int j = 0; j < R; ++j) {
-#pragma unroll
-                    for (int c = 0; c < NC; ++c) {
-                        if (j == 0) ANAL_ACC(true, true, v[c], G[j][c], st[j].pc, st[j].mc);
-                        else ANAL_ACC(true, false, v[c], G[j][c], st[j].pc, st[j].mc);
-                    }
-                    rec_step<SPIN>(st[j], r0.x, r0.y);
-#pragma unroll
-                    for (int c = 0; c < NC; ++c) {
-                        if (j == 0) ANAL_ACC(false, true, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
-                        else ANAL_ACC(false, false, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
-                    }
-                    rec_step<SPIN>(st[j], r1.x, r1.y);
-                }
-#endif
                 const int q = ip - ipb;
 #pragma unroll
                 for (int c = 0; c < NC; ++c) {
                     double* vv = v[c];
-#ifdef LEG_XNORED   // EXPERIMENT ONLY (wrong results): no cross-lane exchange, to measure what the in-loop reduce-scatter costs
-                    vv[0] += vv[2]; vv[1] += vv[3]; vv[4] += vv[6]; vv[5] += vv[7]; vv[0] += vv[1]; vv[4] += vv[5];
-#else
                     vv[0] += __shfl_xor_sync(FULL, vv[2], 16); vv[1] += __shfl_xor_sync(FULL, vv[3], 16);
                     vv[4] += __shfl_xor_sync(FULL, vv[6], 16); vv[5] += __shfl_xor_sync(FULL, vv[7], 16);
                     vv[0] += __shfl_xor_sync(FULL, vv[1], 8);
                     vv[4] += __shfl_xor_sync(FULL, vv[5], 8);
-#endif
                     double2* fbuf = sFoldAll + ((size_t)(w * NC + c)) * (FOLD3_NB * 32);
                     fbuf[q * 32 + (lane ^ cperm ^ ((q & 1) << 2))] = make_double2(vv[0], vv[4]);
                 }
                 if (q == FOLD3_NB - 1) { flush(FOLD3_NB); ipb = ip + 1; }
             }
             if (ip > ipb) flush(ip - ipb);
-        } else
-#endif
-#if LEG_SMEMRED
-        if (SPIN == 2) {
-            int ipb = ip;
-            auto flush = [&](int n) {
-                __syncwarp();
-                const int row = lane & 15, half = lane >> 4;
-#pragma unroll
-                for (int c = 0; c < NC; ++c) {
-                    const double2* rb = sRedAll + ((size_t)(w * NC + c)) * (NBQ * 4 * 32) + row * 32;
-                    double sx = 0.0, sy = 0.0;
-                    if (row < 4 * n) {
-                        double2 a[16];
-#pragma unroll
-                        for (int k = 0; k < 16; ++k) a[k] = rb[(half * 16 + k + row) & 31];
-#pragma unroll
-                        for (int st2 = 8; st2 >= 1; st2 >>= 1)
-#pragma unroll
-                            for (int k = 0; k < st2; ++k) { a[k].x += a[k + st2].x; a[k].y += a[k + st2].y; }
-                        sx = a[0].x; sy = a[0].y;
-                    }
-                    sx += __shfl_xor_sync(FULL, sx, 16);
-                    sy += __shfl_xor_sync(FULL, sy, 16);
-                    if (half == 0 && row < 4 * n) {
-                        double* o = sPart(w, c) + (ipb + (row >> 2)) * NVAL + 2 * (row & 3);
-                        o[0] = sx; o[1] = sy;
-                    }
-                }
-                __syncwarp();
-            };
+        } else {
 #pragma unroll kUnrollA
             for (; ip < npr; ++ip) {  // (C)
                 double v[NC][NVAL];
@@ -1211,57 +1060,25 @@ leg_anal_kernel(PlanDev P, const double2* __restrict__ Fm, double* __restrict__ 
                 for (int j = 0; j < R; ++j) {
 #pragma unroll
                     for (int c = 0; c < NC; ++c) {
-                        if (j == 0) ANAL_ACC(true, true, v[c], G[j][c], st[j].pc, st[j].mc);
-                        else ANAL_ACC(true, false, v[c], G[j][c], st[j].pc, st[j].mc);
+                        if (j == 0) anal_acc<SPIN, true, true>(v[c], G[j][c], st[j].pc, st[j].mc);
+                        else anal_acc<SPIN, true, false>(v[c], G[j][c], st[j].pc, st[j].mc);
                     }
                     rec_step<SPIN>(st[j], r0.x, r0.y);
 #pragma unroll
                     for (int c = 0; c < NC; ++c) {
-                        if (j == 0) ANAL_ACC(false, true, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
-                        else ANAL_ACC(false, false, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
+                        if (j == 0) anal_acc<SPIN, false, true>(v[c] + NV, G[j][c], st[j].pc, st[j].mc);
+                        else anal_acc<SPIN, false, false>(v[c] + NV, G[j][c], st[j].pc, st[j].mc);
                     }
                     rec_step<SPIN>(st[j], r1.x, r1.y);
                 }
-                const int q = ip - ipb;
 #pragma unroll
                 for (int c = 0; c < NC; ++c) {
-                    double2* rb = sRedAll + ((size_t)(w * NC + c)) * (NBQ * 4 * 32) + q * 4 * 32 + lane;
-#pragma unroll
-                    for (int cp = 0; cp < 4; ++cp) rb[cp * 32] = make_double2(v[c][2 * cp], v[c][2 * cp + 1]);
+                    const double s = warp_fold<SPIN>(v[c], lane);
+                    if (writer) sPart(w, c)[ip * NVAL + vidx] = __hiloint2double(__double2hiint(s) ^ flipmask, __double2loint(s));
                 }
-                if (q == NBQ - 1) { flush(NBQ); ipb = ip + 1; }
-            }
-            if (ip > ipb) flush(ip - ipb);
-        } else
-#endif
-        {
-#pragma unroll kUnrollA
-        for (; ip < npr; ++ip) {  // (C)
-            double v[NC][NVAL];
-            const double2 r0 = sR[2 * ip], r1 = sR[2 * ip + 1];
-#pragma unroll
-            for (int j = 0; j < R; ++j) {
-#pragma unroll
-                for (int c = 0; c < NC; ++c) {
-                    if (j == 0) ANAL_ACC(true, true, v[c], G[j][c], st[j].pc, st[j].mc);
-                    else ANAL_ACC(true, false, v[c], G[j][c], st[j].pc, st[j].mc);
-                }
-                rec_step<SPIN>(st[j], r0.x, r0.y);
-#pragma unroll
-                for (int c = 0; c < NC; ++c) {
-                    if (j == 0) ANAL_ACC(false, true, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
-                    else ANAL_ACC(false, false, v[c] + NV, G[j][c], st[j].pc, st[j].mc);
-                }
-                rec_step<SPIN>(st[j], r1.x, r1.y);
-            }
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const double s = ANAL_FOLD(v[c], lane);
-                if (writer) sPart(w, c)[ip * NVAL + vidx] = __hiloint2double(__double2hiint(s) ^ flipmask, __double2loint(s));
             }
         }
-        }
-        TILE_SYNC();
+        __syncthreads();
         // sum over the warps of the block, one deterministic partial per chunk
 #pragma unroll
         for (int c = 0; c < NC; ++c) {

@@ -19,30 +19,7 @@
 
 #include "gs_internal.h"
 
-#ifndef RING_R8
-#define RING_R8 0   // 1: radix-8 passes, 512 threads per CTA at <= 64 registers (32 warps per SM instead of 16)
-#endif
-#ifndef RF_NT
-#define RF_NT (RING_R8 ? 512 : 256)
-#endif
-#ifndef RING_UNPACK_CHIRP
-#define RING_UNPACK_CHIRP 1   // Bluestein rings: last chirp product taken while the spectrum is unpacked (no pass of its own)
-#endif
-#ifndef RING_FUSE_MID
-#define RING_FUSE_MID 0   // Bluestein rings of ring_apply_kernel: pointwise chirp / weight product inside the next transform's first pass
-#endif
-
-#ifndef RING_SUBBAR
-#define RING_SUBBAR 0   // 1: the rings that share a CTA (groups of 2 / 4) synchronise among their own threads (named barriers)
-#endif
-// barrier among the nt threads that work on one transform (all RF_NT threads of the CTA when it holds one ring)
-__device__ __forceinline__ void ring_bar(int nt)
-{
-#if RING_SUBBAR
-    if (nt < RF_NT) { asm volatile("bar.sync %0, %1;" ::"r"(1 + (int)threadIdx.x / nt), "r"(nt) : "memory"); return; }
-#endif
-    __syncthreads();
-}
+#define RF_NT 256   // threads per CTA of the ring kernels
 
 __device__ __forceinline__ double2 cmul(double2 a, double2 b) { return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 __device__ __forceinline__ double2 cmulc(double2 a, double2 b) { return make_double2(a.x * b.x + a.y * b.y, a.y * b.x - a.x * b.y); }  // a conj(b)
@@ -60,14 +37,8 @@ __device__ __forceinline__ double2 csub(double2 a, double2 b) { return make_doub
 // radix-2 and/or radix-4 pass at the top (DIF) / bottom (DIT).
 // Twiddles: quarter table twq[k] = exp(-2 pi i k / twn), k <= twn/4, in shared memory;
 // W^(k + twn/4) = -i W^k covers the second quadrant (indices stay below twn/2).
-#if RING_R8
-// radix-8 build: one pad per 8 elements (the stride-8 accesses of the final radix-8 pass), second level as above
-#define PADI(i) ((i) + ((i) >> 3) + ((i) >> 8))
-#define PADLEN(M) ((M) + ((M) >> 3) + ((M) >> 8) + 2)
-#else
 #define PADI(i) ((i) + ((i) >> 4) + ((i) >> 8))
 #define PADLEN(M) ((M) + ((M) >> 4) + ((M) >> 8) + 2)   // shared-memory slots of a padded M-point buffer
-#endif
 
 __device__ __forceinline__ double2 tw_get(const double2* twq, int idx, int quarter)
 {
@@ -145,7 +116,7 @@ __device__ __forceinline__ void pass16(double2* buf, int M, int N, const double2
             buf[PADI(i0 + k * s)] = v;
         }
     }
-    ring_bar(nt);
+    __syncthreads();
 }
 
 // radix-4 pass over sub-transforms of size N (N >= 4)
@@ -161,16 +132,15 @@ __device__ __forceinline__ void pass4(double2* buf, int M, int N, const double2*
         if (!INV) bf4_dif(a0, a1, a2, a3, w1, w2); else bf4_dit(a0, a1, a2, a3, w1, w2);
         buf[PADI(i0)] = a0; buf[PADI(i0 + q)] = a1; buf[PADI(i0 + 2 * q)] = a2; buf[PADI(i0 + 3 * q)] = a3;
     }
-    ring_bar(nt);
+    __syncthreads();
 }
 
 // radix-8 pass over sub-transforms of size N (N >= 8) = one radix-2 level + one radix-4 level in registers.  Transform lengths
 // 2^(4k+3) (2048: the belt rings of nside 512 and the Bluestein length of the cap rings with 516..1024 pixels) used to take a
 // radix-2 AND a radix-4 trip through shared memory at the top (DIF) / bottom (DIT) of the transform; this is one trip.
 // PRE (DIF only): the loaded element idx is replaced by pre(idx, value) (fused pointwise products, see ring_apply_kernel).
-template <bool INV, class PRE = NoPre, bool POST = false>
-__device__ __forceinline__ void pass8(double2* buf, int M, int N, const double2* twq, int twn, int tid, int nt, PRE pre = PRE(),
-                                      const double2* __restrict__ post = nullptr)
+template <bool INV, class PRE = NoPre>
+__device__ __forceinline__ void pass8(double2* buf, int M, int N, const double2* twq, int twn, int tid, int nt, PRE pre = PRE())
 {
     const int s = N >> 3, ls = 31 - __clz(s), ts = twn / N, quarter = twn >> 2, ng = M >> 3;
     for (int t = tid; t < ng; t += nt) {
@@ -203,13 +173,9 @@ __device__ __forceinline__ void pass8(double2* buf, int M, int N, const double2*
             }
         }
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            double2 v = x[k];
-            if (POST) v = cmul(v, __ldg(&post[i0 + k * s]));
-            buf[PADI(i0 + k * s)] = v;
-        }
+        for (int k = 0; k < 8; ++k) buf[PADI(i0 + k * s)] = x[k];
     }
-    ring_bar(nt);
+    __syncthreads();
 }
 
 // radix-2 pass over sub-transforms of size N (N >= 2)
@@ -224,7 +190,7 @@ __device__ __forceinline__ void pass2(double2* buf, int M, int N, const double2*
         if (!INV) { buf[PADI(i0)] = cadd(a, b); buf[PADI(i0 + h)] = cmul(csub(a, b), w); }
         else { const double2 tb = cmulc(b, w); buf[PADI(i0)] = cadd(a, tb); buf[PADI(i0 + h)] = csub(a, tb); }
     }
-    ring_bar(nt);
+    __syncthreads();
 }
 
 // In-place forward DIF FFT (kernel exp(-2 pi i jk/M)), natural order in, bit-reversed order out;
@@ -237,25 +203,6 @@ template <bool POST, class PRE = NoPre>
 __device__ void fft_dif(double2* buf, int M, const double2* twq, int twn, const double2* __restrict__ post, int tid = threadIdx.x,
                         int nt = RF_NT, PRE pre = PRE())
 {
-#if RING_R8
-    {   // radix-8 passes below a radix-2 / radix-4 top pass (needs M >= 8)
-        const int lg = 31 - __clz(M), r = lg % 3;
-        int N = M;
-        bool first = true;
-        if (r == 1) { pass2<false, PRE>(buf, M, N, twq, twn, tid, nt, pre); N >>= 1; first = false; }
-        else if (r == 2) { pass4<false, PRE>(buf, M, N, twq, twn, tid, nt, pre); N >>= 2; first = false; }
-        while (N >= 8) {
-            if (first) {
-                if (POST && N == 8) pass8<false, PRE, true>(buf, M, N, twq, twn, tid, nt, pre, post);
-                else pass8<false, PRE, false>(buf, M, N, twq, twn, tid, nt, pre);
-            } else if (POST && N == 8) pass8<false, NoPre, true>(buf, M, N, twq, twn, tid, nt, NoPre(), post);
-            else pass8<false>(buf, M, N, twq, twn, tid, nt);
-            first = false;
-            N >>= 3;
-        }
-        return;
-    }
-#endif
     const int lg = 31 - __clz(M), r = lg & 3;
     int N = M;
     bool first = true;
@@ -281,16 +228,6 @@ __device__ void fft_dif(double2* buf, int M, const double2* twq, int twn, const 
 // In-place inverse DIT FFT (kernel exp(+2 pi i jk/M), unnormalised), bit-reversed in, natural out.
 __device__ void fft_dit_inv(double2* buf, int M, const double2* twq, int twn, int tid = threadIdx.x, int nt = RF_NT)
 {
-#if RING_R8
-    {
-        const int lg = 31 - __clz(M), r = lg % 3;
-        const int Ntop = M >> r;
-        for (int N = 8; N <= Ntop; N <<= 3) pass8<true>(buf, M, N, twq, twn, tid, nt);
-        if (r == 2) pass4<true>(buf, M, M, twq, twn, tid, nt);
-        else if (r == 1) pass2<true>(buf, M, M, twq, twn, tid, nt);
-        return;
-    }
-#endif
     const int lg = 31 - __clz(M), r = lg & 3;
     const int Ntop = M >> r;  // largest radix-16 sub-transform size
     for (int N = 16; N <= Ntop; N <<= 4) pass16<true, false>(buf, M, N, twq, twn, nullptr, tid, nt);
@@ -321,18 +258,10 @@ __device__ __forceinline__ double2 chirp_val(int t, int n)
 // All threads of the CTA must call; begins and ends with a barrier.
 __device__ void ring_idft(const PlanDev& P, double2* buf, const double2* twq, int n, int bsi, int tid = threadIdx.x, int nt = RF_NT)
 {
-    ring_bar(nt);
+    __syncthreads();
     if (bsi < 0) { fft_dit_inv(buf, n, twq, P.tw_n, tid, nt); return; }
     const BluesteinDesc d = P.bs[bsi];
     fft_dif<true>(buf, d.M, twq, P.tw_n, P.bs_tab + d.bhat_off, tid, nt);
-    fft_dit_inv(buf, d.M, twq, P.tw_n, tid, nt);
-}
-// Bluestein only: the input of the convolution is pre(k, buf[k]) (chirp products / zero padding applied as the first pass loads)
-template <class PRE>
-__device__ void ring_idft_bs_pre(const PlanDev& P, double2* buf, const double2* twq, int bsi, int tid, int nt, PRE pre)
-{
-    const BluesteinDesc d = P.bs[bsi];
-    fft_dif<true, PRE>(buf, d.M, twq, P.tw_n, P.bs_tab + d.bhat_off, tid, nt, pre);
     fft_dit_inv(buf, d.M, twq, P.tw_n, tid, nt);
 }
 
@@ -594,10 +523,6 @@ __device__ __forceinline__ void ring_build_Z(const PlanDev& P, const RingSub& S,
         else if (S.bsi >= 0 && !plain) v = cmul(v, __ldg(&S.chirp[k]));
         S.buf[pos] = v;
     };
-#ifndef RING_DIRECT_FOLD
-#define RING_DIRECT_FOLD 1
-#endif
-#if RING_DIRECT_FOLD
     if (!SH && 2 * mtop <= n && n > S.nt) {
         // No alias term (most cap rings, the whole belt): F_m alone gives Z_m = e^{i m phi0} (Fa + i Fb)_m and
         // Z_{n-m} = e^{-i m phi0} (conj Fa + i conj Fb)_m; the walk is over m with 2 DU independent loads in flight, every one of them
@@ -629,16 +554,12 @@ __device__ __forceinline__ void ring_build_Z(const PlanDev& P, const RingSub& S,
         }
         for (int k = mtop + 1 + S.tid; k < n - mtop; k += S.nt) put(k, zero);
         for (int k = n + S.tid; k < Mz; k += S.nt) put(k, zero);   // zero padding (Bluestein)
-        ring_bar(S.nt);
+        __syncthreads();
         return;
     }
-#endif
     const bool split = n <= S.nt;
     const double2 q = ring_phase(P, job.ringA, n);
-#ifndef RING_FK
-#define RING_FK (RING_R8 ? 2 : 4)
-#endif
-    constexpr int FK = RING_FK;   // values of k (long rings) / alias terms (short rings) per step: 4 FK loads in flight per thread
+    constexpr int FK = 4;   // values of k (long rings) / alias terms (short rings) per step: 4 FK loads in flight per thread
     if (split) {
         const int J = S.nt / n, kq = S.tid % n, jq = S.tid / n;
         double2 z[1] = {zero};
@@ -666,7 +587,7 @@ __device__ __forceinline__ void ring_build_Z(const PlanDev& P, const RingSub& S,
         }
         for (int k = S.tid + ((n - S.tid + S.nt - 1) / S.nt) * S.nt; k < Mz; k += S.nt) put(k, zero);   // zero padding
     }
-    ring_bar(S.nt);
+    __syncthreads();
     if (split) {
         const int J = S.nt / n;
         for (int k = S.tid; k < Mz; k += S.nt) {
@@ -745,7 +666,7 @@ ring_synth_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __res
         // sqrt(n) Z_k (the unitary DFT of the pixels this launch would have produced) and no transform runs
         const RingSub S = ring_sub(P, jobs, groups, twq + (P.tw_n >> 2) + 1);
         ring_build_Z<SH>(P, S, Fm, min(mcap, ring_mtop(P, S.job.ringA, spin2)), S.scratch, mmax != nullptr, true);
-        ring_bar(S.nt);
+        __syncthreads();
         const double sn = sqrt((double)S.n);
         double* oa = mapQ + ring_first_pixel<SH>(P, S.job.ringA);
         double* ob = mapU + ring_first_pixel<SH>(P, S.job.ringA);
@@ -757,9 +678,6 @@ ring_synth_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __res
         return;
     }
     load_twq(P, twq);
-#if RING_SUBBAR
-    __syncthreads();   // the twiddle table is loaded by the whole CTA; every later barrier may be a sub-ring one
-#endif
     const RingSub S = ring_sub(P, jobs, groups, twq + (P.tw_n >> 2) + 1);
     ring_build_Z<SH>(P, S, Fm, min(mcap, ring_mtop(P, S.job.ringA, spin2)), S.scratch, mmax != nullptr);
     ring_idft(P, S.buf, twq, S.n, S.bsi, S.tid, S.nt);
@@ -788,9 +706,6 @@ ring_anal_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __rest
     mapU += blockIdx.y * map_stride;
     double2* twq = smem;
     load_twq(P, twq);
-#if RING_SUBBAR
-    __syncthreads();   // the twiddle table is loaded by the whole CTA; every later barrier may be a sub-ring one
-#endif
     const RingSub S = ring_sub(P, jobs, groups, twq + (P.tw_n >> 2) + 1);
     const RingJob& job = S.job;
     const int n = S.n;
@@ -824,9 +739,6 @@ ring_mwg_data_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __
     double2* twq = smem;
     const bool spectral = group_const(wconst, jobs, groups);
     if (spectral) load_twq(P, twq);
-#if RING_SUBBAR
-    __syncthreads();
-#endif
     const RingSub S = ring_sub(P, jobs, groups, twq + (P.tw_n >> 2) + 1);
     const int n = S.n;
     const int64_t s0 = P.ring_start[S.job.ringA];
@@ -858,16 +770,6 @@ ring_mwg_data_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __
 // Ring stage of the PCG mat-vec A^T N^-1 A in ONE kernel: F_m(ring) -> pixels of the ring (kept in shared memory) ->
 // times the pixel weights -> F'_m(ring), written over F_m.  Equivalent to ring_synth_kernel + ring_anal_kernel(pixw)
 // without the map round trip through global memory, the second table load and the second launch.
-#ifdef GS_RING_DEBUG
-__device__ unsigned long long g_ring_dbg[4 * 8192];
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-__device__ __forceinline__ unsigned smid() { unsigned r; asm volatile("mov.u32 %0, %smid;" : "=r"(r)); return r; }
-extern "C" int gs_ring_debug_dump(unsigned long long* host, int n) { return (int)cudaMemcpyFromSymbol(host, g_ring_dbg, sizeof(unsigned long long) * n); }
-#define RING_DBG(slot) do { if (threadIdx.x == 0 && blockIdx.x < 8192) g_ring_dbg[4 * blockIdx.x + (slot)] = (slot) == 3 ? ((unsigned long long)smid() << 32 | (unsigned)S.M << 1 | (S.bsi >= 0)) : gtimer(); } while (0)
-#else
-#define RING_DBG(slot) do { } while (0)
-#endif
-
 template <bool SH>
 __global__ void __launch_bounds__(RF_NT, 2)
 ring_apply_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __restrict__ groups, double2* __restrict__ Fm,
@@ -916,24 +818,19 @@ ring_apply_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __res
             return;
         }
         ring_build_Z<SH>(P, S, Fm, mtop, S.scratch, false, true);
-        ring_bar(S.nt);
+        __syncthreads();
         const double half_n = 0.5 * (double)S.n;
         ring_unpack_F<SH>(P, S, UNPACK_PLAIN, Fm, mtop, nullptr, half_n * wA, half_n * wB);
         return;
     }
     load_twq(P, twq);
-#if RING_SUBBAR
-    __syncthreads();   // the twiddle table is loaded by the whole CTA; every later barrier may be a sub-ring one
-#endif
     const RingSub S = ring_sub(P, jobs, groups, twq + (P.tw_n >> 2) + 1);
     const int n = S.n;
     const double* wa = pixw + ring_first_pixel<SH>(P, S.job.ringA);
     const double* wb = S.job.ringB >= 0 ? pixw + ring_first_pixel<SH>(P, S.job.ringB) : wa;
-    RING_DBG(0); RING_DBG(3);
     const int mtop = ring_mtop(P, S.job.ringA, spin2);
     ring_build_Z<SH>(P, S, Fm, mtop, S.scratch);
-    ring_bar(S.nt);
-    RING_DBG(1);
+    __syncthreads();
     ring_idft(P, S.buf, twq, n, S.bsi, S.tid, S.nt);
     if (S.bsi < 0) {
         // pixels z_j = a_j + i b_j in natural order -> weighted (as the first pass of the transform loads them) -> forward DIF
@@ -943,20 +840,10 @@ ring_apply_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __res
         ring_unpack_F<SH>(P, S, UNPACK_BREV, Fm, mtop);
     } else {
         // Bluestein both ways: Z = conj(idft(conj z)); the chirp of the synthesis output, the pixel weights, the chirp of the
-        // analysis input and the zero padding are applied as the first pass of the second convolution loads its input, the last
-        // chirp as the spectrum is unpacked: no pointwise trip through shared memory is left
-        const double2* chirp = S.chirp;
-#if RING_FUSE_MID
-        auto mid = [wa, wb, chirp, n](int j, double2 v) {
-            if (j >= n) return make_double2(0.0, 0.0);
-            const double2 c = __ldg(&chirp[j]);
-            const double2 z = cmul(v, c);
-            return cmul(make_double2(z.x * wa[j], -z.y * wb[j]), c);
-        };
-        ring_idft_bs_pre(P, S.buf, twq, S.bsi, S.tid, S.nt, mid);
-#else
+        // analysis input and the zero padding are applied in one pointwise pass, the last chirp as the spectrum is unpacked
         // (fusing this product into the first radix-16 pass of the next transform was measured SLOWER: 49 vs 43 us per 4096-point
         // ring; 48 more global loads inside a pass that already holds 16 complex values in registers, and spills)
+        const double2* chirp = S.chirp;
         for (int j = S.tid; j < S.M; j += S.nt) {
             if (j >= n) { S.buf[PADI(j)] = make_double2(0.0, 0.0); continue; }
             const double2 c = __ldg(&chirp[j]);
@@ -964,17 +851,9 @@ ring_apply_kernel(PlanDev P, const RingJob* __restrict__ jobs, const int2* __res
             S.buf[PADI(j)] = cmul(make_double2(z.x * wa[j], -z.y * wb[j]), c);
         }
         ring_idft(P, S.buf, twq, n, S.bsi, S.tid, S.nt);
-#endif
-#if RING_UNPACK_CHIRP
         ring_unpack_F<SH>(P, S, UNPACK_CONJ, Fm, mtop, chirp);
-#else
-        for (int k = S.tid; k < n; k += S.nt) S.buf[PADI(k)] = cmul(S.buf[PADI(k)], __ldg(&chirp[k]));
-        ring_bar(S.nt);
-        ring_unpack_F<SH>(P, S, UNPACK_CONJ, Fm, mtop);
-#endif
     }
-    ring_bar(S.nt);
-    RING_DBG(2);
+    __syncthreads();
 }
 
 // ------------------------------------------------------------------ split path (rings longer than one CTA can hold)

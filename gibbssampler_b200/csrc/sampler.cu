@@ -411,7 +411,7 @@ extern "C" int gs_mul(const double* a, const double* b, double* out, int64_t n, 
 //   dM_k = A (dfl_k (.) s_nc),  dfl_k[l] = b_l (sqrt(C'_l) - sqrt(C_l)) on block k, 0 elsewhere,
 // the candidate likelihood of block k is -1/2 sum N^-1 (r - dM_k)^2 and an acceptance is r -= dM_k.  All dM_k of a
 // group of blocks come out of ONE Legendre pass (leg_synth_blocks_kernel) and one batched ring-FFT launch; each
-// Metropolis test is then three small launches (chi^2 partials, decide, conditional r update), nothing leaves the device.
+// Metropolis test is then one launch (mwg_step_kernel), nothing leaves the device.
 __global__ void mwg_dfl_kernel(const double* cur_E, const double* cur_B, const double* prop_E, const double* prop_B,
                                const int* bins_E, int nb_E, const int* bins_B, int nb_B, int eb0, int eb1, int bb0, int bb1,
                                const double* bl, int L, int l_cut, double* flE, double* flB, double* dflE, double* dflB)
@@ -444,51 +444,8 @@ mwg_resid_kernel(const double* __restrict__ dQ, const double* __restrict__ dU, d
     block_sum<1>(v, partials + blockIdx.x);
 }
 
-// chi^2 partials of the candidate r - dM_k (the block's change is already in r when *applied != 0)
-__global__ void __launch_bounds__(SM_NT)
-mwg_test_kernel(const double* __restrict__ rQ, const double* __restrict__ rU, const double* __restrict__ gQ,
-                const double* __restrict__ gU, const double* __restrict__ invn, int64_t n, const int* __restrict__ applied,
-                double* __restrict__ partials)
-{
-    const bool sub = *applied == 0;
-    double v[1] = {0.0};
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        double a = rQ[i], b = rU[i];
-        if (sub) { a -= gQ[i]; b -= gU[i]; }
-        v[0] = fma(fma(b, b, a * a), invn[i], v[0]);
-    }
-    block_sum<1>(v, partials + blockIdx.x);
-}
-
-// lik[0] = old, lik[1] = new; flags[0] = do_apply for the following mwg_apply_kernel
-__global__ void __launch_bounds__(SM_NT)
-mwg_decide_kernel(const double* __restrict__ partials, int np, double* cur, const double* prop, const double* logr, int b0,
-                  int b1, double* lik, const double* u, int* applied, int* do_apply, int* accept_out)
-{
-    double v[1] = {0.0};
-    for (int i = threadIdx.x; i < np; i += blockDim.x) v[0] += partials[i];
-    __shared__ double res[1];
-    block_sum<1>(v, res);
-    __syncthreads();
-    if (threadIdx.x) return;
-    const double new_lik = -0.5 * res[0];
-    double s = 0.0;
-    for (int b = b0; b < b1; ++b) s += logr[b];
-    const bool acc = log(u[0]) < s + (new_lik - lik[0]);
-    int apply = 0;
-    if (acc) {
-        lik[0] = new_lik;
-        if (*applied == 0) {
-            for (int b = b0; b < b1; ++b) cur[b] = prop[b];
-            *applied = 1;
-            apply = 1;
-        }
-    }
-    lik[1] = new_lik;
-    *do_apply = apply;
-    accept_out[0] = acc ? 1 : 0;
-}
-
+// r -= (gQ, gU) when the last test accepted (*do_apply != 0): the pending update of mwg_step_kernel, applied on its own
+// before the block maps it reads are overwritten
 __global__ void __launch_bounds__(SM_NT)
 mwg_apply_kernel(double* __restrict__ rQ, double* __restrict__ rU, const double* __restrict__ gQ, const double* __restrict__ gU,
                  int64_t n, const int* __restrict__ do_apply)
@@ -500,11 +457,11 @@ mwg_apply_kernel(double* __restrict__ rQ, double* __restrict__ rU, const double*
     }
 }
 
-// One Metropolis test in one launch (default; GS_MWG_FUSED=0 restores test / decide / apply): the r update of the PREVIOUS test
-// (pend_flag, maps pQ / pU) is applied as r is read, the chi^2 partials of the candidate follow, and the block that finishes last sums
-// them in the order of mwg_decide_kernel and takes the decision.  Same numbers as the three kernels: 252 instead of 756 launches
-// per sweep and one pass over r less per accepted block.  pend_flag may alias do_apply_out and `applied` is written by the deciding
-// block only: every block reads both before its loop, and the decision comes after all loops (counter).
+// One Metropolis test in one launch: the r update of the PREVIOUS test (pend_flag, maps pQ / pU) is applied as r is read, the
+// chi^2 partials of the candidate r - dM_k follow (the block's change is already in r when *applied != 0), and the block that
+// finishes last sums them in a fixed order and takes the decision: lik[0] = old, lik[1] = new likelihood.  pend_flag may alias
+// do_apply_out and `applied` is written by the deciding block only: every block reads both before its loop, and the decision
+// comes after all loops (counter).
 __global__ void __launch_bounds__(SM_NT)
 mwg_step_kernel(double* __restrict__ rQ, double* __restrict__ rU, const double* __restrict__ pQ, const double* __restrict__ pU,
                 const int* pend_flag, const double* __restrict__ gQ, const double* __restrict__ gU,
@@ -638,7 +595,6 @@ extern "C" int gs_mwg_sweep_blocks(gs_plan* p, const double* snc_E, const double
     int* flags = p->mwg_meta + meta.size();  // [ntot] applied, then do_apply, then the ticket counter of mwg_step_kernel
     int* do_apply = flags + ntot;
     unsigned* ticket = reinterpret_cast<unsigned*>(flags + ntot + 1);
-    static const bool fused_steps = [] { const char* e = getenv("GS_MWG_FUSED"); return !(e && e[0] == '0'); }();
     double* partials = p->mwg_small;
     double* lik = partials + SM_GRID;
     double* flE = lik + 8;
@@ -653,7 +609,7 @@ extern "C" int gs_mwg_sweep_blocks(gs_plan* p, const double* snc_E, const double
     // Rings on which N^-1 is one number w (isotropic noise, not cut by the mask edge; gs_set_ring_const): every quantity of the sweep
     // on such a ring is w sum_j |z_j - z'_j|^2 with z = Q + i U, which the unitary DFT along the ring leaves unchanged.  Data, current
     // model and all block maps of these rings are therefore kept as sqrt(n) times the alias-folded ring spectrum (what the ring FFT
-    // would start from) and their FFTs are never run; test / decide / apply kernels see ordinary arrays.
+    // would start from) and their FFTs are never run; the Metropolis test kernels see ordinary arrays.
     const unsigned char* ract = nullptr;
     const double* wconst = nullptr;
     if (g_gs_ring_skip) {
@@ -710,20 +666,11 @@ extern "C" int gs_mwg_sweep_blocks(gs_plan* p, const double* snc_E, const double
             const double* gU = p->mwg_maps + (int64_t)(G + k - g0) * npix;
             for (int it = 0; it < n_iter; ++it) {
                 const int64_t idx = (int64_t)k * n_iter + it;
-                if (fused_steps) {
-                    mwg_step_kernel<<<SM_GRID, SM_NT, 0, st>>>(rQ, rU, pQ, pU, do_apply, gQ, gU, inv_noise, npix, partials, ticket,
-                                                               isE ? cur_E : cur_B, isE ? prop_E : prop_B, isE ? logr_E : logr_B, blocks[i],
-                                                               blocks[i + 1], lik, u + idx, flags + k, do_apply, accept_out + idx);
-                    pQ = gQ; pU = gU;
-                    g_gs_launches += 1;
-                    continue;
-                }
-                mwg_test_kernel<<<SM_GRID, SM_NT, 0, st>>>(rQ, rU, gQ, gU, inv_noise, npix, flags + k, partials);
-                mwg_decide_kernel<<<1, SM_NT, 0, st>>>(partials, SM_GRID, isE ? cur_E : cur_B, isE ? prop_E : prop_B,
-                                                        isE ? logr_E : logr_B, blocks[i], blocks[i + 1], lik, u + idx, flags + k,
-                                                        do_apply, accept_out + idx);
-                mwg_apply_kernel<<<SM_GRID, SM_NT, 0, st>>>(rQ, rU, gQ, gU, npix, do_apply);
-                g_gs_launches += 3;
+                mwg_step_kernel<<<SM_GRID, SM_NT, 0, st>>>(rQ, rU, pQ, pU, do_apply, gQ, gU, inv_noise, npix, partials, ticket,
+                                                           isE ? cur_E : cur_B, isE ? prop_E : prop_B, isE ? logr_E : logr_B, blocks[i],
+                                                           blocks[i + 1], lik, u + idx, flags + k, do_apply, accept_out + idx);
+                pQ = gQ; pU = gU;
+                g_gs_launches += 1;
             }
         }
         GS_CHECK_LAUNCH();

@@ -2,8 +2,8 @@
 exactly what the device code does lane by lane / thread by thread, so that a change of the scheme has to be made (and
 argued) in two places:
 
-* the spin-2 analysis reduce-scatter (legendre.cu: anal_acc2, the select-free exchange stages, the swizzled shared-memory
-  park + batched sum of LEG_FOLD3): every (l-parity h, value c) must come out as the sum over the 32 lanes, at the index the
+* the spin-2 analysis reduce-scatter (legendre.cu: anal_acc, the select-free exchange stages, the swizzled shared-memory
+  park + batched sum over FOLD3_NB pairs of l in the fast loop of leg_anal_kernel): every (l-parity h, value c) must come out as the sum over the 32 lanes, at the index the
   kernel writes (h * 4 + c), with the sign flip of (h = 1, odd c);
 * the complex-coefficient decode c -> (l, m) of loglik_alm_partial_kernel (sampler.cu) and its real-layout offsets
   (utils.py:49-76 of the reference: r[l] for m = 0, r[2 i - (L+1)], r[2 i - (L+1) + 1] for i > L)."""
