@@ -8,7 +8,13 @@ The reference never finished this path: the per-l 3x3 helpers survive only as by
 3x3 solve:
     Sigma_l = (C_l^-1 + diag(b_l^2 w_X))^-1,  s = Sigma_l (b_l w_X d_X)_X + chol(Sigma_l) xi,  w_X = Npix / (4 pi sigma^2_X)
 and  (C^TT, C^TE, C^EE)_l | s ~ IW(2l - 2, (2l+1) Chat_l),  C^BB_l | s ~ inverse-gamma as in CenteredGibbs.py:54-79.
-Every step is a batched one-thread-per-l (or per-coefficient) kernel of libgibbs_b200.so."""
+Every step is a batched one-thread-per-l (or per-coefficient) kernel of libgibbs_b200.so.
+
+On a cut sky (pixel data, one mask for T and another for P, per-pixel noise) the constrained realization is the joint T/E/B
+system Q x = b of qcinv's joint T+P filter, solved by the TE-coupled PCG of gs_cr_pcg_teb (include/gibbs_b200.h)."""
+import ctypes as C
+import math
+
 import numpy as np
 import torch
 
@@ -18,15 +24,24 @@ from ._lib import check, GS_ALM_REAL
 
 
 class JointConstrainedRealization():
-    def __init__(self, pix_map, noise_temp, noise_pol, bl_gauss, lmax, Npix, *, rng="philox", seed=None):
-        """pix_map: {"TT","EE","BB"} data alms in the real layout; noise_*: per-pixel noise variances (scalars)."""
+    def __init__(self, pix_map, noise_temp, noise_pol, bl_gauss, lmax, Npix, *, mask=None, mask_pol=None, rng="philox", seed=None,
+                 plan=None):
+        """pix_map: either {"TT","EE","BB"} data alms in the real layout (full sky, isotropic noise: closed-form draw; noise_*
+        are scalar per-pixel variances), or {"I","Q","U"} RING maps (masked sky: PCG on the joint T/E/B system).  With maps,
+        noise_* are scalars or per-pixel variance maps, `mask` (RING array) multiplies N_T^-1 and `mask_pol` (default: `mask`)
+        multiplies N_P^-1: N_T^-1 = mask / noise_temp, N_P^-1 = mask_pol / noise_pol.  `plan`: a single-GPU sht.Plan (default:
+        the cached plan of (nside, lmax)); the joint solve does not run on m-sharded plans."""
         self.lmax, self.Npix = int(lmax), int(Npix)
         self.dev = _dev.device()
         self.n = (self.lmax + 1) ** 2
         self.bl = f64(bl_gauss)
+        self.rng = rng if isinstance(rng, _dev.Rng) else _dev.Rng(rng, seed)
+        self.pixel = "I" in pix_map
+        if self.pixel:
+            self._init_masked(pix_map, noise_temp, noise_pol, mask, mask_pol, plan)
+            return
         self.w = torch.tensor([self.Npix / (4 * np.pi * float(noise_temp)), self.Npix / (4 * np.pi * float(noise_pol)),
                                self.Npix / (4 * np.pi * float(noise_pol))], dtype=torch.float64, device=self.dev)
-        self.rng = rng if isinstance(rng, _dev.Rng) else _dev.Rng(rng, seed)
         d = torch.stack([f64(pix_map["TT"]), f64(pix_map["EE"]), f64(pix_map["BB"])], dim=1).contiguous()   # (n, 3)
         from . import utils
         blx = utils.expand_per_l(self.bl, 0)
@@ -44,7 +59,109 @@ class JointConstrainedRealization():
         c[:, 0, 1] = c[:, 1, 0] = f64(all_dls["TE"]) * f
         return c.contiguous()
 
+    # ------------------------------------------------------------------ masked sky: joint PCG
+    def _init_masked(self, pix_map, noise_temp, noise_pol, mask, mask_pol, plan):
+        from .sht import Plan
+        self.nside = int(round(math.sqrt(self.Npix / 12)))
+        if 12 * self.nside ** 2 != self.Npix:
+            raise ValueError("Npix = %d is not 12 nside^2" % self.Npix)
+        self.plan = plan if plan is not None else Plan.get(self.nside, self.lmax)
+        if self.plan.world > 1:
+            raise _lib.GibbsB200Error("the joint T/E/B constrained realization needs a single-GPU plan (this one is m-sharded over "
+                                      "%d ranks)" % self.plan.world)
+        mT = _dev.load_mask(None, self.nside, mask)
+        mP = _dev.load_mask(None, self.nside, mask_pol) if mask_pol is not None else mT
+        self.inv_noise_T = self._inv_noise(noise_temp, mT)
+        same = mask_pol is None and np.array_equal(np.asarray(_dev.to_host(noise_pol)), np.asarray(_dev.to_host(noise_temp)))
+        # one array for both when they are equal: the library then builds its ring flags once per call
+        self.inv_noise_P = self.inv_noise_T if same else self._inv_noise(noise_pol, mP)
+        self.sqrt_inv_noise_T = torch.sqrt(self.inv_noise_T)
+        self.sqrt_inv_noise_P = self.sqrt_inv_noise_T if same else torch.sqrt(self.inv_noise_P)
+        self.ninvT_sum_over_4pi = _dev.dsum(self.inv_noise_T) / (4 * np.pi)
+        self.ninvP_sum_over_4pi = _dev.dsum(self.inv_noise_P) / (4 * np.pi)
+        d_I, d_Q, d_U = f64(pix_map["I"]), f64(pix_map["Q"]), f64(pix_map["U"])
+        # constant data terms B A^T N^-1 d of every right-hand side
+        self.bdata_T = self.plan.map2alm(d_I, adjoint=True, pixw=self.inv_noise_T, fl=self.bl, real_layout=True)
+        self.bdata_E, self.bdata_B = self.plan.map2alm_spin2(d_Q, d_U, adjoint=True, pixw=self.inv_noise_P, fl=self.bl,
+                                                             real_layout=True)
+        self.pcg_accuracy = 1.0e-6      # qcinv chain settings of the TT sampler (ConstrainedRealization.py:41)
+        self.pcg_itermax = 4000
+        self.pcg_check_every = 8
+        self.fluct_iter = 3             # utils.adjoint_synthesis_hp uses iter=3 (utils.py:89)
+        self.last_pcg_iterations, self.last_pcg_residual = 0, 0.0
+        self.last_rhs = None
+
+    def _inv_noise(self, noise, mask):
+        n = f64(noise).reshape(-1)
+        if n.numel() == 1:
+            n = n.expand(self.Npix)
+        if n.numel() != self.Npix:
+            raise ValueError("noise must be a scalar or a map of %d pixels" % self.Npix)
+        inv = (1.0 / n).contiguous()
+        if mask is not None:
+            inv.mul_(f64(mask))
+        return inv
+
+    def _dls(self, all_dls):
+        out = tuple(f64(all_dls[k]).reshape(-1) for k in ("TT", "TE", "EE", "BB"))
+        assert all(x.numel() == self.lmax + 1 for x in out), "need unbinned D_l of length lmax+1"
+        return out
+
+    def _masked_only(self, what):
+        if not self.pixel:
+            raise _lib.GibbsB200Error("%s needs pixel data (pix_map with 'I', 'Q', 'U')" % what)
+
+    def build_rhs(self, all_dls, xi=None):
+        """b of Q x = b.  xi = (xi_I, xi_Q, xi_U, xi_T, xi_E, xi_B) may be injected; drawn in that order otherwise."""
+        self._masked_only("build_rhs")
+        tt, te, ee, bb = self._dls(all_dls)
+        if xi is None:
+            xi = tuple(self.rng.normal(self.Npix) for _ in range(3)) + tuple(self.rng.normal(self.n) for _ in range(3))
+        xi = [f64(x).reshape(-1) for x in xi]
+        rhs = tuple(torch.empty(self.n, dtype=torch.float64, device=self.dev) for _ in range(3))
+        check(_lib.lib().gs_cr_rhs_teb(self.plan._h, ptr(tt), ptr(te), ptr(ee), ptr(bb), ptr(self.bl), ptr(self.inv_noise_T),
+                                       ptr(self.sqrt_inv_noise_T), ptr(self.inv_noise_P), ptr(self.sqrt_inv_noise_P),
+                                       ptr(self.bdata_T), ptr(self.bdata_E), ptr(self.bdata_B), None, None, None,
+                                       *[ptr(x) for x in xi], self.fluct_iter, *[ptr(r) for r in rhs], stream()))
+        return rhs
+
+    def solve(self, all_dls, rhs_t, rhs_e, rhs_b, x0=None):
+        """PCG solve of the joint system; x0 = {"TT","EE","BB"} warm start.  -> (x_T, x_E, x_B)"""
+        self._masked_only("solve")
+        tt, te, ee, bb = self._dls(all_dls)
+        if x0 is None:
+            x = tuple(torch.empty(self.n, dtype=torch.float64, device=self.dev) for _ in range(3))
+        else:
+            x = tuple(f64(x0[k]).clone() for k in ("TT", "EE", "BB"))
+        rhs = tuple(f64(r) for r in (rhs_t, rhs_e, rhs_b))
+        nit, res = C.c_int(0), C.c_double(0.0)
+        rc = _lib.lib().gs_cr_pcg_teb(self.plan._h, ptr(tt), ptr(te), ptr(ee), ptr(bb), ptr(self.bl), ptr(self.inv_noise_T),
+                                      ptr(self.inv_noise_P), self.ninvT_sum_over_4pi, self.ninvP_sum_over_4pi,
+                                      *[ptr(r) for r in rhs], *[ptr(v) for v in x], 0 if x0 is None else 1, self.pcg_accuracy,
+                                      self.pcg_itermax, self.pcg_check_every, C.byref(nit), C.byref(res), stream())
+        self.last_pcg_iterations, self.last_pcg_residual = nit.value, res.value
+        if rc not in (0, -3):  # GS_E_NOTCONVERGED (-3) is reported through last_pcg_residual, as in the E/B sampler
+            check(rc)
+        return x
+
+    def apply_Q(self, all_dls, x):
+        """y = Q x for x = {"TT","EE","BB"} (real layout)."""
+        self._masked_only("apply_Q")
+        tt, te, ee, bb = self._dls(all_dls)
+        xs = [f64(x[k]) for k in ("TT", "EE", "BB")]
+        ys = [torch.empty_like(v) for v in xs]
+        check(_lib.lib().gs_cr_apply_q_teb(self.plan._h, ptr(tt), ptr(te), ptr(ee), ptr(bb), ptr(self.bl), ptr(self.inv_noise_T),
+                                           ptr(self.inv_noise_P), *[ptr(v) for v in xs], *[ptr(v) for v in ys], stream()))
+        return {"TT": ys[0], "EE": ys[1], "BB": ys[2]}
+
     def sample(self, all_dls, xi=None):
+        """-> ({"TT","EE","BB"} real-layout alms, 1).  Pixel data: RHS + joint PCG (xi: the six arrays of build_rhs);
+        harmonic data: the closed-form per-coefficient draw (xi: (n, 3) normals)."""
+        if self.pixel:
+            rhs = self.build_rhs(all_dls, xi)
+            self.last_rhs = rhs
+            x = self.solve(all_dls, *rhs)
+            return {"TT": x[0], "EE": x[1], "BB": x[2]}, 1
         L = _lib.lib()
         cl = self.covariances(all_dls)
         sig = torch.empty_like(cl)
@@ -98,13 +215,16 @@ class JointClsSampler():
 
 
 class JointGibbs():
-    """CR <-> C_l Gibbs loop for (T, E, B) with TE correlation; full sky, isotropic noise."""
+    """CR <-> C_l Gibbs loop for (T, E, B) with TE correlation: full sky with isotropic noise and harmonic data
+    ({"TT","EE","BB"}), or a cut sky with pixel data ({"I","Q","U"}, masks `mask` for T and `mask_pol` for P)."""
 
-    def __init__(self, pix_map, noise_temp, noise_pol, beam_fwhm_deg, nside, lmax, n_iter=1000, *, rng="philox", seed=None):
+    def __init__(self, pix_map, noise_temp, noise_pol, beam_fwhm_deg, nside, lmax, n_iter=1000, *, mask=None, mask_pol=None,
+                 rng="philox", seed=None):
         self.lmax, self.nside, self.n_iter = int(lmax), int(nside), int(n_iter)
         bl = _dev.gauss_beam(np.radians(beam_fwhm_deg), self.lmax)
         shared = _dev.Rng(rng, seed)
-        self.constrained_sampler = JointConstrainedRealization(pix_map, noise_temp, noise_pol, bl, lmax, 12 * nside ** 2, rng=shared)
+        self.constrained_sampler = JointConstrainedRealization(pix_map, noise_temp, noise_pol, bl, lmax, 12 * nside ** 2, mask=mask,
+                                                               mask_pol=mask_pol, rng=shared)
         self.cls_sampler = JointClsSampler(lmax, rng=shared)
 
     def run(self, dls_init):

@@ -55,6 +55,9 @@ SIGNATURES = {
     "gs_cr_rhs_tt": (_i, [_vp] * 9 + [_i, _vp, _vp]),
     "gs_cr_pcg_tt": (_i, [_vp, _vp, _vp, _vp, _d, _vp, _vp, _i, _d, _i, _i, C.POINTER(_i), C.POINTER(_d), _vp]),
     "gs_cr_apply_q_tt": (_i, [_vp] * 7),
+    "gs_cr_rhs_teb": (_i, [_vp] * 22 + [_i, _vp, _vp, _vp, _vp]),
+    "gs_cr_pcg_teb": (_i, [_vp] * 8 + [_d, _d] + [_vp] * 6 + [_i, _d, _i, _i, C.POINTER(_i), C.POINTER(_d), _vp]),
+    "gs_cr_apply_q_teb": (_i, [_vp] * 15),
     "gs_gibbs_run_centered_fullsky": (_i, [_i, _i64, _d, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _i, C.c_uint64, _vp, _vp, _vp, _vp,
                                            _i, _vp]),
     "gs_cr_direct": (_i, [_vp, _vp, _vp, _vp, _d, _i, _i, _vp, _vp]),
@@ -108,6 +111,7 @@ SIGNATURES = {
     "gs_profile_matvec_batch": (_i, [_vp, _i, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _i, C.POINTER(C.c_float), _vp]),
     "gs_measure_fp64_peak": (_i, [C.POINTER(_d), _vp]),
     "gs_profile_pcg_vectors": (_i, [_vp, _i, _i, C.POINTER(C.c_float), _vp]),
+    "gs_profile_matvec_teb": (_i, [_vp, _vp, _vp, _vp, _i, C.POINTER(C.c_float), _vp]),
     "gs_set_ring_fused": (_i, [_i]),
     "gs_set_ring_skip": (_i, [_i]),
     "gs_set_ring_const": (_i, [_i]),

@@ -123,6 +123,18 @@ struct PlanDev {
     ShardDev sh;           // world == 1: unused
 };
 
+// One set of ring flags built from one weight map (gs_active_rings_build): the plan's own set lives in the gs_plan fields of
+// the same names; the joint T/E/B solve keeps a second set for N_T^-1 here and swaps it in while its spin-0 half is enqueued.
+struct RingFlags {
+    unsigned char* act_ring;
+    int* act_pairs;
+    int* act_count;
+    int* act_slot0;
+    double* ring_wconst;
+    int2* groups0_dyn;
+    int2* groups2_dyn;
+};
+
 struct gs_plan {
     int device;
     PlanDev d;
@@ -186,6 +198,8 @@ struct gs_plan {
     void* pcg_ws;       // gs_pcg_ws* (solver.cu): PCG vectors / state of this plan, allocated on the first solve
     void* pcg_ws_batch; // gs_pcg_ws[2]: workspaces of a two-chain batch (gs_cr_pcg_pol_batch), allocated on first use
     int* pcg_alldone;   // device flag: both chains of the batch have converged
+    void* pcg_ws_teb;   // TebWs* (solver.cu): vectors / state of the joint T/E/B solve, allocated on its first use
+    RingFlags flags_T;  // second ring-flag set of the joint T/E/B solve (N_T^-1); all NULL until its first use
     void* comm_stream;  // cudaStream_t the block-wise all-to-all of a sharded plan runs on (NULL until first used)
     std::vector<void*> comm_events;   // cudaEvent_t: NB + 1 of them
     void* work_stream;  // cudaStream_t of the plan for graph-captured solves (NULL until first used)

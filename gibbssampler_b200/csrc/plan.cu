@@ -260,6 +260,8 @@ static int plan_create_impl(gs_plan** out, int nside, int lmax, int device, int 
     p->pcg_ws = nullptr;
     p->pcg_ws_batch = nullptr;
     p->pcg_alldone = nullptr;
+    p->pcg_ws_teb = nullptr;
+    memset(&p->flags_T, 0, sizeof(p->flags_T));
     p->work_stream = nullptr;
     p->work_event = nullptr;
     p->comm_stream = nullptr;

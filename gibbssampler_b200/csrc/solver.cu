@@ -385,8 +385,10 @@ static gs_pcg_ws* get_ws_batch(gs_plan* p)
     return w;
 }
 
+static void teb_ws_free(gs_plan* p);
 void gs_pcg_ws_free(gs_plan* p)
 {
+    teb_ws_free(p);
     gs_pcg_ws* w = (gs_pcg_ws*)p->pcg_ws;
     if (w) {
         if (w->host_state) cudaFreeHost(w->host_state);   // the device buffers are in p->owned
@@ -449,6 +451,107 @@ static int apply_noise_op(gs_plan* p, const double* vE, const double* vB, const 
     return gs_leg_anal(p, spin, qE, qB, GS_ALM_REAL, bl, 1.0, 0, st, skip, fuse, nc, stride);
 }
 
+// The poll loop shared by the PCG solves: `iteration(stream)` enqueues one PCG iteration whose launches take every scalar
+// (alpha, beta, the done flag) from `state` on the device.  The solver state has been initialised on `st` before the call.
+template <class Iteration>
+static int pcg_poll_loop(gs_plan* p, cudaStream_t st, PcgState* state, PcgState* host_state, bool dist, double eps, int itermax,
+                         int check_every, Iteration& iteration, int* n_iter_out, double* resid_out)
+{
+    // Unsharded plans: the `check_every` iterations between two polls of the convergence flag are captured ONCE per solve in a
+    // CUDA graph on a stream of the plan (capture is not allowed on the legacy default stream) and replayed: one graph launch
+    // instead of 7 check_every kernel launches per poll (the host side of a solve was ~2300 launches; SCALE_r01 lost 1.8 % at 8
+    // GPUs to 8 processes doing that on shared cores).  gs_set_pcg_graph(0) restores plain launches.
+    int rc = GS_OK;
+    int launched = 0;
+    bool finished = false;
+    cudaGraphExec_t gexec = nullptr;
+    long long launches_per_graph = 0;
+    static const bool env_graph_off = [] { const char* e = getenv("GS_PCG_GRAPH"); return e && e[0] == '0'; }();   // GS_PCG_GRAPH=0: plain launches
+    if (g_gs_pcg_graph && !env_graph_off && !dist && itermax >= check_every) {
+        if (!p->work_stream) {
+            cudaStream_t ws = nullptr;
+            GS_CHECK_CUDA(cudaStreamCreateWithFlags(&ws, cudaStreamNonBlocking));
+            p->work_stream = ws;
+            cudaEvent_t ev = nullptr;
+            GS_CHECK_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+            p->work_event = ev;
+        }
+        cudaStream_t ws = (cudaStream_t)p->work_stream;
+        GS_CHECK_CUDA(cudaEventRecord((cudaEvent_t)p->work_event, st));
+        GS_CHECK_CUDA(cudaStreamWaitEvent(ws, (cudaEvent_t)p->work_event, 0));
+        st = ws;   // the rest of the solve runs here; every poll (and the return) synchronises it with the host
+        cudaGraph_t graph = nullptr;
+        const long long l0 = g_gs_launches;
+        GS_CHECK_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+        rc = GS_OK;
+        for (int k = 0; k < check_every && rc == GS_OK; ++k) rc = iteration(st);
+        cudaError_t ce = cudaStreamEndCapture(st, &graph);
+        launches_per_graph = g_gs_launches - l0;
+        g_gs_launches = l0;   // nothing ran yet: counted per replay below
+        if (rc != GS_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
+        if (ce != cudaSuccess) { gs_set_error("PCG graph capture: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
+        ce = cudaGraphInstantiate(&gexec, graph, 0);
+        cudaGraphDestroy(graph);
+        if (ce != cudaSuccess) { gs_set_error("PCG graph instantiate: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
+    }
+    if (gexec) {
+        // Two batches in flight: the host enqueues batch k + 1 (graph replay + copy of the solver state + event) BEFORE it waits for the
+        // state that follows batch k, so the wake-up after a poll and the next graph launch are hidden behind 8 iterations of GPU work
+        // (43 polls per solve at NSIDE 512; with 8 ranks on shared host cores this was the remaining loss of the chains mode).  Once
+        // the done flag is set every kernel of a later batch returns at once: at most one batch of no-ops per solve, same iterations.
+        PcgState* hs = host_state;
+        cudaEvent_t ev[2] = {nullptr, nullptr};
+        cudaError_t ce = cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming);
+        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming);
+        int cur = 0, inflight = 0;
+        while (ce == cudaSuccess && !finished) {
+            while (ce == cudaSuccess && inflight < 2 && launched + check_every <= itermax) {
+                const int sl = (cur + inflight) & 1;
+                ce = cudaGraphLaunch(gexec, st);
+                if (ce == cudaSuccess) ce = cudaMemcpyAsync(hs + sl, state, sizeof(PcgState), cudaMemcpyDeviceToHost, st);
+                if (ce == cudaSuccess) ce = cudaEventRecord(ev[sl], st);
+                launched += check_every;
+                g_gs_launches += launches_per_graph;
+                ++inflight;
+            }
+            if (ce != cudaSuccess || inflight == 0) break;   // fewer than check_every iterations left: the loop below runs them
+            ce = cudaEventSynchronize(ev[cur]);
+            if (ce != cudaSuccess) break;
+            --inflight;
+            if (hs[cur].done || launched >= itermax) {
+                if (inflight) ce = cudaStreamSynchronize(st);   // the batch behind it: no-ops after `done`, or the last iterations
+                if (inflight && ce == cudaSuccess) cur ^= 1;
+                hs[0] = hs[cur];
+                finished = hs[0].done || launched >= itermax;
+                inflight = 0;
+                if (!finished) cur = 0;
+                continue;
+            }
+            cur ^= 1;
+        }
+        if (ev[0]) cudaEventDestroy(ev[0]);
+        if (ev[1]) cudaEventDestroy(ev[1]);
+        if (ce != cudaSuccess) { cudaGraphExecDestroy(gexec); gs_set_error("PCG graph loop: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
+    }
+    while (!finished) {
+        for (int k = 0; k < check_every && launched < itermax; ++k, ++launched)
+            if ((rc = iteration(st))) { if (gexec) cudaGraphExecDestroy(gexec); return rc; }
+        cudaError_t ce = cudaMemcpyAsync(host_state, state, sizeof(PcgState), cudaMemcpyDeviceToHost, st);
+        if (ce == cudaSuccess) ce = cudaStreamSynchronize(st);
+        if (ce != cudaSuccess) { if (gexec) cudaGraphExecDestroy(gexec); gs_set_error("PCG poll: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
+        finished = host_state->done || launched >= itermax;
+    }
+    if (gexec) cudaGraphExecDestroy(gexec);
+    const PcgState& s = *host_state;
+    if (n_iter_out) *n_iter_out = s.iter;
+    if (resid_out) *resid_out = s.d0 > 0.0 ? sqrt(s.rr / s.d0) : 0.0;
+    if (s.d0 > 0.0 && s.rr > s.eps2 * s.d0) {
+        gs_set_error("PCG stopped at iter_max = %d with |r|/|r0| = %.3e > eps = %.1e", itermax, sqrt(s.rr / s.d0), eps);
+        return GS_E_NOTCONVERGED;
+    }
+    return GS_OK;
+}
+
 // spin 2: (E, B) system; spin 0: temperature (dl_BB, rhs_B, x_B unused)
 static int cr_pcg_impl(gs_plan* p, int spin, const double* dl_EE, const double* dl_BB, const double* bl,
                        const double* inv_noise, double ninv_sum_over_4pi, const double* rhs_E,
@@ -505,8 +608,6 @@ static int cr_pcg_impl(gs_plan* p, int spin, const double* dl_EE, const double* 
     ff.pE = w->p[0]; ff.pB = w->p[1]; ff.icE = tmp_l; ff.icB = tmp_l + 2 * (L + 1);
     ff.partials = w->fuse_partials; ff.counter = &w->state->counter; ff.out = w->fuse_out;
     const bool fused_apq = !dist && g_gs_fuse_apq;
-    int launched = 0;
-    bool finished = false;
     // one PCG iteration: 7 launches whose arguments do not change during the solve (alpha, beta and the done flag live on the device)
     auto iteration = [&](cudaStream_t s) -> int {
         int r;
@@ -527,96 +628,7 @@ static int cr_pcg_impl(gs_plan* p, int spin, const double* dl_EE, const double* 
         g_gs_launches += 3;
         return GS_OK;
     };
-    // Unsharded plans: the `check_every` iterations between two polls of the convergence flag are captured ONCE per solve in a
-    // CUDA graph on a stream of the plan (capture is not allowed on the legacy default stream) and replayed: one graph launch
-    // instead of 7 check_every kernel launches per poll (the host side of a solve was ~2300 launches; SCALE_r01 lost 1.8 % at 8
-    // GPUs to 8 processes doing that on shared cores).  gs_set_pcg_graph(0) restores plain launches.
-    cudaGraphExec_t gexec = nullptr;
-    long long launches_per_graph = 0;
-    static const bool env_graph_off = [] { const char* e = getenv("GS_PCG_GRAPH"); return e && e[0] == '0'; }();   // GS_PCG_GRAPH=0: plain launches
-    if (g_gs_pcg_graph && !env_graph_off && !dist && itermax >= check_every) {
-        if (!p->work_stream) {
-            cudaStream_t ws = nullptr;
-            GS_CHECK_CUDA(cudaStreamCreateWithFlags(&ws, cudaStreamNonBlocking));
-            p->work_stream = ws;
-            cudaEvent_t ev = nullptr;
-            GS_CHECK_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            p->work_event = ev;
-        }
-        cudaStream_t ws = (cudaStream_t)p->work_stream;
-        GS_CHECK_CUDA(cudaEventRecord((cudaEvent_t)p->work_event, st));
-        GS_CHECK_CUDA(cudaStreamWaitEvent(ws, (cudaEvent_t)p->work_event, 0));
-        st = ws;   // the rest of the solve runs here; every poll (and the return) synchronises it with the host
-        cudaGraph_t graph = nullptr;
-        const long long l0 = g_gs_launches;
-        GS_CHECK_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-        rc = GS_OK;
-        for (int k = 0; k < check_every && rc == GS_OK; ++k) rc = iteration(st);
-        cudaError_t ce = cudaStreamEndCapture(st, &graph);
-        launches_per_graph = g_gs_launches - l0;
-        g_gs_launches = l0;   // nothing ran yet: counted per replay below
-        if (rc != GS_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
-        if (ce != cudaSuccess) { gs_set_error("PCG graph capture: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
-        ce = cudaGraphInstantiate(&gexec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (ce != cudaSuccess) { gs_set_error("PCG graph instantiate: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
-    }
-    if (gexec) {
-        // Two batches in flight: the host enqueues batch k + 1 (graph replay + copy of the solver state + event) BEFORE it waits for the
-        // state that follows batch k, so the wake-up after a poll and the next graph launch are hidden behind 8 iterations of GPU work
-        // (43 polls per solve at NSIDE 512; with 8 ranks on shared host cores this was the remaining loss of the chains mode).  Once
-        // the done flag is set every kernel of a later batch returns at once: at most one batch of no-ops per solve, same iterations.
-        PcgState* hs = w->host_state;
-        cudaEvent_t ev[2] = {nullptr, nullptr};
-        cudaError_t ce = cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming);
-        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming);
-        int cur = 0, inflight = 0;
-        while (ce == cudaSuccess && !finished) {
-            while (ce == cudaSuccess && inflight < 2 && launched + check_every <= itermax) {
-                const int sl = (cur + inflight) & 1;
-                ce = cudaGraphLaunch(gexec, st);
-                if (ce == cudaSuccess) ce = cudaMemcpyAsync(hs + sl, w->state, sizeof(PcgState), cudaMemcpyDeviceToHost, st);
-                if (ce == cudaSuccess) ce = cudaEventRecord(ev[sl], st);
-                launched += check_every;
-                g_gs_launches += launches_per_graph;
-                ++inflight;
-            }
-            if (ce != cudaSuccess || inflight == 0) break;   // fewer than check_every iterations left: the loop below runs them
-            ce = cudaEventSynchronize(ev[cur]);
-            if (ce != cudaSuccess) break;
-            --inflight;
-            if (hs[cur].done || launched >= itermax) {
-                if (inflight) ce = cudaStreamSynchronize(st);   // the batch behind it: no-ops after `done`, or the last iterations
-                if (inflight && ce == cudaSuccess) cur ^= 1;
-                hs[0] = hs[cur];
-                finished = hs[0].done || launched >= itermax;
-                inflight = 0;
-                if (!finished) cur = 0;
-                continue;
-            }
-            cur ^= 1;
-        }
-        if (ev[0]) cudaEventDestroy(ev[0]);
-        if (ev[1]) cudaEventDestroy(ev[1]);
-        if (ce != cudaSuccess) { cudaGraphExecDestroy(gexec); gs_set_error("PCG graph loop: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
-    }
-    while (!finished) {
-        for (int k = 0; k < check_every && launched < itermax; ++k, ++launched)
-            if ((rc = iteration(st))) { if (gexec) cudaGraphExecDestroy(gexec); return rc; }
-        cudaError_t ce = cudaMemcpyAsync(w->host_state, w->state, sizeof(PcgState), cudaMemcpyDeviceToHost, st);
-        if (ce == cudaSuccess) ce = cudaStreamSynchronize(st);
-        if (ce != cudaSuccess) { if (gexec) cudaGraphExecDestroy(gexec); gs_set_error("PCG poll: %s", cudaGetErrorString(ce)); return GS_E_CUDA; }
-        finished = w->host_state->done || launched >= itermax;
-    }
-    if (gexec) cudaGraphExecDestroy(gexec);
-    const PcgState& s = *w->host_state;
-    if (n_iter_out) *n_iter_out = s.iter;
-    if (resid_out) *resid_out = s.d0 > 0.0 ? sqrt(s.rr / s.d0) : 0.0;
-    if (s.d0 > 0.0 && s.rr > s.eps2 * s.d0) {
-        gs_set_error("PCG stopped at iter_max = %d with |r|/|r0| = %.3e > eps = %.1e", itermax, sqrt(s.rr / s.d0), eps);
-        return GS_E_NOTCONVERGED;
-    }
-    return GS_OK;
+    return pcg_poll_loop(p, st, w->state, w->host_state, dist, eps, itermax, check_every, iteration, n_iter_out, resid_out);
 }
 
 extern "C" int gs_cr_pcg_pol(gs_plan* p, const double* dl_EE, const double* dl_BB, const double* bl,
@@ -842,6 +854,539 @@ extern "C" int gs_cr_rhs_pol(gs_plan* p, const double* dl_EE, const double* dl_B
     return GS_OK;
 }
 
+
+// ------------------------------------------------------------------ joint T/E/B system on a cut sky
+// qcinv's joint T+P filter (opfilt_tp upstream; not vendored, restated here): the (T, E, B) coefficients of every (l, m) are
+// coupled by the per-l prior C_l = [[TT, TE, 0], [TE, EE, 0], [0, 0, BB]], the data by two pixel weight maps:
+//   Q = C^-1 + B A^T N^-1 A B,   A B x = (alm2map_spin0(b x_T), alm2map_spin2(b x_E, b x_B)),  N^-1 = diag(N_T^-1, N_P^-1, N_P^-1)
+// The mat-vec is the spin-0 mat-vec of the TT solve on x_T with N_T^-1 followed by the spin-2 mat-vec of the E/B solve on
+// (x_E, x_B) with N_P^-1; the vector kernels take one coefficient of all three fields per thread, because T_j and E_j meet in
+// the 2x2 block of C^-1 and of the preconditioner.  Singular blocks follow safe_inv: a zero field inverts to zero, a block with
+// C^TE = 0 inverts field by field, and a TE block with zero determinant gives a zero C^-1 block.
+
+// Per-l tables of the joint solve: [ic_TT, ic_TE, ic_EE, ic_BB, M_TT, M_TE, M_EE, M_BB] for every l (8 doubles)
+#define TEB_TAB 8
+
+struct TebWs {
+    double *r[3], *p[3], *q[3];   // T, E, B
+    const unsigned short* lof;     // multipole of every coefficient (shared with gs_pcg_ws)
+    double* tab;                   // [L+1][TEB_TAB]
+    double* partials;              // SV_GRID * 2
+    PcgState* state;
+    PcgState* host_state;          // pinned, two slots
+};
+
+__device__ __forceinline__ double safe_rcp(double v) { return v != 0.0 ? 1.0 / v : 0.0; }
+
+// inverse of the symmetric 2x2 [[a, b], [b, d]] (safe_inv convention above)
+__device__ __forceinline__ void inv2x2(double a, double b, double d, double& i11, double& i12, double& i22)
+{
+    if (b == 0.0) { i11 = safe_rcp(a); i12 = 0.0; i22 = safe_rcp(d); return; }
+    const double det = a * d - b * b;
+    const double id = safe_rcp(det);
+    i11 = d * id; i12 = -b * id; i22 = a * id;
+}
+
+// C_l (l = 0: D_0 as it is, the convention of generate_var_cl / precond_kernel)
+__device__ __forceinline__ double dl_to_cl(const double* dl, int l)
+{
+    const double c = dl[l];
+    return l ? c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1)) : c;
+}
+
+// One thread per l: C_l^-1 and the diag_cl preconditioner M_l = (C_l^-1 + diag(b_l^2 nT, b_l^2 nP, b_l^2 nP))^-1,
+// nX = sum(N_X^-1) / (4 pi)
+__global__ void teb_tables_kernel(const double* __restrict__ dlTT, const double* __restrict__ dlTE, const double* __restrict__ dlEE,
+                                  const double* __restrict__ dlBB, const double* __restrict__ bl, double nT, double nP, int L,
+                                  double* __restrict__ tab)
+{
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    if (l > L) return;
+    double i11, i12, i22;
+    inv2x2(dl_to_cl(dlTT, l), dl_to_cl(dlTE, l), dl_to_cl(dlEE, l), i11, i12, i22);
+    const double ibb = safe_rcp(dl_to_cl(dlBB, l));
+    const double b2 = bl[l] * bl[l];
+    double m11, m12, m22;
+    inv2x2(i11 + b2 * nT, i12, i22 + b2 * nP, m11, m12, m22);
+    double* t = tab + (int64_t)l * TEB_TAB;
+    t[0] = i11; t[1] = i12; t[2] = i22; t[3] = ibb;
+    t[4] = m11; t[5] = m12; t[6] = m22; t[7] = safe_rcp(ibb + b2 * nP);
+}
+
+// the four entries of a per-l block (off 0: C^-1, off 4: M) through the read-only cache
+__device__ __forceinline__ double4 teb_blk(const double* tab, int l, int off)
+{
+    const double2 u = __ldg((const double2*)(tab + l * TEB_TAB + off));
+    const double2 v = __ldg((const double2*)(tab + l * TEB_TAB + off + 2));
+    return make_double4(u.x, u.y, v.x, v.y);
+}
+
+// y = q + K v with the per-l block K = (tt, te, ee, bb) on (T, E) and B
+__device__ __forceinline__ void teb_mul_add(const double4& k, double vT, double vE, double vB, double qT, double qE, double qB,
+                                            double& yT, double& yE, double& yB)
+{
+    yT = fma(k.x, vT, fma(k.y, vE, qT));
+    yE = fma(k.y, vT, fma(k.z, vE, qE));
+    yB = fma(k.w, vB, qB);
+}
+
+// Each thread takes TEB_U coefficients j (grid stride), T, E and B of each; all loads are issued before the first store.
+#define TEB_U 2
+
+// r = b - (q + C^-1 x)  (warm start; q = B A^T N^-1 A B x) or r = b ; p = M r ; delta = <r, M r> ; d0 = rr = <r, r>
+__global__ void __launch_bounds__(SV_NT)
+teb_init_kernel(TebWs W, const double* bT, const double* bE, const double* bB, const double* xT, const double* xE, const double* xB,
+                int have_q, int64_t n)
+{
+    double v[2] = {0.0, 0.0};
+    for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
+        const int l = W.lof[j];
+        double rT = bT[j], rE = bE[j], rB = bB[j];
+        if (have_q) {
+            double yT, yE, yB;
+            teb_mul_add(teb_blk(W.tab, l, 0), xT[j], xE[j], xB[j], W.q[0][j], W.q[1][j], W.q[2][j], yT, yE, yB);
+            rT -= yT; rE -= yE; rB -= yB;
+        }
+        double zT, zE, zB;
+        teb_mul_add(teb_blk(W.tab, l, 4), rT, rE, rB, 0.0, 0.0, 0.0, zT, zE, zB);
+        W.r[0][j] = rT; W.r[1][j] = rE; W.r[2][j] = rB;
+        W.p[0][j] = zT; W.p[1][j] = zE; W.p[2][j] = zB;
+        v[0] += rT * rT + rE * rE + rB * rB;
+        v[1] += rT * zT + rE * zE + rB * zB;
+    }
+    double tot[2];
+    if (grid_reduce<2>(v, W.partials, &W.state->counter, tot) && threadIdx.x == 0) fin_init(W.state, tot[0], tot[1]);
+}
+
+// pq = <p, q + C^-1 p> ; alpha = delta / pq.  q keeps B A^T N^-1 A B p: teb_update_kernel adds C^-1 p again on the fly (same
+// arithmetic), which saves the store of q and its second read.
+__global__ void __launch_bounds__(SV_NT) teb_apq_kernel(TebWs W, int64_t n)
+{
+    if (W.state->done) return;
+    double v[1] = {0.0};
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t j0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j0 < n; j0 += TEB_U * stride) {
+        double p[TEB_U][3], q[TEB_U][3];
+        double4 ic[TEB_U];
+#pragma unroll
+        for (int k = 0; k < TEB_U; ++k) {
+            const int64_t j = j0 + k * stride;
+            const bool ok = j < n;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) { p[k][c] = ok ? W.p[c][j] : 0.0; q[k][c] = ok ? W.q[c][j] : 0.0; }
+            ic[k] = ok ? teb_blk(W.tab, W.lof[j], 0) : make_double4(0.0, 0.0, 0.0, 0.0);
+        }
+#pragma unroll
+        for (int k = 0; k < TEB_U; ++k) {
+            double yT, yE, yB;
+            teb_mul_add(ic[k], p[k][0], p[k][1], p[k][2], q[k][0], q[k][1], q[k][2], yT, yE, yB);
+            v[0] += p[k][0] * yT + p[k][1] * yE + p[k][2] * yB;
+        }
+    }
+    double tot[1];
+    if (grid_reduce<1>(v, W.partials, &W.state->counter, tot) && threadIdx.x == 0) fin_apq(W.state, tot[0]);
+}
+
+// x += alpha p ; r -= alpha (q + C^-1 p) ; rr = <r, r> ; rz = <r, M r> ; beta = rz / delta ; convergence test
+__global__ void __launch_bounds__(SV_NT) teb_update_kernel(TebWs W, double* xT, double* xE, double* xB, int64_t n)
+{
+    if (W.state->done) return;
+    const double alpha = W.state->alpha;
+    double* const x[3] = {xT, xE, xB};
+    double v[2] = {0.0, 0.0};
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t j0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j0 < n; j0 += TEB_U * stride) {
+        double xv[TEB_U][3], p[TEB_U][3], q[TEB_U][3], r[TEB_U][3];
+        double4 ic[TEB_U], m[TEB_U];
+#pragma unroll
+        for (int k = 0; k < TEB_U; ++k) {
+            const int64_t j = j0 + k * stride;
+            const bool ok = j < n;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                xv[k][c] = ok ? x[c][j] : 0.0; p[k][c] = ok ? W.p[c][j] : 0.0;
+                q[k][c] = ok ? W.q[c][j] : 0.0; r[k][c] = ok ? W.r[c][j] : 0.0;
+            }
+            const int l = ok ? W.lof[j] : 0;
+            ic[k] = teb_blk(W.tab, l, 0);
+            m[k] = teb_blk(W.tab, l, 4);
+        }
+#pragma unroll
+        for (int k = 0; k < TEB_U; ++k) {
+            const int64_t j = j0 + k * stride;
+            if (j >= n) break;
+            double y[3], z[3];
+            teb_mul_add(ic[k], p[k][0], p[k][1], p[k][2], q[k][0], q[k][1], q[k][2], y[0], y[1], y[2]);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                x[c][j] = fma(alpha, p[k][c], xv[k][c]);
+                r[k][c] = fma(-alpha, y[c], r[k][c]);
+                W.r[c][j] = r[k][c];
+            }
+            teb_mul_add(m[k], r[k][0], r[k][1], r[k][2], 0.0, 0.0, 0.0, z[0], z[1], z[2]);
+            v[0] += r[k][0] * r[k][0] + r[k][1] * r[k][1] + r[k][2] * r[k][2];
+            v[1] += r[k][0] * z[0] + r[k][1] * z[1] + r[k][2] * z[2];
+        }
+    }
+    double tot[2];
+    if (grid_reduce<2>(v, W.partials, &W.state->counter, tot) && threadIdx.x == 0) fin_update(W.state, tot[0], tot[1]);
+}
+
+// p = M r + beta p
+__global__ void __launch_bounds__(SV_NT) teb_dir_kernel(TebWs W, int64_t n)
+{
+    if (W.state->done) return;
+    const double beta = W.state->beta;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t j0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j0 < n; j0 += TEB_U * stride) {
+        double p[TEB_U][3], r[TEB_U][3];
+        double4 m[TEB_U];
+#pragma unroll
+        for (int k = 0; k < TEB_U; ++k) {
+            const int64_t j = j0 + k * stride;
+            const bool ok = j < n;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) { p[k][c] = ok ? W.p[c][j] : 0.0; r[k][c] = ok ? W.r[c][j] : 0.0; }
+            m[k] = teb_blk(W.tab, ok ? W.lof[j] : 0, 4);
+        }
+#pragma unroll
+        for (int k = 0; k < TEB_U; ++k) {
+            const int64_t j = j0 + k * stride;
+            if (j >= n) break;
+            double bp[3];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) bp[c] = beta * p[k][c];
+            double o[3];
+            teb_mul_add(m[k], r[k][0], r[k][1], r[k][2], bp[0], bp[1], bp[2], o[0], o[1], o[2]);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) W.p[c][j] = o[c];
+        }
+    }
+}
+
+// y = q + C^-1 x  (gs_cr_apply_q_teb)
+__global__ void teb_add_cinv_kernel(TebWs W, const double* xT, const double* xE, const double* xB, double* yT, double* yE, double* yB,
+                                    int64_t n)
+{
+    for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
+        double a, b, c;
+        teb_mul_add(teb_blk(W.tab, W.lof[j], 0), xT[j], xE[j], xB[j], W.q[0][j], W.q[1][j], W.q[2][j], a, b, c);
+        yT[j] = a; yE[j] = b; yB[j] = c;
+    }
+}
+
+// rhs = resc rhs + F xi_alm + bdata, F = L^-T on (T, E) with C^TE block = L L^T (lower Cholesky), 1/sqrt(C^BB) on B:
+// F F^T = C^-1, so the prior term has covariance C^-1.  A field with C = 0 gets F = 0 (safe_inv, as mode 4 of gs_expand_per_l).
+__global__ void teb_rhs_combine_kernel(const unsigned short* __restrict__ lof, const double* __restrict__ dlTT,
+                                       const double* __restrict__ dlTE, const double* __restrict__ dlEE,
+                                       const double* __restrict__ dlBB, const double* xiT, const double* xiE, const double* xiB,
+                                       const double* bdT, const double* bdE, const double* bdB, double resc, double* rT, double* rE,
+                                       double* rB, int64_t n)
+{
+    for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
+        const int l = lof[j];
+        const double a = dl_to_cl(dlTT, l), b = dl_to_cl(dlTE, l), d = dl_to_cl(dlEE, l), e = dl_to_cl(dlBB, l);
+        double fTT, fTE, fEE;
+        if (b == 0.0) {
+            fTT = a != 0.0 ? sqrt(1.0 / a) : 0.0;
+            fTE = 0.0;
+            fEE = d != 0.0 ? sqrt(1.0 / d) : 0.0;
+        } else {
+            const double l11 = sqrt(a), l21 = b / l11, l22 = sqrt(d - l21 * l21);
+            fTT = 1.0 / l11;
+            fTE = -l21 / (l11 * l22);
+            fEE = 1.0 / l22;
+        }
+        const double fBB = e != 0.0 ? sqrt(1.0 / e) : 0.0;
+        const double xt = xiT[j], xe = xiE[j], xb = xiB[j];
+        rT[j] = fma(resc, rT[j], fma(fTT, xt, fma(fTE, xe, bdT[j])));
+        rE[j] = fma(resc, rE[j], fma(fEE, xe, bdE[j]));
+        rB[j] = fma(resc, rB[j], fma(fBB, xb, bdB[j]));
+    }
+}
+
+static TebWs* get_ws_teb(gs_plan* p)
+{
+    if (p->pcg_ws_teb) return (TebWs*)p->pcg_ws_teb;
+    gs_pcg_ws* base = get_ws(p);   // for its per-coefficient multipole index
+    if (!base) return nullptr;
+    TebWs* w = new TebWs();
+    const size_t n = (size_t)p->nreal_loc;
+    auto alloc = [&](double** q, size_t cnt) { void* d = nullptr; if (cudaMalloc(&d, cnt * sizeof(double)) != cudaSuccess) return false; p->owned.push_back(d); *q = (double*)d; return true; };
+    bool ok = true;
+    for (int c = 0; c < 3 && ok; ++c) ok = alloc(&w->r[c], n) && alloc(&w->p[c], n) && alloc(&w->q[c], n);
+    ok = ok && alloc(&w->tab, (size_t)TEB_TAB * (p->d.lmax + 1)) && alloc(&w->partials, SV_GRID * 2);
+    w->lof = base->lof;
+    void* d = nullptr;
+    ok = ok && cudaMalloc(&d, sizeof(PcgState)) == cudaSuccess;
+    if (ok) { p->owned.push_back(d); w->state = (PcgState*)d; }
+    ok = ok && cudaMallocHost((void**)&w->host_state, 2 * sizeof(PcgState)) == cudaSuccess;
+    if (!ok) { gs_set_error("joint T/E/B workspace allocation failed: %s", cudaGetErrorString(cudaGetLastError())); delete w; return nullptr; }
+    p->pcg_ws_teb = w;
+    return w;
+}
+
+static void teb_ws_free(gs_plan* p)
+{
+    TebWs* w = (TebWs*)p->pcg_ws_teb;
+    if (!w) return;
+    if (w->host_state) cudaFreeHost(w->host_state);   // the device buffers are in p->owned
+    delete w;
+    p->pcg_ws_teb = nullptr;
+}
+
+// Two weight maps, one set of plan-wide ring flags: the Legendre and ring launchers read act_ring / act_pairs / act_slot0 /
+// ring_wconst and the dynamic group order from the plan, and ring_apply_kernel takes the weight of a constant-weight ring from
+// ring_wconst, not from the map.  So the joint solve builds the flags of N_P^-1 in the plan's own set and those of N_T^-1 in
+// p->flags_T, once per call, and swaps the two sets while it enqueues the spin-0 half (the launch arguments are fixed at enqueue
+// time, graph capture included).  When both weight maps are the same array the plan's set serves both halves.
+static void swap_flags(gs_plan* p)
+{
+    RingFlags& f = p->flags_T;
+    std::swap(p->act_ring, f.act_ring);
+    std::swap(p->act_pairs, f.act_pairs);
+    std::swap(p->act_count, f.act_count);
+    std::swap(p->act_slot0, f.act_slot0);
+    std::swap(p->ring_wconst, f.ring_wconst);
+    std::swap(p->groups0_dyn, f.groups0_dyn);
+    std::swap(p->groups2_dyn, f.groups2_dyn);
+}
+
+static int alloc_flags_T(gs_plan* p)
+{
+    RingFlags& f = p->flags_T;
+    if (f.act_ring) return GS_OK;
+    const int L1 = p->d.lmax + 1;
+    auto alloc = [&](void** q, size_t bytes) { void* d = nullptr; if (cudaMalloc(&d, std::max<size_t>(16, bytes)) != cudaSuccess) return false; p->owned.push_back(d); *q = d; return true; };
+    bool ok = alloc((void**)&f.act_ring, (size_t)p->d.nring) && alloc((void**)&f.act_pairs, (size_t)p->d.npair * sizeof(int)) &&
+              alloc((void**)&f.act_count, sizeof(int)) && alloc((void**)&f.act_slot0, (size_t)2 * L1 * sizeof(int)) &&
+              alloc((void**)&f.ring_wconst, (size_t)p->d.nring * sizeof(double)) &&
+              alloc((void**)&f.groups0_dyn, (size_t)p->ngroups0 * sizeof(int2)) && alloc((void**)&f.groups2_dyn, (size_t)p->ngroups2 * sizeof(int2));
+    if (!ok) { memset(&f, 0, sizeof(f)); gs_set_error("ring flag allocation failed: %s", cudaGetErrorString(cudaGetLastError())); return GS_E_NOMEM; }
+    return GS_OK;
+}
+
+struct TebRings {   // scope guard: both flag sets of one joint call; the plan's own set afterwards as before
+    gs_plan* p;
+    ActiveRings act;
+    bool two;       // the spin-0 half runs on p->flags_T
+    TebRings(gs_plan* p_) : p(p_), act(p_), two(false) {}
+    int begin(const double* invT, const double* invP, cudaStream_t st)
+    {
+        int rc = act.begin(invP, st);
+        if (rc || !act.on || invT == invP) return rc;
+        if ((rc = alloc_flags_T(p))) return rc;
+        swap_flags(p);
+        rc = gs_active_rings_build(p, invT, st);
+        swap_flags(p);
+        two = rc == GS_OK;
+        return rc;
+    }
+};
+
+// q = B A^T N^-1 A B v on (T, E, B): the spin-0 half on N_T^-1, then the spin-2 half on N_P^-1
+static int teb_noise_op(gs_plan* p, TebRings& tr, const double* vT, const double* vE, const double* vB, const double* bl,
+                        const double* invT, const double* invP, double* qT, double* qE, double* qB, cudaStream_t st, const int* skip)
+{
+    if (tr.two) swap_flags(p);
+    int rc = apply_noise_op(p, vT, nullptr, bl, invT, qT, nullptr, st, skip, 0);
+    if (tr.two) swap_flags(p);
+    if (rc) return rc;
+    return apply_noise_op(p, vE, vB, bl, invP, qE, qB, st, skip, 2);
+}
+
+static int teb_unsharded(gs_plan* p, const char* who)
+{
+    if (p->world > 1) {
+        gs_set_error("%s: the joint T/E/B solve needs an unsharded plan (this plan is sharded over %d ranks)", who, p->world);
+        return GS_E_BADARG;
+    }
+    return GS_OK;
+}
+
+// Joint twin of gs_cr_pcg_pol / gs_cr_pcg_tt (include/gibbs_b200.h): one poll loop, one CUDA graph per solve
+extern "C" int gs_cr_pcg_teb(gs_plan* p, const double* dl_TT, const double* dl_TE, const double* dl_EE, const double* dl_BB,
+                             const double* bl, const double* inv_noise_T, const double* inv_noise_P, double ninvT_sum_over_4pi,
+                             double ninvP_sum_over_4pi, const double* rhs_T, const double* rhs_E, const double* rhs_B, double* x_T,
+                             double* x_E, double* x_B, int warm_start, double eps, int itermax, int check_every, int* n_iter_out,
+                             double* resid_out, void* stream)
+{
+    if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
+    GS_REQUIRE(dl_TT && dl_TE && dl_EE && dl_BB && bl && inv_noise_T && inv_noise_P && rhs_T && rhs_E && rhs_B && x_T && x_E && x_B,
+               "null pointer argument");
+    GS_REQUIRE(eps > 0.0 && itermax >= 0, "eps must be > 0 and itermax >= 0");
+    int rc;
+    if ((rc = teb_unsharded(p, __func__))) return rc;
+    GS_CHECK_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    TebWs* w = get_ws_teb(p);
+    if (!w) return GS_E_NOMEM;
+    const int L = p->d.lmax;
+    const int64_t n = p->nreal_loc;
+    if (check_every < 1) check_every = 8;
+    teb_tables_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_TT, dl_TE, dl_EE, dl_BB, bl, ninvT_sum_over_4pi, ninvP_sum_over_4pi, L, w->tab);
+    GS_CHECK_LAUNCH();
+    TebRings tr(p);
+    if ((rc = tr.begin(inv_noise_T, inv_noise_P, st))) return rc;
+
+    PcgState h;
+    memset(&h, 0, sizeof(h));
+    h.eps2 = eps * eps;
+    h.itermax = itermax;
+    *w->host_state = h;
+    GS_CHECK_CUDA(cudaMemcpyAsync(w->state, w->host_state, sizeof(PcgState), cudaMemcpyHostToDevice, st));
+    if (warm_start) {  // r0 = b - Q x0
+        if ((rc = teb_noise_op(p, tr, x_T, x_E, x_B, bl, inv_noise_T, inv_noise_P, w->q[0], w->q[1], w->q[2], st, nullptr))) return rc;
+    } else {
+        zero2_kernel<<<SV_GRID, SV_NT, 0, st>>>(x_T, x_E, n);
+        zero2_kernel<<<SV_GRID, SV_NT, 0, st>>>(x_B, x_B, n);
+    }
+    teb_init_kernel<<<SV_GRID, SV_NT, 0, st>>>(*w, rhs_T, rhs_E, rhs_B, x_T, x_E, x_B, warm_start ? 1 : 0, n);
+    GS_CHECK_LAUNCH();
+
+    const int* done = &w->state->done;
+    // one PCG iteration: the spin-0 and spin-2 mat-vecs, then 3 vector kernels; every argument is fixed for the whole solve
+    auto iteration = [&](cudaStream_t s) -> int {
+        int r;
+        if ((r = teb_noise_op(p, tr, w->p[0], w->p[1], w->p[2], bl, inv_noise_T, inv_noise_P, w->q[0], w->q[1], w->q[2], s, done))) return r;
+        teb_apq_kernel<<<SV_GRID, SV_NT, 0, s>>>(*w, n);
+        teb_update_kernel<<<SV_GRID, SV_NT, 0, s>>>(*w, x_T, x_E, x_B, n);
+        teb_dir_kernel<<<SV_GRID, SV_NT, 0, s>>>(*w, n);
+        GS_CHECK_LAUNCH();
+        g_gs_launches += 3;
+        return GS_OK;
+    };
+    return pcg_poll_loop(p, st, w->state, w->host_state, false, eps, itermax, check_every, iteration, n_iter_out, resid_out);
+}
+
+extern "C" int gs_cr_apply_q_teb(gs_plan* p, const double* dl_TT, const double* dl_TE, const double* dl_EE, const double* dl_BB,
+                                 const double* bl, const double* inv_noise_T, const double* inv_noise_P, const double* x_T,
+                                 const double* x_E, const double* x_B, double* y_T, double* y_E, double* y_B, void* stream)
+{
+    if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
+    GS_REQUIRE(dl_TT && dl_TE && dl_EE && dl_BB && bl && inv_noise_T && inv_noise_P && x_T && x_E && x_B && y_T && y_E && y_B,
+               "null pointer argument");
+    int rc;
+    if ((rc = teb_unsharded(p, __func__))) return rc;
+    GS_CHECK_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    TebWs* w = get_ws_teb(p);
+    if (!w) return GS_E_NOMEM;
+    const int L = p->d.lmax;
+    teb_tables_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_TT, dl_TE, dl_EE, dl_BB, bl, 0.0, 0.0, L, w->tab);
+    GS_CHECK_LAUNCH();
+    TebRings tr(p);
+    if ((rc = tr.begin(inv_noise_T, inv_noise_P, st))) return rc;
+    if ((rc = teb_noise_op(p, tr, x_T, x_E, x_B, bl, inv_noise_T, inv_noise_P, w->q[0], w->q[1], w->q[2], st, nullptr))) return rc;
+    teb_add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(*w, x_T, x_E, x_B, y_T, y_E, y_B, p->nreal_loc);
+    GS_CHECK_LAUNCH();
+    return GS_OK;
+}
+
+// b = B A^T N^-1 d + B (Npix/4pi) map2alm_{iter}(N^-1/2 xi_pix) + F xi_alm  (the two pixel terms as in gs_cr_rhs_tt / _pol)
+extern "C" int gs_cr_rhs_teb(gs_plan* p, const double* dl_TT, const double* dl_TE, const double* dl_EE, const double* dl_BB,
+                             const double* bl, const double* inv_noise_T, const double* sqrt_inv_noise_T, const double* inv_noise_P,
+                             const double* sqrt_inv_noise_P, const double* bdata_T, const double* bdata_E, const double* bdata_B,
+                             const double* d_I, const double* d_Q, const double* d_U, const double* xi_I, const double* xi_Q,
+                             const double* xi_U, const double* xi_T, const double* xi_E, const double* xi_B, int fluct_iter,
+                             double* rhs_T, double* rhs_E, double* rhs_B, void* stream)
+{
+    if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
+    GS_REQUIRE(dl_TT && dl_TE && dl_EE && dl_BB && bl && inv_noise_T && sqrt_inv_noise_T && inv_noise_P && sqrt_inv_noise_P && xi_I &&
+               xi_Q && xi_U && xi_T && xi_E && xi_B && rhs_T && rhs_E && rhs_B, "null pointer argument");
+    GS_REQUIRE((bdata_T && bdata_E && bdata_B) || (d_I && d_Q && d_U), "need either the precomputed data terms or the data maps");
+    GS_REQUIRE(fluct_iter >= 0, "fluct_iter must be >= 0");
+    int rc;
+    if ((rc = teb_unsharded(p, __func__))) return rc;
+    GS_CHECK_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    TebWs* w = get_ws_teb(p);
+    if (!w) return GS_E_NOMEM;
+    if ((rc = gs_map2alm_spin0(p, xi_I, sqrt_inv_noise_T, fluct_iter, 0, bl, rhs_T, GS_ALM_REAL, stream))) return rc;
+    if ((rc = gs_map2alm_spin2(p, xi_Q, xi_U, sqrt_inv_noise_P, fluct_iter, 0, bl, rhs_E, rhs_B, GS_ALM_REAL, stream))) return rc;
+    const double* bd[3] = {bdata_T, bdata_E, bdata_B};
+    if (!bdata_T || !bdata_E || !bdata_B) {   // data terms into the r vectors of the workspace
+        if ((rc = gs_map2alm_spin0(p, d_I, inv_noise_T, 0, 1, bl, w->r[0], GS_ALM_REAL, stream))) return rc;
+        if ((rc = gs_map2alm_spin2(p, d_Q, d_U, inv_noise_P, 0, 1, bl, w->r[1], w->r[2], GS_ALM_REAL, stream))) return rc;
+        for (int c = 0; c < 3; ++c) bd[c] = w->r[c];
+    }
+    const double resc = (double)p->d.npix / (4.0 * 3.14159265358979323846);
+    teb_rhs_combine_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->lof, dl_TT, dl_TE, dl_EE, dl_BB, xi_T, xi_E, xi_B, bd[0], bd[1], bd[2], resc,
+                                                      rhs_T, rhs_E, rhs_B, p->nreal_loc);
+    GS_CHECK_LAUNCH();
+    return GS_OK;
+}
+
+// Times the parts of one joint PCG iteration with CUDA events on `stream` (average of nrep, after one warm-up): ms_out[0] the
+// spin-0 half of the mat-vec (N_T^-1), [1] the spin-2 half (N_P^-1), [2..4] the vector kernels teb_apq / teb_update / teb_dir on
+// the joint workspace, zero-filled, with the analysis workspace overwritten before each (the arrays come from HBM, not L2).
+// The vector kernels' reductions go to a scratch state, so no solver state changes.
+extern "C" int gs_profile_matvec_teb(gs_plan* p, const double* bl, const double* inv_noise_T, const double* inv_noise_P, int nrep,
+                                     float* ms_out, void* stream)
+{
+    if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
+    GS_REQUIRE(bl && inv_noise_T && inv_noise_P && ms_out && nrep >= 1, "bad arguments");
+    int rc;
+    if ((rc = teb_unsharded(p, __func__))) return rc;
+    GS_CHECK_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    TebWs* w = get_ws_teb(p);
+    if (!w) return GS_E_NOMEM;
+    const int64_t n = p->nreal_loc;
+    for (int c = 0; c < 3; ++c) {
+        double* arrs[3] = {w->r[c], w->p[c], w->q[c]};
+        for (double* a : arrs) GS_CHECK_CUDA(cudaMemsetAsync(a, 0, (size_t)n * sizeof(double), st));
+    }
+    GS_CHECK_CUDA(cudaMemsetAsync(w->tab, 0, (size_t)TEB_TAB * (p->d.lmax + 1) * sizeof(double), st));
+    double* x[3] = {p->almE_tmp, p->almB_tmp, p->almE_tmp2};
+    for (double* a : x) GS_CHECK_CUDA(cudaMemsetAsync(a, 0, (size_t)n * sizeof(double), st));
+    PcgState* scratch = nullptr;
+    GS_CHECK_CUDA(cudaMalloc(&scratch, sizeof(PcgState)));
+    GS_CHECK_CUDA(cudaMemsetAsync(scratch, 0, sizeof(PcgState), st));
+    TebWs v = *w;
+    v.state = scratch;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    double acc[5] = {0, 0, 0, 0, 0};
+    const size_t flush_bytes = (size_t)p->anal_chunks * (size_t)p->d.nalm * 4 * sizeof(double);
+    {
+        TebRings tr(p);
+        rc = tr.begin(inv_noise_T, inv_noise_P, st);
+        if (rc == GS_OK && (cudaEventCreate(&e0) != cudaSuccess || cudaEventCreate(&e1) != cudaSuccess)) rc = GS_E_CUDA;
+        for (int k = 0; k < 5 && rc == GS_OK; ++k) {
+            for (int rep = -1; rep < nrep && rc == GS_OK; ++rep) {
+                // the flush, and a fresh scratch state: a reduction on zero vectors marks it converged, which would turn
+                // every later launch into an early exit
+                if (k >= 2 && (cudaMemsetAsync(p->partial, 0, flush_bytes, st) != cudaSuccess ||
+                               cudaMemsetAsync(scratch, 0, sizeof(PcgState), st) != cudaSuccess)) { rc = GS_E_CUDA; break; }
+                cudaEventRecord(e0, st);
+                if (k == 0) {
+                    if (tr.two) swap_flags(p);
+                    rc = apply_noise_op(p, w->p[0], nullptr, bl, inv_noise_T, w->q[0], nullptr, st, nullptr, 0);
+                    if (tr.two) swap_flags(p);
+                } else if (k == 1) {
+                    rc = apply_noise_op(p, w->p[1], w->p[2], bl, inv_noise_P, w->q[1], w->q[2], st, nullptr, 2);
+                } else if (k == 2) {
+                    teb_apq_kernel<<<SV_GRID, SV_NT, 0, st>>>(v, n);
+                } else if (k == 3) {
+                    teb_update_kernel<<<SV_GRID, SV_NT, 0, st>>>(v, x[0], x[1], x[2], n);
+                } else {
+                    teb_dir_kernel<<<SV_GRID, SV_NT, 0, st>>>(v, n);
+                }
+                cudaEventRecord(e1, st);
+                if (cudaEventSynchronize(e1) != cudaSuccess) { rc = GS_E_CUDA; break; }
+                float ms = 0;
+                cudaEventElapsedTime(&ms, e0, e1);
+                if (rep >= 0) acc[k] += ms;
+            }
+        }
+    }
+    if (rc == GS_E_CUDA) gs_set_error("gs_profile_matvec_teb: %s", cudaGetErrorString(cudaGetLastError()));
+    for (int k = 0; k < 5; ++k) ms_out[k] = (float)(acc[k] / nrep);
+    if (e0) cudaEventDestroy(e0);
+    if (e1) cudaEventDestroy(e1);
+    cudaFree(scratch);
+    return rc;
+}
 
 // ------------------------------------------------------------------ measurement helpers (bench.py)
 long long g_gs_launches = 0;

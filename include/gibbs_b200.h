@@ -194,6 +194,37 @@ int gs_cr_pcg_tt(gs_plan* plan, const double* dl_TT, const double* bl, const dou
 int gs_cr_apply_q_tt(gs_plan* plan, const double* dl_TT, const double* bl, const double* inv_noise,
                      const double* x, double* y, void* stream);
 
+/* Joint T/E/B twins: T and E coupled through C^TE on a cut sky (qcinv's joint T+P filter, opfilt_tp upstream, not vendored;
+ * the reference only has the full-sky per-coefficient 3x3 solve, utils.compute_inverse_and_cholesky + utils.matrix_product, see
+ * gs_inv_chol_3x3).  Real layout, one beam bl for the three fields (the reference applies the temperature beam to E/B):
+ *   Q = C^-1 + B A^T N^-1 A B,  C_l = [[TT, TE, 0], [TE, EE, 0], [0, 0, BB]] on (T_j, E_j, B_j) of every coefficient j,
+ *   A B x = (alm2map_spin0(b x_T), alm2map_spin2(b x_E, b x_B)),  N^-1 = diag(inv_noise_T, inv_noise_P, inv_noise_P) on (I, Q, U).
+ * inv_noise_X = mask_X / noise_X (Npix each; the T and P masks may differ), dl_* unbinned D_l (L+1).
+ * Right-hand side  b = B A^T N^-1 d + B (Npix/4pi) map2alm_{iter=fluct_iter}(N^-1/2 xi_pix) + F xi_alm  with F = L^-T on (T, E),
+ * C^{TE block}_l = L L^T the lower Cholesky factor, and F = 1/sqrt(C^BB) on B, so F F^T = C^-1: with fluct_iter = 0 the
+ * right-hand side has covariance Q and x = Q^-1 b is an exact draw of s | C, d.  RNG order: xi_I, xi_Q, xi_U [Npix each], then
+ * xi_T, xi_E, xi_B [(L+1)^2 each] (pixel draws first, as in the polarised reference, CenteredGibbs.py:472-479).  The data terms
+ * B A^T N^-1 d are passed precomputed (bdata_T/E/B) or computed from d_I, d_Q, d_U.
+ * PCG: preconditioner diag_cl per l, M_l = (C_l^-1 + diag(b_l^2 nT, b_l^2 nP, b_l^2 nP))^-1 with nX = sum(inv_noise_X)/(4 pi)
+ * (a 2x2 inverse on (T, E), a scalar on B); stop when <r,r> <= eps^2 <r0,r0> with the sums over all three fields (qcinv
+ * monitor_basic).  Singular blocks follow safe_inv: at l < 2 (D_l = 0) C^-1 = 0, a block with C^TE = 0 inverts field by
+ * field; where C^TE != 0 the TE block must be positive definite.  warm_start, check_every, the outputs and GS_E_NOTCONVERGED as
+ * in gs_cr_pcg_pol.  Unsharded plans only (GS_E_BADARG otherwise). */
+int gs_cr_rhs_teb(gs_plan* plan, const double* dl_TT, const double* dl_TE, const double* dl_EE, const double* dl_BB,
+                  const double* bl, const double* inv_noise_T, const double* sqrt_inv_noise_T, const double* inv_noise_P,
+                  const double* sqrt_inv_noise_P, const double* bdata_T, const double* bdata_E, const double* bdata_B,
+                  const double* d_I, const double* d_Q, const double* d_U, const double* xi_I, const double* xi_Q,
+                  const double* xi_U, const double* xi_T, const double* xi_E, const double* xi_B, int fluct_iter,
+                  double* rhs_T, double* rhs_E, double* rhs_B, void* stream);
+int gs_cr_pcg_teb(gs_plan* plan, const double* dl_TT, const double* dl_TE, const double* dl_EE, const double* dl_BB,
+                  const double* bl, const double* inv_noise_T, const double* inv_noise_P, double ninvT_sum_over_4pi,
+                  double ninvP_sum_over_4pi, const double* rhs_T, const double* rhs_E, const double* rhs_B, double* x_T,
+                  double* x_E, double* x_B, int warm_start, double eps, int itermax, int check_every, int* n_iter_out,
+                  double* resid_out, void* stream);
+int gs_cr_apply_q_teb(gs_plan* plan, const double* dl_TT, const double* dl_TE, const double* dl_EE, const double* dl_BB,
+                      const double* bl, const double* inv_noise_T, const double* inv_noise_P, const double* x_T,
+                      const double* x_E, const double* x_B, double* y_T, double* y_E, double* y_B, void* stream);
+
 /* Diagonal draw for full sky + isotropic noise, one field, real layout, w = Npix/(noise 4 pi):
  *   mode 0 centred     (CenteredGibbs.py:317-353): sigma = 1/(w b^2 + 1/C), s = sigma b w d + xi sqrt(sigma)
  *   mode 1 non-centred (NonCenteredGibbs.py:138-176, all_sph): sigma = 1/(1 + b^2 C w),
@@ -431,6 +462,13 @@ int gs_profile_matvec_batch(gs_plan* plan, int n_chain, const double* x_E, const
  * beta p  (4 arrays); n = (lmax+1)^2, 2 fields for spin 2.  Every launch is timed alone after the plan's analysis workspace
  * (larger than L2 at NSIDE >= 512) has been overwritten.  No solver state is changed.  Synchronous. */
 int gs_profile_pcg_vectors(gs_plan* plan, int spin, int nrep, float* ms_out, void* stream);
+/* The parts of one gs_cr_pcg_teb iteration, average ms over nrep (CUDA events on `stream`, one warm-up): ms_out[0] the spin-0
+ * mat-vec on inv_noise_T, [1] the spin-2 mat-vec on inv_noise_P (each with its own ring flags, as in the solve), [2] <p, Q p>
+ * (6 arrays of 8 (L+1)^2 bytes), [3] the x / r update with <r,r>, <r,M r> (18 arrays), [4] p = M r + beta p (9 arrays), the
+ * vector kernels on the zero-filled joint workspace after the analysis workspace has been overwritten.  Unsharded plans;
+ * no solver state changes.  Synchronous. */
+int gs_profile_matvec_teb(gs_plan* plan, const double* bl, const double* inv_noise_T, const double* inv_noise_P, int nrep,
+                          float* ms_out, void* stream);
 /* Ring stage of the PCG mat-vec (opfilt_pp.fwd_op's alm2map_spin -> N^-1 -> map2alm_spin, CenteredGibbs.py:629,653):
  * fused != 0 (default): one kernel per mat-vec keeps each ring's pixels in shared memory; 0: ring synthesis to the
  * plan's scratch maps, then weighted ring analysis.  Same result to rounding.  Returns the previous setting. */
