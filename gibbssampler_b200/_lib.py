@@ -115,7 +115,6 @@ SIGNATURES = {
     "gs_set_ring_fused": (_i, [_i]),
     "gs_set_ring_skip": (_i, [_i]),
     "gs_set_ring_const": (_i, [_i]),
-    "gs_set_fuse_apq": (_i, [_i]),
     "gs_constant_rings": (_i, [_vp, C.POINTER(_i)]),
     "gs_active_ring_pairs": (_i, [_vp, C.POINTER(_i), C.POINTER(_i)]),
 }

@@ -325,7 +325,7 @@ extern "C" int gs_map2alm_batch(gs_plan* p, int spin, int n_chain, const double*
         double* e = almE + c * alm_stride;
         double* b = spin ? almB + c * alm_stride : nullptr;
         if ((rc = gs_ring_anal(p, spin, q, u, pixw, st, nullptr, nc, map_stride))) return rc;
-        if ((rc = gs_leg_anal(p, spin, e, b, layout, fl, scale, 0, st, nullptr, nullptr, nc, alm_stride))) return rc;
+        if ((rc = gs_leg_anal(p, spin, e, b, layout, fl, scale, 0, st, nullptr, nc, alm_stride))) return rc;
     }
     return GS_OK;
 }

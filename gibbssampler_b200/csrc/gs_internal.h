@@ -212,19 +212,6 @@ extern int g_gs_ring_fused;       // 1: the PCG mat-vec runs its ring stage as o
 extern long long g_gs_launches;  // kernels launched by this library (bench.py's gpu_launches)
 static inline int64_t gs_nalm(int lmax) { return (int64_t)(lmax + 1) * (lmax + 2) / 2; }
 
-// Fusion of the PCG's  q += C^-1 p ; <p, q>  into the last kernel of the analysis (unsharded plans, real layout):
-// ic* are per-l inverse spectra, the dot product is reduced in a fixed order (one partial per block, the last block to
-// finish sums them) and left in out[0].
-struct FinishFuse {
-    const double* pE;
-    const double* pB;     // unused for spin 0
-    const double* icE;    // [lmax+1]
-    const double* icB;
-    double* partials;     // one per block of the finish grid: ((lmax + 256) / 256) * (lmax + 1)
-    unsigned* counter;    // zero on entry, zero again on exit
-    double* out;
-};
-
 // legendre.cu
 // `skip` (nullable device int): when *skip != 0 the kernels return immediately (device-side early exit)
 // nc = 2: chain batch (two right-hand sides share one recurrence; chain c at alm + c alm_stride, spectra at p->Fm + c gs_fm_stride(p));
@@ -232,8 +219,7 @@ struct FinishFuse {
 int gs_leg_synth(gs_plan* p, int spin, const double* almE, const double* almB, int layout, const double* fl,
                  cudaStream_t st, const int* skip = nullptr, const double* flB = nullptr, int nc = 1, int64_t alm_stride = 0);
 int gs_leg_anal(gs_plan* p, int spin, double* almE, double* almB, int layout, const double* fl, double scale,
-                int accumulate, cudaStream_t st, const int* skip = nullptr, const FinishFuse* fuse = nullptr, int nc = 1,
-                int64_t alm_stride = 0);
+                int accumulate, cudaStream_t st, const int* skip = nullptr, int nc = 1, int64_t alm_stride = 0);
 int64_t gs_fm_stride(const gs_plan* p);            // double2 entries of one chain's ring spectra
 int64_t gs_part_stride(const gs_plan* p, int nc);  // doubles of one chain's analysis partial sums
 int gs_active_rings_build(gs_plan* p, const double* pixw, cudaStream_t st);

@@ -1160,92 +1160,6 @@ __global__ void leg_finish_kernel(PlanDev P, const double* __restrict__ partial,
     }
 }
 
-// leg_finish_kernel for the PCG mat-vec (unsharded, real layout, scale 1, no accumulation) with the solver's next step fused:
-// q = B A^T N^-1 A B p (from the partials) + C^-1 p, and the dot product <p, q> (see FinishFuse).
-template <int SPIN>
-__global__ void __launch_bounds__(256)
-leg_finish_apq_kernel(PlanDev P, const double* __restrict__ partial, double* __restrict__ qE, double* __restrict__ qB,
-                      const double* __restrict__ fl, const int* __restrict__ skip, const int* __restrict__ pcount,
-                      const int* __restrict__ slot0, int chunk_pairs, FinishFuse ff)
-{
-    if (skip && *skip) return;
-    constexpr int NV = SPIN ? 4 : 2;
-    __shared__ double sm[8];
-    __shared__ bool last;
-    const int L = P.lmax, m = blockIdx.y, tid = threadIdx.x;
-    const int nact = (pcount ? *pcount : P.npair) - slot0[m];
-    const int nchunk = nact > 0 ? (nact + chunk_pairs - 1) / chunk_pairs : 0;
-    const int l = m + blockIdx.x * blockDim.x + tid;
-    double dot = 0.0;
-    if (l <= L) {
-        const int64_t base = (int64_t)m * (2 * L + 1 - m) / 2, id = base + l;
-        double v[NV];
-#pragma unroll
-        for (int c = 0; c < NV; ++c) v[c] = 0.0;
-        if (l >= SPIN) {
-            for (int k = 0; k < nchunk; ++k) {
-                const double* q = partial + ((int64_t)k * P.nalm + id) * NV;
-#pragma unroll
-                for (int c = 0; c < NV; ++c) v[c] += q[c];
-            }
-            if (SPIN) {  // E.re = Y1+Y2, E.im = Y3+Y4, B.re = Y3-Y4, B.im = Y2-Y1
-                const double y1 = v[0], y2 = v[1], y3 = v[2], y4 = v[3];
-                v[0] = y1 + y2; v[1] = y3 + y4; v[2] = y3 - y4; v[3] = y2 - y1;
-            }
-            double post = SPIN ? -0.5 * P.alpha2[id] : P.alpha0[id];
-            if (fl) post *= fl[l];
-            if (m > 0) post *= 1.41421356237309504880;
-#pragma unroll
-            for (int c = 0; c < NV; ++c) v[c] *= post;
-        }
-        const double icE = ff.icE[l], icB = SPIN ? ff.icB[l] : 0.0;
-        if (m == 0) {
-            const double pe = ff.pE[l], qe = fma(icE, pe, v[0]);
-            qE[l] = qe;
-            dot = pe * qe;
-            if (SPIN) { const double pb = ff.pB[l], qb = fma(icB, pb, v[2]); qB[l] = qb; dot = fma(pb, qb, dot); }
-        } else {
-            const int64_t off = 2 * id - (L + 1);
-            const double p0 = ff.pE[off], p1 = ff.pE[off + 1];
-            const double q0 = fma(icE, p0, v[0]), q1 = fma(icE, p1, v[1]);
-            qE[off] = q0; qE[off + 1] = q1;
-            dot = fma(p1, q1, p0 * q0);
-            if (SPIN) {
-                const double b0 = ff.pB[off], b1 = ff.pB[off + 1];
-                const double r0 = fma(icB, b0, v[2]), r1 = fma(icB, b1, v[3]);
-                qB[off] = r0; qB[off + 1] = r1;
-                dot = fma(b0, r0, fma(b1, r1, dot));
-            }
-        }
-    }
-    // block sum, then the last block to finish adds the per-block partials in a fixed order
-    for (int o = 16; o; o >>= 1) dot += __shfl_xor_sync(FULL, dot, o);
-    if ((tid & 31) == 0) sm[tid >> 5] = dot;
-    __syncthreads();
-    const unsigned nblocks = gridDim.x * gridDim.y, bid = blockIdx.y * gridDim.x + blockIdx.x;
-    if (tid == 0) {
-        double s = 0.0;
-        for (int i = 0; i < 8; ++i) s += sm[i];
-        ff.partials[bid] = s;
-        __threadfence();
-        last = atomicInc(ff.counter, nblocks - 1) == nblocks - 1;
-    }
-    __syncthreads();
-    if (!last) return;
-    __threadfence();
-    double s = 0.0;
-    for (unsigned i = tid; i < nblocks; i += blockDim.x) s += ff.partials[i];
-    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(FULL, s, o);
-    __syncthreads();
-    if ((tid & 31) == 0) sm[tid >> 5] = s;
-    __syncthreads();
-    if (tid == 0) {
-        double t = 0.0;
-        for (int i = 0; i < 8; ++i) t += sm[i];
-        ff.out[0] = t;
-    }
-}
-
 // ------------------------------------------------------------------ active rings of a pixel-weight map
 // In the PCG mat-vec A^T N^-1 A the rings whose N^-1 vanishes identically (inside a galactic mask) contribute exactly
 // nothing: their synthesis is multiplied by zero and their analysis input is zero.  gs_active_rings_build marks the rings
@@ -1436,7 +1350,7 @@ int gs_leg_prepare(gs_plan* p)
 }
 
 int gs_leg_anal(gs_plan* p, int spin, double* almE, double* almB, int layout, const double* fl, double scale,
-                int accumulate, cudaStream_t st, const int* skip, const FinishFuse* fuse, int nc, int64_t alm_stride)
+                int accumulate, cudaStream_t st, const int* skip, int nc, int64_t alm_stride)
 {
     const bool sh = p->world > 1;
     if (sh && layout != GS_ALM_REAL) { gs_set_error("sharded plans take the (local) real alm layout only"); return GS_E_BADARG; }
@@ -1454,22 +1368,12 @@ int gs_leg_anal(gs_plan* p, int spin, double* almE, double* almB, int layout, co
     const int cp = LEG_NT * (nc > 1 ? LEG_RA2 : LEG_RA);   // ring pairs per chunk
 
     if (nc == 2) {
-        if (fuse) { gs_set_error("gs_leg_anal: the fused finish takes one right-hand side"); return GS_E_BADARG; }
         if (spin == 0) {
             if ((rc = launch_anal<0, LEG_RA2, false, 2>(p, grid, st, skip, plist, pcount, slot0, fs, ps))) return rc;
             leg_finish_kernel<0, false><<<fgrid, 256, 0, st>>>(p->d, p->partial, nchunk, almE, almB, layout, fl, scale, accumulate, skip, pcount, slot0, cp, ps, alm_stride);
         } else {
             if ((rc = launch_anal<2, LEG_RA2, false, 2>(p, grid, st, skip, plist, pcount, slot0, fs, ps))) return rc;
             leg_finish_kernel<2, false><<<fgrid, 256, 0, st>>>(p->d, p->partial, nchunk, almE, almB, layout, fl, scale, accumulate, skip, pcount, slot0, cp, ps, alm_stride);
-        }
-    } else if (fuse) {
-        if (sh || layout != GS_ALM_REAL || accumulate || scale != 1.0) { gs_set_error("gs_leg_anal: fused finish needs an unsharded real-layout plain analysis"); return GS_E_BADARG; }
-        if (spin == 0) {
-            if ((rc = launch_anal<0, LEG_RA, false, 1>(p, grid, st, skip, plist, pcount, slot0, 0, 0))) return rc;
-            leg_finish_apq_kernel<0><<<dim3(fgrid.x, fgrid.y), 256, 0, st>>>(p->d, p->partial, almE, almB, fl, skip, pcount, slot0, cp, *fuse);
-        } else {
-            if ((rc = launch_anal<2, LEG_RA, false, 1>(p, grid, st, skip, plist, pcount, slot0, 0, 0))) return rc;
-            leg_finish_apq_kernel<2><<<dim3(fgrid.x, fgrid.y), 256, 0, st>>>(p->d, p->partial, almE, almB, fl, skip, pcount, slot0, cp, *fuse);
         }
     } else if (!sh) {
         if (spin == 0) {

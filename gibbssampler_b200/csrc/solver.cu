@@ -11,7 +11,6 @@
 // so alpha/beta and the convergence flag never travel to the host inside the loop; once the flag
 // is set every later kernel (SHT stages included) returns immediately.
 #include <math.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
@@ -29,15 +28,13 @@ struct PcgState {
 };
 
 struct gs_pcg_ws {
-    double *r[2], *p[2], *q[2], *invc[2], *pre[2];
+    double *r[2], *p[2], *q[2];
     // r02: the solver regenerates C^-1_l and the preconditioner M_l per coefficient from per-l tables (L1-resident) and a 2-byte
     // multipole index per coefficient instead of streaming two expanded 8-byte arrays: 12 instead of 15 array passes per iteration
     const unsigned short* lof;   // [n] multipole of every coefficient of the (local) real layout
-    const double* ic_l[2];       // [L+1] 1 / C_l (E, B)
-    const double* pre_l[2];      // [L+1] M_l
+    double* ic_l[2];             // [L+1] 1 / C_l (E, B), filled by precond_kernel at the start of a solve
+    double* pre_l[2];            // [L+1] M_l
     double* partials;  // SV_GRID * 2
-    double* fuse_partials;  // per-block partials of the fused analysis-finish + <p, q> kernel (unsharded plans)
-    double* fuse_out;       // its result
     double* red;       // sharded plans: local sums in, all-reduced sums out (NULL on one GPU)
     PcgState* state;
     PcgState* host_state;  // pinned, two slots (the graph path of a solve keeps two polls in flight)
@@ -128,12 +125,6 @@ __device__ __forceinline__ void fin_update(PcgState* s, double rr, double rz)
     s->iter += 1;
     // qcinv cd_monitors.monitor_basic: stop when <r,r> <= eps^2 <r0,r0> or iter >= iter_max
     if (rr <= s->eps2 * s->d0 || s->iter >= s->itermax) s->done = 1;
-}
-// after the fused analysis-finish kernel: alpha = delta / <p, q>
-__global__ void pcg_apq_scalar_kernel(gs_pcg_ws W)
-{
-    if (W.state->done) return;
-    fin_apq(W.state, W.fuse_out[0]);
 }
 __global__ void pcg_scalar_kernel(gs_pcg_ws W, int stage)
 {
@@ -280,11 +271,12 @@ __global__ void zero2_kernel(double* a, double* b, int64_t n)
     }
 }
 
-// out = a + x * y   (per coefficient, real layout)
-__global__ void axy_kernel(const double* a, const double* __restrict__ x, const double* __restrict__ y, double* out, int64_t n)
+// y = q + C^-1 x with C^-1 from the per-l table (warm start of a solve, gs_cr_apply_q_*); y may be q
+__global__ void add_cinv_kernel(const double* q, const double* __restrict__ ic_l, const unsigned short* __restrict__ lof,
+                                const double* __restrict__ x, double* y, int64_t n)
 {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        out[i] = fma(x[i], y[i], a ? a[i] : 0.0);
+        y[i] = fma(ic_l[lof[i]], x[i], q[i]);
 }
 
 __global__ void scale_map_kernel(const double* __restrict__ a, const double* __restrict__ w, double* __restrict__ out, int64_t n)
@@ -317,30 +309,42 @@ static bool build_lof(gs_plan* p, const unsigned short** out)
 }
 
 // ------------------------------------------------------------------ workspace
-// The workspace belongs to the plan (gs_plan::pcg_ws): created on the first solve, released by gs_plan_destroy through
-// gs_pcg_ws_free.  A plan is used by one host thread at a time (include/gibbs_b200.h), so no lock is taken.
+// The workspaces belong to the plan (gs_plan::pcg_ws, pcg_ws_batch, pcg_ws_teb): created on the first solve, released by
+// gs_plan_destroy, which frees the device buffers recorded in p->owned and calls gs_pcg_ws_free for the rest.  A plan is used by
+// one host thread at a time (include/gibbs_b200.h), so no lock is taken.
+static bool alloc_owned(gs_plan* p, double** q, size_t cnt)
+{
+    void* d = nullptr;
+    if (cudaMalloc(&d, cnt * sizeof(double)) != cudaSuccess) return false;
+    p->owned.push_back(d);
+    *q = (double*)d;
+    return true;
+}
+
+// the solver state on the device (in p->owned) and its pinned host copy with two slots (the graph path of a solve keeps two
+// polls in flight), released by the workspace's free function
+static bool alloc_state(gs_plan* p, PcgState** state, PcgState** host_state)
+{
+    void* d = nullptr;
+    if (cudaMalloc(&d, sizeof(PcgState)) != cudaSuccess) return false;
+    p->owned.push_back(d);
+    *state = (PcgState*)d;
+    return cudaMallocHost((void**)host_state, 2 * sizeof(PcgState)) == cudaSuccess;
+}
+
 static gs_pcg_ws* get_ws(gs_plan* p)
 {
     if (p->pcg_ws) return (gs_pcg_ws*)p->pcg_ws;
     gs_pcg_ws* w = new gs_pcg_ws();
     const size_t n = (size_t)p->nreal_loc;
     w->red = p->world > 1 ? p->red_loc : nullptr;
-    auto alloc = [&](double** q, size_t cnt) { void* d = nullptr; if (cudaMalloc(&d, cnt * sizeof(double)) != cudaSuccess) return false; p->owned.push_back(d); *q = (double*)d; return true; };
     bool ok = true;
-    for (int c = 0; c < 2 && ok; ++c) ok = alloc(&w->r[c], n) && alloc(&w->p[c], n) && alloc(&w->q[c], n) && alloc(&w->invc[c], n) && alloc(&w->pre[c], n);
-    ok = ok && alloc(&w->partials, SV_GRID * 2 + 4 * (size_t)(p->d.lmax + 1));
-    ok = ok && build_lof(p, &w->lof);
-    if (ok) {
-        double* tl = w->partials + SV_GRID * 2;   // [icE | preE | icB | preB], filled by precond_kernel at the start of a solve
-        const int L1 = p->d.lmax + 1;
-        w->ic_l[0] = tl; w->pre_l[0] = tl + L1; w->ic_l[1] = tl + 2 * L1; w->pre_l[1] = tl + 3 * L1;
-    }
-    ok = ok && alloc(&w->fuse_partials, (size_t)((p->d.lmax + 256) / 256) * (p->d.lmax + 1));
-    ok = ok && alloc(&w->fuse_out, 4);
-    void* d = nullptr;
-    ok = ok && cudaMalloc(&d, sizeof(PcgState)) == cudaSuccess;
-    if (ok) { p->owned.push_back(d); w->state = (PcgState*)d; }
-    ok = ok && cudaMallocHost((void**)&w->host_state, 2 * sizeof(PcgState)) == cudaSuccess;
+    const size_t L1 = (size_t)p->d.lmax + 1;
+    for (int c = 0; c < 2 && ok; ++c)
+        ok = alloc_owned(p, &w->r[c], n) && alloc_owned(p, &w->p[c], n) && alloc_owned(p, &w->q[c], n) && alloc_owned(p, &w->ic_l[c], L1) &&
+             alloc_owned(p, &w->pre_l[c], L1);
+    ok = ok && alloc_owned(p, &w->partials, SV_GRID * 2) && build_lof(p, &w->lof);
+    ok = ok && alloc_state(p, &w->state, &w->host_state);
     if (!ok) { gs_set_error("PCG workspace allocation failed: %s", cudaGetErrorString(cudaGetLastError())); delete w; return nullptr; }
     p->pcg_ws = w;
     return w;
@@ -352,30 +356,19 @@ static gs_pcg_ws* get_ws_batch(gs_plan* p)
 {
     if (p->pcg_ws_batch) return (gs_pcg_ws*)p->pcg_ws_batch;
     gs_pcg_ws* w = new gs_pcg_ws[2]();
-    const size_t n = (size_t)p->nreal_loc;
-    auto alloc = [&](double** q, size_t cnt) { void* d = nullptr; if (cudaMalloc(&d, cnt * sizeof(double)) != cudaSuccess) return false; p->owned.push_back(d); *q = (double*)d; return true; };
+    const size_t n = (size_t)p->nreal_loc, L1 = (size_t)p->d.lmax + 1;
     double *P = nullptr, *Q = nullptr;
-    bool ok = alloc(&P, 4 * n) && alloc(&Q, 4 * n);
+    bool ok = alloc_owned(p, &P, 4 * n) && alloc_owned(p, &Q, 4 * n);
     for (int k = 0; k < 2 && ok; ++k) {
         w[k].red = nullptr;
         for (int c = 0; c < 2 && ok; ++c) {
             w[k].p[c] = P + (2 * k + c) * n;
             w[k].q[c] = Q + (2 * k + c) * n;
-            ok = alloc(&w[k].r[c], n) && alloc(&w[k].invc[c], n) && alloc(&w[k].pre[c], n);
+            ok = alloc_owned(p, &w[k].r[c], n) && alloc_owned(p, &w[k].ic_l[c], L1) && alloc_owned(p, &w[k].pre_l[c], L1);
         }
-        ok = ok && alloc(&w[k].partials, SV_GRID * 2 + 4 * (size_t)(p->d.lmax + 1));
-        if (ok) {
-            if (k == 0) ok = build_lof(p, &w[0].lof); else w[1].lof = w[0].lof;
-            double* tl = w[k].partials + SV_GRID * 2;
-            const int L1 = p->d.lmax + 1;
-            w[k].ic_l[0] = tl; w[k].pre_l[0] = tl + L1; w[k].ic_l[1] = tl + 2 * L1; w[k].pre_l[1] = tl + 3 * L1;
-        }
-        w[k].fuse_partials = nullptr;
-        ok = ok && alloc(&w[k].fuse_out, 4);
-        void* d = nullptr;
-        ok = ok && cudaMalloc(&d, sizeof(PcgState)) == cudaSuccess;
-        if (ok) { p->owned.push_back(d); w[k].state = (PcgState*)d; }
-        ok = ok && cudaMallocHost((void**)&w[k].host_state, 2 * sizeof(PcgState)) == cudaSuccess;
+        ok = ok && alloc_owned(p, &w[k].partials, SV_GRID * 2);
+        if (ok) { if (k == 0) ok = build_lof(p, &w[0].lof); else w[1].lof = w[0].lof; }
+        ok = ok && alloc_state(p, &w[k].state, &w[k].host_state);
     }
     void* d = nullptr;
     ok = ok && cudaMalloc(&d, sizeof(int)) == cudaSuccess;
@@ -391,7 +384,7 @@ void gs_pcg_ws_free(gs_plan* p)
     teb_ws_free(p);
     gs_pcg_ws* w = (gs_pcg_ws*)p->pcg_ws;
     if (w) {
-        if (w->host_state) cudaFreeHost(w->host_state);   // the device buffers are in p->owned
+        if (w->host_state) cudaFreeHost(w->host_state);
         delete w;
         p->pcg_ws = nullptr;
     }
@@ -403,9 +396,6 @@ void gs_pcg_ws_free(gs_plan* p)
     }
 }
 
-int g_gs_fuse_apq = 0;   // 1: fused analysis-finish + (q += C^-1 p, <p, q>) kernel in the unsharded PCG (measured 0.4 % SLOWER
-                         // than the separate pass at NSIDE 512: 5125 block partials + a scalar kernel; kept as an option)
-extern "C" int gs_set_fuse_apq(int on) { const int old = g_gs_fuse_apq; g_gs_fuse_apq = on ? 1 : 0; return old; }
 int g_gs_pcg_graph = 1;   // 1: the iterations between two convergence polls of an unsharded PCG solve are replayed from a CUDA graph
 extern "C" int gs_set_pcg_graph(int on) { const int old = g_gs_pcg_graph; g_gs_pcg_graph = on ? 1 : 0; return old; }
 int g_gs_ring_fused = 1;
@@ -437,8 +427,7 @@ struct ActiveRings {   // scope guard: the plan's launchers use the active lists
 // q = B A^T N^-1 A B v   (C^-1 v is added by pcg_apq_kernel / the caller)
 // nc = 2 (chain batch): chain c reads vE/vB + c stride and writes qE/qB + c stride; one recurrence serves both chains
 static int apply_noise_op(gs_plan* p, const double* vE, const double* vB, const double* bl, const double* inv_noise,
-                          double* qE, double* qB, cudaStream_t st, const int* skip, int spin = 2, const FinishFuse* fuse = nullptr,
-                          int nc = 1, int64_t stride = 0)
+                          double* qE, double* qB, cudaStream_t st, const int* skip, int spin = 2, int nc = 1, int64_t stride = 0)
 {
     int rc;
     if ((rc = gs_leg_synth(p, spin, vE, vB, GS_ALM_REAL, bl, st, skip, nullptr, nc, stride))) return rc;
@@ -448,7 +437,7 @@ static int apply_noise_op(gs_plan* p, const double* vE, const double* vB, const 
         if ((rc = gs_ring_synth(p, spin, p->mapQ_tmp, p->mapU_tmp, st, skip))) return rc;
         if ((rc = gs_ring_anal(p, spin, p->mapQ_tmp, p->mapU_tmp, inv_noise, st, skip))) return rc;
     }
-    return gs_leg_anal(p, spin, qE, qB, GS_ALM_REAL, bl, 1.0, 0, st, skip, fuse, nc, stride);
+    return gs_leg_anal(p, spin, qE, qB, GS_ALM_REAL, bl, 1.0, 0, st, skip, nc, stride);
 }
 
 // The poll loop shared by the PCG solves: `iteration(stream)` enqueues one PCG iteration whose launches take every scalar
@@ -466,8 +455,7 @@ static int pcg_poll_loop(gs_plan* p, cudaStream_t st, PcgState* state, PcgState*
     bool finished = false;
     cudaGraphExec_t gexec = nullptr;
     long long launches_per_graph = 0;
-    static const bool env_graph_off = [] { const char* e = getenv("GS_PCG_GRAPH"); return e && e[0] == '0'; }();   // GS_PCG_GRAPH=0: plain launches
-    if (g_gs_pcg_graph && !env_graph_off && !dist && itermax >= check_every) {
+    if (g_gs_pcg_graph && !dist && itermax >= check_every) {
         if (!p->work_stream) {
             cudaStream_t ws = nullptr;
             GS_CHECK_CUDA(cudaStreamCreateWithFlags(&ws, cudaStreamNonBlocking));
@@ -568,14 +556,12 @@ static int cr_pcg_impl(gs_plan* p, int spin, const double* dl_EE, const double* 
     const int64_t n = p->nreal_loc;
     if (check_every < 1) check_every = 8;
 
-    // per-l C^-1 and preconditioner, expanded to the real layout
-    double* tmp_l = w->partials + SV_GRID * 2;  // 4 (L+1) doubles of scratch
+    // per-l C^-1 and preconditioner: the vector kernels index them with the multipole of each coefficient, w->lof
     const int lb = (L + 256) / 256;
-    precond_kernel<<<lb, 256, 0, st>>>(dl_EE, bl, ninv_sum_over_4pi, L, tmp_l, tmp_l + (L + 1));
-    if (nc == 2) precond_kernel<<<lb, 256, 0, st>>>(dl_BB, bl, ninv_sum_over_4pi, L, tmp_l + 2 * (L + 1), tmp_l + 3 * (L + 1));
+    precond_kernel<<<lb, 256, 0, st>>>(dl_EE, bl, ninv_sum_over_4pi, L, w->ic_l[0], w->pre_l[0]);
+    if (nc == 2) precond_kernel<<<lb, 256, 0, st>>>(dl_BB, bl, ninv_sum_over_4pi, L, w->ic_l[1], w->pre_l[1]);
     GS_CHECK_LAUNCH();
     int rc;
-    // (the per-l tables are used as they are: the vector kernels index them with the multipole of each coefficient, w->lof)
     const bool dist = p->world > 1;
     ActiveRings act(p);
     if ((rc = act.begin(inv_noise, st))) return rc;
@@ -587,11 +573,9 @@ static int cr_pcg_impl(gs_plan* p, int spin, const double* dl_EE, const double* 
     *w->host_state = h;
     GS_CHECK_CUDA(cudaMemcpyAsync(w->state, w->host_state, sizeof(PcgState), cudaMemcpyHostToDevice, st));
     if (warm_start) {  // r0 = b - Q x0
-        if ((rc = gs_plan_expand_per_l(p, tmp_l, 0, w->invc[0], st))) return rc;
-        if (nc == 2 && (rc = gs_plan_expand_per_l(p, tmp_l + 2 * (L + 1), 0, w->invc[1], st))) return rc;
         if ((rc = apply_noise_op(p, x_E, x_B, bl, inv_noise, w->q[0], w->q[1], st, nullptr, spin))) return rc;
-        axy_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->invc[0], x_E, w->q[0], n);
-        if (nc == 2) axy_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[1], w->invc[1], x_B, w->q[1], n);
+        add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->ic_l[0], w->lof, x_E, w->q[0], n);
+        if (nc == 2) add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[1], w->ic_l[1], w->lof, x_B, w->q[1], n);
     } else {
         zero2_kernel<<<SV_GRID, SV_NT, 0, st>>>(x_E, nc == 2 ? x_B : x_E, n);
     }
@@ -603,17 +587,11 @@ static int cr_pcg_impl(gs_plan* p, int spin, const double* dl_EE, const double* 
     }
 
     const int* done = &w->state->done;
-    // optional (gs_set_fuse_apq): q += C^-1 p and <p, q> ride on the last kernel of the analysis
-    FinishFuse ff;
-    ff.pE = w->p[0]; ff.pB = w->p[1]; ff.icE = tmp_l; ff.icB = tmp_l + 2 * (L + 1);
-    ff.partials = w->fuse_partials; ff.counter = &w->state->counter; ff.out = w->fuse_out;
-    const bool fused_apq = !dist && g_gs_fuse_apq;
     // one PCG iteration: 7 launches whose arguments do not change during the solve (alpha, beta and the done flag live on the device)
     auto iteration = [&](cudaStream_t s) -> int {
         int r;
-        if ((r = apply_noise_op(p, w->p[0], w->p[1], bl, inv_noise, w->q[0], w->q[1], s, done, spin, fused_apq ? &ff : nullptr))) return r;
-        if (fused_apq) pcg_apq_scalar_kernel<<<1, 1, 0, s>>>(*w);
-        else pcg_apq_kernel<<<SV_GRID, SV_NT, 0, s>>>(*w, n, nc);
+        if ((r = apply_noise_op(p, w->p[0], w->p[1], bl, inv_noise, w->q[0], w->q[1], s, done, spin))) return r;
+        pcg_apq_kernel<<<SV_GRID, SV_NT, 0, s>>>(*w, n, nc);
         if (dist) {
             if ((r = gs_shard_allreduce(p, w->red, 1, s))) return r;
             pcg_scalar_kernel<<<1, 1, 0, s>>>(*w, 1);
@@ -676,9 +654,8 @@ extern "C" int gs_cr_pcg_pol_batch(gs_plan* p, int n_chain, const double* dl_EE,
     if ((rc = act.begin(inv_noise, st))) return rc;
     for (int k = 0; k < 2; ++k) {
         gs_pcg_ws* w = &W[k];
-        double* tmp_l = w->partials + SV_GRID * 2;
-        precond_kernel<<<lb, 256, 0, st>>>(dl_EE + k * (L + 1), bl, ninv_sum_over_4pi, L, tmp_l, tmp_l + (L + 1));
-        precond_kernel<<<lb, 256, 0, st>>>(dl_BB + k * (L + 1), bl, ninv_sum_over_4pi, L, tmp_l + 2 * (L + 1), tmp_l + 3 * (L + 1));
+        precond_kernel<<<lb, 256, 0, st>>>(dl_EE + k * (L + 1), bl, ninv_sum_over_4pi, L, w->ic_l[0], w->pre_l[0]);
+        precond_kernel<<<lb, 256, 0, st>>>(dl_BB + k * (L + 1), bl, ninv_sum_over_4pi, L, w->ic_l[1], w->pre_l[1]);
         GS_CHECK_LAUNCH();
         PcgState h;
         memset(&h, 0, sizeof(h));
@@ -697,7 +674,7 @@ extern "C" int gs_cr_pcg_pol_batch(gs_plan* p, int n_chain, const double* dl_EE,
     while (!(done[0] && done[1]) && launched < itermax) {
         for (int it = 0; it < check_every && launched < itermax; ++it, ++launched) {
             if (!done[0] && !done[1]) {
-                if ((rc = apply_noise_op(p, W[0].p[0], W[0].p[1], bl, inv_noise, W[0].q[0], W[0].q[1], st, p->pcg_alldone, 2, nullptr, 2, bstride))) return rc;
+                if ((rc = apply_noise_op(p, W[0].p[0], W[0].p[1], bl, inv_noise, W[0].q[0], W[0].q[1], st, p->pcg_alldone, 2, 2, bstride))) return rc;
             } else {
                 gs_pcg_ws* w = &W[done[0] ? 1 : 0];
                 if ((rc = apply_noise_op(p, w->p[0], w->p[1], bl, inv_noise, w->q[0], w->q[1], st, &w->state->done, 2))) return rc;
@@ -753,9 +730,10 @@ extern "C" int gs_cr_apply_q_tt(gs_plan* p, const double* dl_TT, const double* b
     int rc;
     ActiveRings act(p);
     if ((rc = act.begin(inv_noise, st))) return rc;
-    if ((rc = gs_plan_expand_per_l(p, dl_TT, 2, w->invc[0], st))) return rc;
+    const int L = p->d.lmax;
+    precond_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_TT, bl, 0.0, L, w->ic_l[0], w->pre_l[0]);   // only C^-1 is read
     if ((rc = apply_noise_op(p, x, nullptr, bl, inv_noise, w->q[0], nullptr, st, nullptr, 0))) return rc;
-    axy_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->invc[0], x, y, p->nreal_loc);
+    add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->ic_l[0], w->lof, x, y, p->nreal_loc);
     GS_CHECK_LAUNCH();
     return GS_OK;
 }
@@ -804,11 +782,12 @@ extern "C" int gs_cr_apply_q_pol(gs_plan* p, const double* dl_EE, const double* 
     int rc;
     ActiveRings act(p);
     if ((rc = act.begin(inv_noise, st))) return rc;
-    if ((rc = gs_plan_expand_per_l(p, dl_EE, 2, w->invc[0], st))) return rc;
-    if ((rc = gs_plan_expand_per_l(p, dl_BB, 2, w->invc[1], st))) return rc;
+    const int L = p->d.lmax;
+    precond_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_EE, bl, 0.0, L, w->ic_l[0], w->pre_l[0]);   // only C^-1 is read
+    precond_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_BB, bl, 0.0, L, w->ic_l[1], w->pre_l[1]);
     if ((rc = apply_noise_op(p, x_E, x_B, bl, inv_noise, w->q[0], w->q[1], st, nullptr))) return rc;
-    axy_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->invc[0], x_E, y_E, n);
-    axy_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[1], w->invc[1], x_B, y_B, n);
+    add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->ic_l[0], w->lof, x_E, y_E, n);
+    add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[1], w->ic_l[1], w->lof, x_B, y_B, n);
     GS_CHECK_LAUNCH();
     return GS_OK;
 }
@@ -1112,15 +1091,11 @@ static TebWs* get_ws_teb(gs_plan* p)
     if (!base) return nullptr;
     TebWs* w = new TebWs();
     const size_t n = (size_t)p->nreal_loc;
-    auto alloc = [&](double** q, size_t cnt) { void* d = nullptr; if (cudaMalloc(&d, cnt * sizeof(double)) != cudaSuccess) return false; p->owned.push_back(d); *q = (double*)d; return true; };
     bool ok = true;
-    for (int c = 0; c < 3 && ok; ++c) ok = alloc(&w->r[c], n) && alloc(&w->p[c], n) && alloc(&w->q[c], n);
-    ok = ok && alloc(&w->tab, (size_t)TEB_TAB * (p->d.lmax + 1)) && alloc(&w->partials, SV_GRID * 2);
+    for (int c = 0; c < 3 && ok; ++c) ok = alloc_owned(p, &w->r[c], n) && alloc_owned(p, &w->p[c], n) && alloc_owned(p, &w->q[c], n);
+    ok = ok && alloc_owned(p, &w->tab, (size_t)TEB_TAB * (p->d.lmax + 1)) && alloc_owned(p, &w->partials, SV_GRID * 2);
     w->lof = base->lof;
-    void* d = nullptr;
-    ok = ok && cudaMalloc(&d, sizeof(PcgState)) == cudaSuccess;
-    if (ok) { p->owned.push_back(d); w->state = (PcgState*)d; }
-    ok = ok && cudaMallocHost((void**)&w->host_state, 2 * sizeof(PcgState)) == cudaSuccess;
+    ok = ok && alloc_state(p, &w->state, &w->host_state);
     if (!ok) { gs_set_error("joint T/E/B workspace allocation failed: %s", cudaGetErrorString(cudaGetLastError())); delete w; return nullptr; }
     p->pcg_ws_teb = w;
     return w;
@@ -1130,7 +1105,7 @@ static void teb_ws_free(gs_plan* p)
 {
     TebWs* w = (TebWs*)p->pcg_ws_teb;
     if (!w) return;
-    if (w->host_state) cudaFreeHost(w->host_state);   // the device buffers are in p->owned
+    if (w->host_state) cudaFreeHost(w->host_state);
     delete w;
     p->pcg_ws_teb = nullptr;
 }
@@ -1454,7 +1429,7 @@ extern "C" int gs_profile_matvec_batch(gs_plan* p, int n_chain, const double* x_
             cudaEventRecord(ev[1], st);
             if (!rc) rc = gs_ring_apply(p, 2, inv_noise, st, nullptr, n_chain);
             cudaEventRecord(ev[2], st);
-            if (!rc) rc = gs_leg_anal(p, 2, y_E, y_B, GS_ALM_REAL, bl, 1.0, 0, st, nullptr, nullptr, n_chain, stride);
+            if (!rc) rc = gs_leg_anal(p, 2, y_E, y_B, GS_ALM_REAL, bl, 1.0, 0, st, nullptr, n_chain, stride);
             cudaEventRecord(ev[3], st);
             if (cudaEventSynchronize(ev[3]) != cudaSuccess) { gs_set_error("gs_profile_matvec_batch: %s", cudaGetErrorString(cudaGetLastError())); rc = GS_E_CUDA; break; }
             for (int i = 0; i < 3; ++i) { float ms = 0; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); acc[i] += ms; }
@@ -1467,7 +1442,7 @@ extern "C" int gs_profile_matvec_batch(gs_plan* p, int n_chain, const double* x_
 
 // Times the three vector kernels of one PCG iteration (q += C^-1 p with <p,q>; x, r update with <r,r>, <r,Mr>; p = M r + beta p)
 // on the plan's own workspace, zero-filled, with CUDA events on `stream`: ms_out[0..2] = average of nrep launches each.  The
-// reductions run as in the solver but their results go to a scratch slot, so no solver state changes.
+// reductions run as in the solver but their results go to a scratch buffer, so no solver state changes.
 extern "C" int gs_profile_pcg_vectors(gs_plan* p, int spin, int nrep, float* ms_out, void* stream)
 {
     if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
@@ -1479,46 +1454,45 @@ extern "C" int gs_profile_pcg_vectors(gs_plan* p, int spin, int nrep, float* ms_
     const int nc = spin ? 2 : 1;
     const int64_t n = p->nreal_loc;
     for (int c = 0; c < 2; ++c) {
-        double* arrs[5] = {w->r[c], w->p[c], w->q[c], w->invc[c], w->pre[c]};
+        double* arrs[3] = {w->r[c], w->p[c], w->q[c]};
         for (double* a : arrs) GS_CHECK_CUDA(cudaMemsetAsync(a, 0, (size_t)n * sizeof(double), st));
+        double* tabs[2] = {w->ic_l[c], w->pre_l[c]};   // per-l tables
+        for (double* a : tabs) GS_CHECK_CUDA(cudaMemsetAsync(a, 0, (size_t)(p->d.lmax + 1) * sizeof(double), st));
     }
     GS_CHECK_CUDA(cudaMemsetAsync(p->almE_tmp, 0, (size_t)n * sizeof(double), st));
     GS_CHECK_CUDA(cudaMemsetAsync(p->almB_tmp, 0, (size_t)n * sizeof(double), st));
     GS_CHECK_CUDA(cudaMemsetAsync(w->state, 0, sizeof(PcgState), st));
-    GS_CHECK_CUDA(cudaMemsetAsync(w->partials + SV_GRID * 2, 0, (size_t)4 * (p->d.lmax + 1) * sizeof(double), st));   // per-l tables
+    double* red = nullptr;   // the reductions land here: the solver state (done flag, alpha, beta = 0) stays untouched
+    GS_CHECK_CUDA(cudaMalloc(&red, 2 * sizeof(double)));
     gs_pcg_ws v = *w;
-    v.red = w->fuse_out;   // reductions land here: the solver state (done flag, alpha, beta = 0) stays untouched
-    cudaEvent_t e0, e1;
-    GS_CHECK_CUDA(cudaEventCreate(&e0));
-    GS_CHECK_CUDA(cudaEventCreate(&e1));
+    v.red = red;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    int rc = GS_OK;
+    if (cudaEventCreate(&e0) != cudaSuccess || cudaEventCreate(&e1) != cudaSuccess) rc = GS_E_CUDA;
     // between launches the analysis partials (> L2 at the bench size) are overwritten, as the Legendre / ring kernels do
     // between the vector kernels of a real iteration: the arrays come from HBM, not from the 126 MB L2
     const size_t flush_bytes = (size_t)p->anal_chunks * (size_t)(p->world > 1 ? p->d.sh.nalm_loc : p->d.nalm) * 4 * sizeof(double);
-    for (int k = 0; k < 3; ++k) {
+    for (int k = 0; k < 3 && rc == GS_OK; ++k) {
         double acc = 0.0;
         for (int rep = -2; rep < nrep; ++rep) {   // two warm-up launches
-            if (cudaMemsetAsync(p->partial, 0, flush_bytes, st) != cudaSuccess) {
-                gs_set_error("gs_profile_pcg_vectors: %s", cudaGetErrorString(cudaGetLastError()));
-                cudaEventDestroy(e0); cudaEventDestroy(e1);
-                return GS_E_CUDA;
-            }
+            if (cudaMemsetAsync(p->partial, 0, flush_bytes, st) != cudaSuccess) { rc = GS_E_CUDA; break; }
             cudaEventRecord(e0, st);
             if (k == 0) pcg_apq_kernel<<<SV_GRID, SV_NT, 0, st>>>(v, n, nc);
             else if (k == 1) pcg_update_kernel<<<SV_GRID, SV_NT, 0, st>>>(v, p->almE_tmp, p->almB_tmp, n, nc);
             else pcg_dir_kernel<<<SV_GRID, SV_NT, 0, st>>>(v, n, nc);
             cudaEventRecord(e1, st);
-            if (cudaEventSynchronize(e1) != cudaSuccess) {
-                gs_set_error("gs_profile_pcg_vectors: %s", cudaGetErrorString(cudaGetLastError()));
-                cudaEventDestroy(e0); cudaEventDestroy(e1);
-                return GS_E_CUDA;
-            }
+            if (cudaEventSynchronize(e1) != cudaSuccess) { rc = GS_E_CUDA; break; }
             float ms = 0;
             cudaEventElapsedTime(&ms, e0, e1);
             if (rep >= 0) acc += ms;
         }
         ms_out[k] = (float)(acc / nrep);
     }
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
+    if (rc == GS_E_CUDA) gs_set_error("gs_profile_pcg_vectors: %s", cudaGetErrorString(cudaGetLastError()));
+    if (e0) cudaEventDestroy(e0);
+    if (e1) cudaEventDestroy(e1);
+    cudaFree(red);
+    if (rc) return rc;
     GS_CHECK_LAUNCH();
     return GS_OK;
 }

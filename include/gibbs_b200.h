@@ -488,10 +488,6 @@ int gs_set_ring_skip(int on);
  * DFT of Q + iU along the ring (the weighted sums of squares of NonCenteredGibbs.py:380-399 are invariant under it), so their ring
  * FFTs are not run either; 0: every ring is transformed.  Same result to rounding.  Returns the previous setting. */
 int gs_set_ring_const(int on);
-/* on != 0: in gs_cr_pcg_* on unsharded plans the step  q += C^-1 p ; <p, q>  rides on the last kernel of the Legendre
- * analysis instead of a separate pass; 0 (default; the fused form measured 0.4 % slower at NSIDE 512): separate kernel.
- * Same numbers up to the summation order of the dot product.  Returns the previous setting. */
-int gs_set_fuse_apq(int on);
 /* Number of rings (of 4 nside - 1) whose pixel weights were all equal in the weight map of the last gs_cr_pcg_* /
  * gs_cr_apply_q_* / gs_profile_matvec call on this plan (rings inside the mask count: their weight is the constant 0);
  * 0 on sharded plans.  See gs_set_ring_const. */

@@ -1,5 +1,5 @@
 """A/B timing of one masked-sky PCG solve (NSIDE 512 / lmax 1024, the bench system) with a library switch on and off.
-usage: python scripts/ab_pcg.py gs_set_fuse_apq | gs_set_ring_skip | gs_set_ring_fused"""
+usage: python scripts/ab_pcg.py [gs_set_ring_skip | gs_set_ring_fused]"""
 import os
 import sys
 
@@ -13,7 +13,7 @@ from gibbssampler_b200 import _dev, _lib, utils  # noqa: E402
 from gibbssampler_b200.CenteredGibbs import PolarizedCenteredConstrainedRealization as CR  # noqa: E402
 from gibbssampler_b200.sht import Plan  # noqa: E402
 
-setter = sys.argv[1] if len(sys.argv) > 1 else "gs_set_fuse_apq"
+setter = sys.argv[1] if len(sys.argv) > 1 else "gs_set_ring_skip"
 nside, lmax = 512, 1024
 npix, nre = 12 * nside ** 2, (lmax + 1) ** 2
 L = _lib.lib()
