@@ -8,6 +8,9 @@ The reference never finished this path: the per-l 3x3 helpers survive only as by
 3x3 solve:
     Sigma_l = (C_l^-1 + diag(b_l^2 w_X))^-1,  s = Sigma_l (b_l w_X d_X)_X + chol(Sigma_l) xi,  w_X = Npix / (4 pi sigma^2_X)
 and  (C^TT, C^TE, C^EE)_l | s ~ IW(2l - 2, (2l+1) Chat_l),  C^BB_l | s ~ inverse-gamma as in CenteredGibbs.py:54-79.
+With bins (D constant on each bin, as the reference bins EE/BB) the TT/TE/EE block of bin b is
+    D_b | s ~ IW(nu_b, Psi_b),  nu_b = sum_{l in b} (2l+1) - 3,  Psi_b = sum_{l in b} (2l+1) l(l+1)/(2 pi) Chat_l
+and BB takes the reference's binned inverse-gamma.
 Every step is a batched one-thread-per-l (or per-coefficient) kernel of libgibbs_b200.so.
 
 On a cut sky (pixel data, one mask for T and another for P, per-pixel noise) the constrained realization is the joint T/E/B
@@ -176,13 +179,42 @@ class JointConstrainedRealization():
         return {"TT": out[:, 0].contiguous(), "EE": out[:, 1].contiguous(), "BB": out[:, 2].contiguous()}, 1
 
 
+def _joint_bins(bins, lmax):
+    """Validated bin edges {"TT": edges, "BB": edges} of the joint C_l step (int64 numpy arrays, host)."""
+    if "TT" not in bins or "BB" not in bins:
+        raise ValueError("bins needs 'TT' (shared by TE and EE) and 'BB' edges")
+    out = {}
+    for key in ("TT", "BB"):
+        e = np.asarray(bins[key])
+        if e.ndim != 1 or e.size < 3 or not np.issubdtype(e.dtype, np.integer):
+            raise ValueError("bins[%r] must be a 1-d integer array of at least 3 edges" % key)
+        e = e.astype(np.int64)
+        if list(e[:3]) != [0, 1, 2]:
+            raise ValueError("bins[%r] must start with the edges 0, 1, 2 (l = 0 and l = 1 are bins of their own)" % key)
+        if e[-1] != lmax + 1:
+            raise ValueError("bins[%r] must end at lmax + 1 = %d, not %d" % (key, lmax + 1, e[-1]))
+        if np.any(np.diff(e) <= 0):
+            raise ValueError("bins[%r] must be strictly ascending" % key)
+        out[key] = e
+    for key in ("TE", "EE"):   # one 2x2 matrix per bin: TT, TE and EE share the binning
+        if key in bins and not np.array_equal(np.asarray(bins[key]), out["TT"]):
+            raise ValueError("bins[%r] must equal bins['TT']" % key)
+    return out
+
+
 class JointClsSampler():
-    def __init__(self, lmax, *, rng="philox", seed=None):
+    def __init__(self, lmax, *, bins=None, rng="philox", seed=None):
+        """bins: None (one draw per multipole) or {"TT": edges, "BB": edges} with int edges that start 0, 1, 2 and end at
+        lmax + 1 ("TE" / "EE" may be given and must equal "TT"): then sample() draws D constant on each bin, TT/TE/EE by the
+        binned inverse-Wishart of gs_cls_invwishart_binned and BB by the binned inverse-gamma of CenteredGibbs.py:54-79."""
         self.lmax = int(lmax)
+        self.bins = None if bins is None else _joint_bins(bins, self.lmax)
         self.dev = _dev.device()
         self.rng = rng if isinstance(rng, _dev.Rng) else _dev.Rng(rng, seed)
         self._call = 0
         self.bins1 = _dev.i32(np.arange(self.lmax + 2))
+        if self.bins is not None:
+            self._bins_dev = {k: _dev.i32(v) for k, v in self.bins.items()}
 
     def empirical(self, alms):
         L = _lib.lib()
@@ -195,8 +227,11 @@ class JointClsSampler():
         return out
 
     def sample(self, alms, inject=None, gamma_inject=None):
-        """-> unbinned D_l dict {"TT","EE","BB","TE"}.  inject: (L+1,3) (chi2_df, chi2_{df-1}, normal) and gamma_inject
-        (L+1) Gamma variates for parity runs; default Philox."""
+        """-> D dict {"TT","EE","BB","TE"}: unbinned D_l (L+1) without bins, binned D (nbins_TT for TT/TE/EE, nbins_BB for BB)
+        with bins.  inject: (L+1,3) or (nbins_TT,3) (chi2_df, chi2_{df-1}, normal) and gamma_inject (L+1) or (nbins_BB) Gamma
+        variates for parity runs; default Philox."""
+        if self.bins is not None:
+            return self._sample_binned(alms, inject, gamma_inject)
         L = _lib.lib()
         ch = self.empirical(alms)
         self.rng.counter += 2          # shared generator counter (see ClsSampler._invgamma_draw): one index per draw kernel
@@ -213,26 +248,60 @@ class JointClsSampler():
                                 ptr(bb), None, None, stream()))
         return {"TT": tt * c2d, "TE": te * c2d, "EE": ee * c2d, "BB": bb}
 
+    def _sample_binned(self, alms, inject, gamma_inject):
+        L = _lib.lib()
+        nt, nb = len(self.bins["TT"]) - 1, len(self.bins["BB"]) - 1
+        inj = f64(inject).contiguous() if inject is not None else None
+        gi = f64(gamma_inject).contiguous() if gamma_inject is not None else None
+        if inj is not None and tuple(inj.shape) != (nt, 3):
+            raise ValueError("inject must have shape (%d, 3), got %s" % (nt, tuple(inj.shape)))
+        if gi is not None and gi.numel() != nb:
+            raise ValueError("gamma_inject must have %d entries, got %d" % (nb, gi.numel()))
+        ch = self.empirical(alms)
+        self.rng.counter += 2          # the same two call indices as the per-l draw
+        self._call = self.rng.counter - 1
+        tt, te, ee = (torch.empty(nt, dtype=torch.float64, device=self.dev) for _ in range(3))
+        check(L.gs_cls_invwishart_binned(ptr(ch["TT"]), ptr(ch["TE"]), ptr(ch["EE"]), self.lmax, ptr(self._bins_dev["TT"]), nt,
+                                         ptr(inj), self.rng.seed, self._call, ptr(tt), ptr(te), ptr(ee), stream()))
+        bb = torch.empty(nb, dtype=torch.float64, device=self.dev)
+        check(L.gs_cls_invgamma(ptr(ch["BB"]), ptr(self._bins_dev["BB"]), nb, ptr(gi), self.rng.seed, self._call + 1, ptr(bb), None,
+                                None, stream()))
+        return {"TT": tt, "TE": te, "EE": ee, "BB": bb}
+
 
 class JointGibbs():
     """CR <-> C_l Gibbs loop for (T, E, B) with TE correlation: full sky with isotropic noise and harmonic data
-    ({"TT","EE","BB"}), or a cut sky with pixel data ({"I","Q","U"}, masks `mask` for T and `mask_pol` for P)."""
+    ({"TT","EE","BB"}), or a cut sky with pixel data ({"I","Q","U"}, masks `mask` for T and `mask_pol` for P).
+    bins (see JointClsSampler): D is sampled per bin; run() then takes binned initial D and returns binned histories, and each
+    constrained realization sees D unfolded to L+1 multipoles (utils.unfold_bins)."""
 
     def __init__(self, pix_map, noise_temp, noise_pol, beam_fwhm_deg, nside, lmax, n_iter=1000, *, mask=None, mask_pol=None,
-                 rng="philox", seed=None):
+                 bins=None, rng="philox", seed=None):
         self.lmax, self.nside, self.n_iter = int(lmax), int(nside), int(n_iter)
         bl = _dev.gauss_beam(np.radians(beam_fwhm_deg), self.lmax)
         shared = _dev.Rng(rng, seed)
+        self.cls_sampler = JointClsSampler(lmax, bins=bins, rng=shared)     # first: bad bins fail before the plan is built
+        self.bins = self.cls_sampler.bins
         self.constrained_sampler = JointConstrainedRealization(pix_map, noise_temp, noise_pol, bl, lmax, 12 * nside ** 2, mask=mask,
                                                                mask_pol=mask_pol, rng=shared)
-        self.cls_sampler = JointClsSampler(lmax, rng=shared)
+
+    def _unfold(self, dls):
+        if self.bins is None:
+            return dls
+        from . import utils
+        return {k: utils.unfold_bins(v, self.bins["BB" if k == "BB" else "TT"]) for k, v in dls.items()}
 
     def run(self, dls_init):
         keys = ("TT", "EE", "BB", "TE")
-        h = {k: [_dev.to_host(f64(dls_init[k]))] for k in keys}
         dls = {k: f64(dls_init[k]) for k in keys}
+        if self.bins is not None:
+            for k in keys:
+                want = len(self.bins["BB" if k == "BB" else "TT"]) - 1
+                if dls[k].numel() != want:
+                    raise ValueError("dls_init[%r] must hold %d binned values, got %d" % (k, want, dls[k].numel()))
+        h = {k: [_dev.to_host(dls[k])] for k in keys}
         for _ in range(self.n_iter):
-            sky, _ = self.constrained_sampler.sample(dls)
+            sky, _ = self.constrained_sampler.sample(self._unfold(dls))
             dls = self.cls_sampler.sample(sky)
             for k in keys:
                 h[k].append(_dev.to_host(dls[k]))

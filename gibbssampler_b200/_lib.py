@@ -89,6 +89,7 @@ SIGNATURES = {
     "gs_matvec_3x3": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "gs_alm2cl_cross": (_i, [_vp, _vp, _i, _vp, _vp]),
     "gs_cls_invwishart": (_i, [_vp, _vp, _vp, _i, _vp, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
+    "gs_cls_invwishart_binned": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
     "gs_nccl_unique_id": (_i, [C.c_char_p]),
     "gs_plan_create_sharded": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _i, C.c_char_p]),
     "gs_local_group_create": (_i, [C.POINTER(_vp), _i]),

@@ -4,7 +4,8 @@
 // recovered utils.compute_inverse_and_cholesky / utils.matrix_product and the deleted native module
 // linear_algebra.pyx (LAPACK dgesv/dpotrf/dpotri per l; SURVEY.md 2.3) by closed-form 3x3 algebra with one
 // thread per multipole (or per coefficient), and adds the inverse-Wishart draw the reference intended for
-// the TT/TE/EE block (.ipynb_checkpoints/main-checkpoint.py:39-44, 333-346: df = 2l - 2, scale = (2l+1) Chat_l).
+// the TT/TE/EE block (.ipynb_checkpoints/main-checkpoint.py:39-44, 333-346: df = 2l - 2, scale = (2l+1) Chat_l), per multipole
+// or, with D_l constant on each bin as in the reference's binned EE/BB (CenteredGibbs.py:54-79), per bin.
 // All arrays are row-major: per-l matrices (L+1,3,3), per-coefficient matrices ((L+1)^2,3,3), vectors
 // ((L+1)^2,3) with component order (T, E, B).
 #include <algorithm>
@@ -103,28 +104,23 @@ __global__ void alm2cl_cross_kernel(const double* __restrict__ x, const double* 
     if (lane == 0) cl[l] = s / (2.0 * l + 1.0);
 }
 
-// ---- inverse-Wishart draw of the (TT, TE; TE, EE) block per multipole, Bartlett decomposition:
-//   X ~ IW(nu, Psi), nu = 2l - 2, Psi = (2l+1) Chat_l   <=>   X^-1 ~ Wishart(nu, Psi^-1)
+// ---- inverse-Wishart draw of a (TT, TE; TE, EE) block, Bartlett decomposition:
+//   X ~ IW(nu, Psi)   <=>   X^-1 ~ Wishart(nu, Psi^-1)
 //   Psi^-1 = G G^T,  A = [[sqrt(chi2_nu), 0], [N(0,1), sqrt(chi2_{nu-1})]],  X^-1 = (G A)(G A)^T.
-// inject (nullable): (L+1, 3) = (chi2_nu, chi2_{nu-1}, normal) supplied by the caller (parity with a numpy
-// stream); otherwise Philox / Marsaglia-Tsang.  l < 2 -> 0.  Output in C_l units.
-__global__ void invwishart_2x2_kernel(const double* __restrict__ tt, const double* __restrict__ te, const double* __restrict__ ee, int L,
-                                      const double* __restrict__ inject, uint64_t seed, uint64_t call, double* __restrict__ o_tt,
-                                      double* __restrict__ o_te, double* __restrict__ o_ee)
+// Draw k (a multipole or a bin) takes row k of inject ((chi2_nu, chi2_{nu-1}, normal) supplied by the caller, parity with a numpy
+// stream) or, without inject, Philox / Marsaglia-Tsang on the streams base, base + 1, base + 2 with
+// base = (0x57 << 56) | ((call << 22) + 4 k): the "W"ishart domain (see sampler.cu).
+__device__ __forceinline__ void invwishart_2x2_draw(double p00, double p01, double p11, double nu, const double* __restrict__ inject, int k,
+                                                    uint64_t seed, uint64_t call, double& x00, double& x01, double& x11)
 {
-    const int l = blockIdx.x * blockDim.x + threadIdx.x;
-    if (l > L) return;
-    if (l < 2) { o_tt[l] = 0.0; o_te[l] = 0.0; o_ee[l] = 0.0; return; }
-    const double f = 2.0 * l + 1.0, nu = 2.0 * l - 2.0;
-    const double p00 = f * tt[l], p01 = f * te[l], p11 = f * ee[l];
     const double det = p00 * p11 - p01 * p01;
     const double q00 = p11 / det, q01 = -p01 / det, q11 = p00 / det;  // Psi^-1
     const double g00 = sqrt(q00), g10 = q01 / g00, g11 = sqrt(q11 - g10 * g10);  // lower Cholesky of Psi^-1
     double c1, c2, z;
-    if (inject) { c1 = inject[3 * l]; c2 = inject[3 * l + 1]; z = inject[3 * l + 2]; }
+    if (inject) { c1 = inject[3 * k]; c2 = inject[3 * k + 1]; z = inject[3 * k + 2]; }
     else {
         const Philox ph(seed);
-        const uint64_t base = (0x57ull << 56) | (((call << 22) + 4ull * (uint64_t)l) & 0x00ffffffffffffffull);   // "W"ishart domain (see sampler.cu)
+        const uint64_t base = (0x57ull << 56) | (((call << 22) + 4ull * (uint64_t)k) & 0x00ffffffffffffffull);
         c1 = 2.0 * gamma_mt(0.5 * nu, ph, base);
         c2 = 2.0 * gamma_mt(0.5 * (nu - 1.0), ph, base + 1);
         double z2;
@@ -135,7 +131,55 @@ __global__ void invwishart_2x2_kernel(const double* __restrict__ tt, const doubl
     const double h00 = g00 * a00, h10 = g10 * a00 + g11 * a10, h11 = g11 * a11;
     const double w00 = h00 * h00, w01 = h00 * h10, w11 = h10 * h10 + h11 * h11;
     const double dw = w00 * w11 - w01 * w01;
-    o_tt[l] = w11 / dw; o_te[l] = -w01 / dw; o_ee[l] = w00 / dw;
+    x00 = w11 / dw; x01 = -w01 / dw; x11 = w00 / dw;
+}
+
+// Per multipole (.ipynb_checkpoints/main-checkpoint.py:39-44, 333-346): C_l ~ IW(2l - 2, (2l+1) Chat_l), draw k = l.
+// inject (nullable): (L+1, 3).  l < 2 -> 0.  Output in C_l units.
+__global__ void invwishart_2x2_kernel(const double* __restrict__ tt, const double* __restrict__ te, const double* __restrict__ ee, int L,
+                                      const double* __restrict__ inject, uint64_t seed, uint64_t call, double* __restrict__ o_tt,
+                                      double* __restrict__ o_te, double* __restrict__ o_ee)
+{
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    if (l > L) return;
+    if (l < 2) { o_tt[l] = 0.0; o_te[l] = 0.0; o_ee[l] = 0.0; return; }
+    const double f = 2.0 * l + 1.0, nu = 2.0 * l - 2.0;
+    double x00, x01, x11;
+    invwishart_2x2_draw(f * tt[l], f * te[l], f * ee[l], nu, inject, l, seed, call, x00, x01, x11);
+    o_tt[l] = x00; o_te[l] = x01; o_ee[l] = x11;
+}
+
+// Per bin, with D_l = D_b constant on bin b (the binned model of CenteredGibbs.py:54-79, utils.unfold_bins):
+//   D_b | s ~ IW(nu_b, Psi_b),  nu_b = sum_{l in b} (2l+1) - 3,  Psi_b = sum_{l in b} (2l+1) l(l+1)/(2 pi) Chat_l,
+// the product over l in b of the per-l likelihoods |C_l|^{-(2l+1)/2} exp(-(2l+1)/2 tr(C_l^-1 Chat_l)) times the flat prior of the
+// per-l draw (for p = 1 the inverse-gamma alpha = sum (2l+1)/2 - 1 of cls_invgamma_kernel).  With one-l bins this is the per-l
+// draw scaled by l(l+1)/(2 pi), on the same variates (draw k = b).  Psi_b is summed in ascending l (deterministic); bins 0 and 1
+// are l = 0 and l = 1 (edges start 0, 1, 2) and are 0.  inject (nullable): (nbins, 3).  Output in D units.
+// The edges live on the device, so the host cannot check them without a copy and a synchronisation: each thread checks its own
+// bin instead and writes NaN where the edges break the conditions (bin 0 / 1 not [0, 1) / [1, 2), a bin empty, below l = 2 or
+// past L, a last edge other than L + 1), so such a binning shows up in the output instead of being zeroed or read out of range.
+__global__ void invwishart_binned_kernel(const double* __restrict__ tt, const double* __restrict__ te, const double* __restrict__ ee, int L,
+                                         const int* __restrict__ bins, int nbins, const double* __restrict__ inject, uint64_t seed,
+                                         uint64_t call, double* __restrict__ o_tt, double* __restrict__ o_te, double* __restrict__ o_ee)
+{
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nbins) return;
+    const int l0 = bins[b], l1 = bins[b + 1];
+    const bool ok = b < 2 ? (l0 == b && l1 == b + 1) : (l0 >= 2 && l1 > l0 && l1 <= L + 1 && (b < nbins - 1 || l1 == L + 1));
+    if (b < 2 || !ok) {
+        const double v = ok ? 0.0 : __longlong_as_double(0x7ff8000000000000ll);   // 0 for l = 0, 1; NaN for a bad bin
+        o_tt[b] = v; o_te[b] = v; o_ee[b] = v;
+        return;
+    }
+    double p00 = 0.0, p01 = 0.0, p11 = 0.0, nu = -3.0;
+    for (int l = l0; l < l1; ++l) {
+        const double f = 2.0 * l + 1.0, w = f * ((double)l * (double)(l + 1) / (2.0 * 3.14159265358979323846));
+        p00 += w * tt[l]; p01 += w * te[l]; p11 += w * ee[l];
+        nu += f;
+    }
+    double x00, x01, x11;
+    invwishart_2x2_draw(p00, p01, p11, nu, inject, b, seed, call, x00, x01, x11);
+    o_tt[b] = x00; o_te[b] = x01; o_ee[b] = x11;
 }
 
 // ---- C ABI
@@ -177,6 +221,18 @@ extern "C" int gs_cls_invwishart(const double* cl_tt, const double* cl_te, const
     GS_REQUIRE(cl_tt && cl_te && cl_ee && out_tt && out_te && out_ee && lmax >= 0, "bad arguments");
     invwishart_2x2_kernel<<<(lmax + TB_NT) / TB_NT, TB_NT, 0, STREAM(stream)>>>(cl_tt, cl_te, cl_ee, lmax, inject, seed, call, out_tt, out_te,
                                                                                out_ee);
+    GS_CHECK_LAUNCH();
+    return GS_OK;
+}
+
+extern "C" int gs_cls_invwishart_binned(const double* cl_tt, const double* cl_te, const double* cl_ee, int lmax, const int* bins, int nbins,
+                                        const double* inject, uint64_t seed, uint64_t call, double* dl_tt, double* dl_te, double* dl_ee,
+                                        void* stream)
+{
+    GS_REQUIRE(cl_tt && cl_te && cl_ee && bins && dl_tt && dl_te && dl_ee, "null pointer");
+    GS_REQUIRE(lmax >= 0 && nbins >= 1 && nbins <= lmax + 1, "need lmax >= 0 and 1 <= nbins <= lmax + 1");
+    invwishart_binned_kernel<<<(nbins + TB_NT - 1) / TB_NT, TB_NT, 0, STREAM(stream)>>>(cl_tt, cl_te, cl_ee, lmax, bins, nbins, inject, seed,
+                                                                                       call, dl_tt, dl_te, dl_ee);
     GS_CHECK_LAUNCH();
     return GS_OK;
 }

@@ -383,6 +383,19 @@ int gs_alm2cl_cross(const double* alm_x, const double* alm_y, int lmax, double* 
 int gs_cls_invwishart(const double* cl_tt, const double* cl_te, const double* cl_ee, int lmax,
                       const double* inject, uint64_t seed, uint64_t call, double* out_tt, double* out_te,
                       double* out_ee, void* stream);
+/* Binned twin of gs_cls_invwishart (.ipynb_checkpoints/main-checkpoint.py:39-44, 333-346 with the binning of
+ * CenteredGibbs.py:54-79): D_l = D_b on each bin b, and per bin, one thread each,
+ *   D_b | s ~ IW(nu_b, Psi_b),  nu_b = sum_{l in b} (2l+1) - 3,  Psi_b = sum_{l in b} (2l+1) l(l+1)/(2pi) Chat_l,
+ * Psi_b summed in ascending l.  With one-l bins this is gs_cls_invwishart times l(l+1)/(2pi) on the same variates.
+ * cl_* are the unbinned empirical spectra (L+1); bins = nbins + 1 ascending int32 edges (device) that start 0, 1, 2
+ * and end at lmax + 1 (bins 0 and 1 are l = 0 and l = 1 and come out 0); outputs dl_* are nbins binned D each.
+ * inject (nullable, (nbins,3)) = (chi2_nu, chi2_{nu-1}, N(0,1)) per bin; NULL: Philox stream of draw b keyed as draw
+ * l = b of gs_cls_invwishart.  GS_E_BADARG for null pointers, lmax < 0 or nbins outside [1, lmax + 1].  The edges are
+ * checked on the device, bin by bin: a bin whose edges break the conditions above (bin 0 or 1 other than [0,1) / [1,2), an
+ * empty bin, a bin below l = 2 or past lmax, a last edge other than lmax + 1) comes out NaN in all three outputs. */
+int gs_cls_invwishart_binned(const double* cl_tt, const double* cl_te, const double* cl_ee, int lmax,
+                             const int* bins, int nbins, const double* inject, uint64_t seed, uint64_t call,
+                             double* dl_tt, double* dl_te, double* dl_ee, void* stream);
 
 /* ---- whole chain in one call (SURVEY.md 8b gs_gibbs_step_centered; BASELINE config #1) -----------------------------------
  * GibbsSampler.run_polarization (GibbsSampler.py:118-180) for the full-sky isotropic-noise centred sampler: every iteration is

@@ -1,8 +1,9 @@
 """Joint T/E/B constrained realization on a cut sky (gs_cr_pcg_teb) at NSIDE 512 / lmax 1024: PCG iterations and time of the
 masked joint solve, the mat-vec split into its spin-0 half, spin-2 half and vector kernels (CUDA events,
 gs_profile_matvec_teb), the vector kernels' bytes and share of HBM peak, masked JointGibbs iterations per second, and the E/B-only
-solve on the same P mask for context.  T mask: bench.make_mask "galplane"; P mask: "band".  Writes one JSON line (stdout, and
---out if given).  Needs a GPU."""
+solve on the same P mask for context.  T mask: bench.make_mask "galplane"; P mask: "band".  With --bins planck it measures the
+binned joint sampler instead (planck_bins): masked JointGibbs it/s with bins, and the binned C_l step alone (CUDA events) next to
+the per-l one.  Writes one JSON line (stdout, and --out if given).  Needs a GPU."""
 import argparse
 import ctypes as C
 import json
@@ -17,8 +18,8 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.dont_write_bytecode = True
 import bench  # noqa: E402
-from gibbssampler_b200 import _dev, _lib  # noqa: E402
-from gibbssampler_b200.JointSampler import JointConstrainedRealization, JointGibbs  # noqa: E402
+from gibbssampler_b200 import _dev, _lib, utils  # noqa: E402
+from gibbssampler_b200.JointSampler import JointClsSampler, JointConstrainedRealization, JointGibbs  # noqa: E402
 from gibbssampler_b200.sht import Plan  # noqa: E402
 
 HBM_PEAK = 7.7e12   # B/s, one B200 (data sheet); the share below is bytes moved / kernel time / this
@@ -32,6 +33,70 @@ def fiducial_teb(lmax):
     tt = np.where(ell >= 2, 30.0 * (np.exp(-(ell / 900.0) ** 2) + 0.05), 0.0)
     te = 0.5 * np.sqrt(tt * ee) * np.cos(ell / 60.0)
     return {"TT": tt, "TE": te, "EE": ee, "BB": bb}
+
+
+def planck_bins(lmax):
+    """TT/TE/EE: one multipole per bin up to l = 30, then bins of width 10 (the last one ends at lmax + 1); BB: the Planck-like
+    edges of bench.bins_for."""
+    tt = np.unique(np.concatenate([np.arange(0, min(lmax, 30) + 1), np.arange(40, lmax + 1, 10), [lmax + 1]]))
+    return {"TT": tt, "BB": np.asarray(bench.bins_for(lmax)["BB"])}
+
+
+def cuda_ms(fn, nrep):
+    """mean time of fn() between two CUDA events over nrep calls, after one warm-up call"""
+    fn()
+    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    t0.record()
+    for _ in range(nrep):
+        fn()
+    t1.record()
+    torch.cuda.synchronize()
+    return t0.elapsed_time(t1) / nrep
+
+
+def binned_report(a, data, noise_T, noise_P, fwhm, maskT, maskP, dls):
+    """masked JointGibbs with planck_bins (it/s) and the C_l step alone, binned and per l"""
+    lmax = a.lmax
+    bins = planck_bins(lmax)
+    binned = {k: dls[k][bins["BB" if k == "BB" else "TT"][:-1]] for k in dls}   # D at the first multipole of each bin
+    gs = JointGibbs(data, noise_T, noise_P, fwhm, a.nside, lmax, n_iter=1, mask=maskT, mask_pol=maskP, bins=bins, seed=11)
+    gs.run(binned)
+    gs.n_iter = a.gibbs_iters
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    gs.run(binned)
+    torch.cuda.synchronize()
+    gibbs_s = time.perf_counter() - t0
+    unfolded = {k: utils.unfold_bins(v, bins["BB" if k == "BB" else "TT"]) for k, v in binned.items()}
+    sky, _ = gs.constrained_sampler.sample(unfolded)
+    per_l = JointClsSampler(lmax, seed=12)
+    ch = gs.cls_sampler.empirical(sky)
+    nt = len(bins["TT"]) - 1
+    out = [torch.empty(nt, dtype=torch.float64, device="cuda") for _ in range(3)]
+    e_tt = _dev.i32(bins["TT"])
+    L = _lib.lib()
+
+    def kernel():
+        _lib.check(L.gs_cls_invwishart_binned(*[_dev.ptr(ch[k]) for k in ("TT", "TE", "EE")], lmax, _dev.ptr(e_tt), nt, None,
+                                              gs.cls_sampler.rng.seed, 1, *[_dev.ptr(o) for o in out], _dev.stream()))
+
+    return {
+        "what": "binned joint T/E/B sampler: masked JointGibbs(bins=) and the binned C_l step (gs_cls_invwishart_binned + "
+                "gs_cls_invgamma)",
+        "nside": a.nside, "lmax": lmax, "beam_fwhm_deg": fwhm,
+        "mask_T": "bench.make_mask galplane, f_sky 0.8", "mask_P": "bench.make_mask band, f_sky 0.8",
+        "noise": "isotropic per pixel: noise_P = %.4g (bench.py), noise_T = noise_P / 2" % noise_P,
+        "spectra": TT_FORMULA, "pcg_eps": gs.constrained_sampler.pcg_accuracy,
+        "bins": "TT/TE/EE: one l per bin to l = 30, width 10 above (%d bins); BB: bench.bins_for (%d bins)"
+                % (nt, len(bins["BB"]) - 1),
+        "joint_gibbs_binned_it_per_s": round(a.gibbs_iters / gibbs_s, 3), "joint_gibbs_iters_timed": a.gibbs_iters,
+        "cl_step_ms": {"binned": round(cuda_ms(lambda: gs.cls_sampler.sample(sky), a.nrep), 4),
+                       "per_l": round(cuda_ms(lambda: per_l.sample(sky), a.nrep), 4),
+                       "invwishart_binned_kernel": round(cuda_ms(kernel, a.nrep), 4)},
+        "cl_step_note": "CUDA events around nrep calls after one warm-up: JointClsSampler.sample (4 cross spectra, the TT/TE/EE "
+                        "draw, the BB draw and their host-side launches) and the binned inverse-Wishart launch alone",
+        "nrep": a.nrep,
+    }
 
 
 def gpu_info():
@@ -51,6 +116,7 @@ def main():
     ap.add_argument("--solves", type=int, default=3)
     ap.add_argument("--gibbs-iters", type=int, default=4)
     ap.add_argument("--nrep", type=int, default=20)
+    ap.add_argument("--bins", choices=("none", "planck"), default="none")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -82,6 +148,11 @@ def main():
     data = {"I": (mI + dev(rng.standard_normal(npix) * np.sqrt(noise_T))) * dev(maskT),
             "Q": (mQ + dev(rng.standard_normal(npix) * np.sqrt(noise_P))) * dev(maskP),
             "U": (mU + dev(rng.standard_normal(npix) * np.sqrt(noise_P))) * dev(maskP)}
+    if a.bins == "planck":
+        res = binned_report(a, data, noise_T, noise_P, fwhm, maskT, maskP, dls)
+        res.update(gpu_info())
+        emit(res, a.out)
+        return
     cr = JointConstrainedRealization(data, noise_T, noise_P, bl, lmax, npix, mask=maskT, mask_pol=maskP, seed=7)
     dd = {k: dev(v) for k, v in dls.items()}
 
@@ -150,11 +221,15 @@ def main():
         "per_iteration_ms_estimate": round(spin0 + spin2 + vec_ms, 4),
     }
     res.update(gpu_info())
+    emit(res, a.out)
+
+
+def emit(res, out):
     line = json.dumps(res)
     print(line)
-    if a.out:
-        os.makedirs(os.path.dirname(a.out) or ".", exist_ok=True)
-        with open(a.out, "a") as fh:
+    if out:
+        os.makedirs(os.path.dirname(out) or ".", exist_ok=True)
+        with open(out, "a") as fh:
             fh.write(line + "\n")
 
 
