@@ -7,7 +7,7 @@ import torch
 
 from . import _dev, _lib, utils
 from ._dev import f64, ptr, stream
-from ._lib import check
+from ._lib import check, GS_E_NOTCONVERGED
 from .ClsSampler import ClsSampler
 from .ConstrainedRealization import ConstrainedRealization
 from .GibbsSampler import GibbsSampler
@@ -140,7 +140,7 @@ class PolarizedCenteredConstrainedRealization(ConstrainedRealization):
                                       0 if x0 is None else 1, self.pcg_accuracy, self.pcg_itermax,
                                       self.pcg_check_every, C.byref(nit), C.byref(res), stream())
         self.last_pcg_iterations, self.last_pcg_residual = nit.value, res.value
-        if rc not in (0, -3):  # GS_E_NOTCONVERGED (-3) is reported through last_pcg_residual: qcinv also just stops at iter_max
+        if rc not in (0, GS_E_NOTCONVERGED):  # GS_E_NOTCONVERGED is reported through last_pcg_residual: qcinv also just stops at iter_max
             check(rc)
         return xe, xb
 
@@ -339,7 +339,7 @@ def sample_mask_batch(crs, dls_list, xis=None):
     rc = _lib.lib().gs_cr_pcg_pol_batch(a.plan._h, 2, ptr(dl[0]), ptr(dl[1]), ptr(a.bl_gauss_d), ptr(a.inv_noise_pol),
                                         a.ninv_sum_over_4pi, ptr(rhs[0, 0]), ptr(rhs[0, 1]), ptr(x[0, 0]), ptr(x[0, 1]), 2 * n,
                                         a.pcg_accuracy, a.pcg_itermax, a.pcg_check_every, nit, res, stream())
-    if rc not in (0, -3):
+    if rc not in (0, GS_E_NOTCONVERGED):
         check(rc)
     out = []
     for k, (cr, dls) in enumerate(zip(crs, dls_list)):

@@ -23,7 +23,7 @@ import torch
 
 from . import _dev, _lib
 from ._dev import f64, ptr, stream
-from ._lib import check, GS_ALM_REAL
+from ._lib import check, GS_ALM_REAL, GS_E_NOTCONVERGED
 
 
 class JointConstrainedRealization():
@@ -143,7 +143,7 @@ class JointConstrainedRealization():
                                       *[ptr(r) for r in rhs], *[ptr(v) for v in x], 0 if x0 is None else 1, self.pcg_accuracy,
                                       self.pcg_itermax, self.pcg_check_every, C.byref(nit), C.byref(res), stream())
         self.last_pcg_iterations, self.last_pcg_residual = nit.value, res.value
-        if rc not in (0, -3):  # GS_E_NOTCONVERGED (-3) is reported through last_pcg_residual, as in the E/B sampler
+        if rc not in (0, GS_E_NOTCONVERGED):  # GS_E_NOTCONVERGED is reported through last_pcg_residual, as in the E/B sampler
             check(rc)
         return x
 

@@ -18,7 +18,7 @@ import torch
 
 from . import _dev, _lib, utils
 from ._dev import f64, ptr, stream
-from ._lib import check, GS_ALM_REAL
+from ._lib import check, GS_ALM_REAL, GS_E_NOTCONVERGED
 from .ClsSampler import MHClsSampler
 from .ConstrainedRealization import ConstrainedRealization
 
@@ -70,7 +70,7 @@ class _TemperatureCR(ConstrainedRealization):
                                      ptr(rhs), ptr(x), 0 if x0 is None else 1, self.pcg_accuracy, self.pcg_itermax,
                                      self.pcg_check_every, C.byref(nit), C.byref(res), stream())
         self.last_pcg_iterations, self.last_pcg_residual = nit.value, res.value
-        if rc not in (0, -3):
+        if rc not in (0, GS_E_NOTCONVERGED):
             check(rc)
         return x
 

@@ -13,6 +13,8 @@ LIB_PATH = os.environ.get("GIBBS_B200_LIB") or os.path.join(_HERE, "csrc", "_bui
 GS_ALM_COMPLEX = 0
 GS_ALM_REAL = 1
 
+GS_E_NOTCONVERGED = -3   # a PCG solve stopped at its iteration limit (include/gibbs_b200.h)
+
 _lib = None
 
 _vp = C.c_void_p

@@ -146,7 +146,8 @@ struct gs_plan {
     double2* Fx;        // second spectra buffer (all-to-all peer of Fm) on sharded plans
     double* red_loc;    // 4 doubles: local partial sums / all-reduced sums of the sharded PCG
     std::vector<int> h_mlist, h_rings;
-    std::vector<void*> owned;  // device allocations to free
+    std::vector<void*> owned;       // device allocations to free
+    std::vector<void*> owned_host;  // pinned host allocations to free (cudaFreeHost)
     // job lists (device) for the ring-FFT stage
     RingJob* jobs2;  // spin 2: (Q,U) of each ring, heavy first
     int njobs2;

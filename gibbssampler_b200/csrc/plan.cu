@@ -369,6 +369,7 @@ extern "C" int gs_plan_destroy(gs_plan* p)
     if (p->work_event) cudaEventDestroy((cudaEvent_t)p->work_event);
     if (p->work_stream) cudaStreamDestroy((cudaStream_t)p->work_stream);
     for (void* d : p->owned) cudaFree(d);
+    for (void* h : p->owned_host) cudaFreeHost(h);
     cudaFree(p->mwg_F);
     cudaFree(p->mwg_maps);
     cudaFree(p->mwg_small);

@@ -310,8 +310,9 @@ static bool build_lof(gs_plan* p, const unsigned short** out)
 
 // ------------------------------------------------------------------ workspace
 // The workspaces belong to the plan (gs_plan::pcg_ws, pcg_ws_batch, pcg_ws_teb): created on the first solve, released by
-// gs_plan_destroy, which frees the device buffers recorded in p->owned and calls gs_pcg_ws_free for the rest.  A plan is used by
-// one host thread at a time (include/gibbs_b200.h), so no lock is taken.
+// gs_plan_destroy, which frees the device buffers recorded in p->owned and the pinned host buffers in p->owned_host and calls
+// gs_pcg_ws_free for the workspace structs.  A plan is used by one host thread at a time (include/gibbs_b200.h), so no lock is
+// taken.
 static bool alloc_owned(gs_plan* p, double** q, size_t cnt)
 {
     void* d = nullptr;
@@ -322,14 +323,18 @@ static bool alloc_owned(gs_plan* p, double** q, size_t cnt)
 }
 
 // the solver state on the device (in p->owned) and its pinned host copy with two slots (the graph path of a solve keeps two
-// polls in flight), released by the workspace's free function
+// polls in flight; in p->owned_host)
 static bool alloc_state(gs_plan* p, PcgState** state, PcgState** host_state)
 {
     void* d = nullptr;
     if (cudaMalloc(&d, sizeof(PcgState)) != cudaSuccess) return false;
     p->owned.push_back(d);
     *state = (PcgState*)d;
-    return cudaMallocHost((void**)host_state, 2 * sizeof(PcgState)) == cudaSuccess;
+    void* h = nullptr;
+    if (cudaMallocHost(&h, 2 * sizeof(PcgState)) != cudaSuccess) return false;
+    p->owned_host.push_back(h);
+    *host_state = (PcgState*)h;
+    return true;
 }
 
 static gs_pcg_ws* get_ws(gs_plan* p)
@@ -378,24 +383,6 @@ static gs_pcg_ws* get_ws_batch(gs_plan* p)
     return w;
 }
 
-static void teb_ws_free(gs_plan* p);
-void gs_pcg_ws_free(gs_plan* p)
-{
-    teb_ws_free(p);
-    gs_pcg_ws* w = (gs_pcg_ws*)p->pcg_ws;
-    if (w) {
-        if (w->host_state) cudaFreeHost(w->host_state);
-        delete w;
-        p->pcg_ws = nullptr;
-    }
-    gs_pcg_ws* b = (gs_pcg_ws*)p->pcg_ws_batch;
-    if (b) {
-        for (int k = 0; k < 2; ++k) if (b[k].host_state) cudaFreeHost(b[k].host_state);
-        delete[] b;
-        p->pcg_ws_batch = nullptr;
-    }
-}
-
 int g_gs_pcg_graph = 1;   // 1: the iterations between two convergence polls of an unsharded PCG solve are replayed from a CUDA graph
 extern "C" int gs_set_pcg_graph(int on) { const int old = g_gs_pcg_graph; g_gs_pcg_graph = on ? 1 : 0; return old; }
 int g_gs_ring_fused = 1;
@@ -438,6 +425,29 @@ static int apply_noise_op(gs_plan* p, const double* vE, const double* vB, const 
         if ((rc = gs_ring_anal(p, spin, p->mapQ_tmp, p->mapU_tmp, inv_noise, st, skip))) return rc;
     }
     return gs_leg_anal(p, spin, qE, qB, GS_ALM_REAL, bl, 1.0, 0, st, skip, nc, stride);
+}
+
+// Start of a solve: a zeroed solver state with the stopping rule, written to the pinned host slot and copied to the device on `st`
+static int pcg_state_reset(PcgState* state, PcgState* host_state, double eps, int itermax, cudaStream_t st)
+{
+    memset(host_state, 0, sizeof(PcgState));
+    host_state->eps2 = eps * eps;
+    host_state->itermax = itermax;
+    GS_CHECK_CUDA(cudaMemcpyAsync(state, host_state, sizeof(PcgState), cudaMemcpyHostToDevice, st));
+    return GS_OK;
+}
+
+// End of a solve: iterations and |r|/|r0| to the caller, GS_E_NOTCONVERGED if iter_max came first.  chain >= 0: the solve is
+// that chain of a batch, which the message names.
+static int pcg_report(const PcgState& s, double eps, int itermax, int chain, int* n_iter_out, double* resid_out)
+{
+    const double rel = s.d0 > 0.0 ? sqrt(s.rr / s.d0) : 0.0;
+    if (n_iter_out) *n_iter_out = s.iter;
+    if (resid_out) *resid_out = rel;
+    if (!(s.d0 > 0.0 && s.rr > s.eps2 * s.d0)) return GS_OK;
+    if (chain < 0) gs_set_error("PCG stopped at iter_max = %d with |r|/|r0| = %.3e > eps = %.1e", itermax, rel, eps);
+    else gs_set_error("PCG (chain %d of the batch) stopped at iter_max = %d with |r|/|r0| = %.3e > eps = %.1e", chain, itermax, rel, eps);
+    return GS_E_NOTCONVERGED;
 }
 
 // The poll loop shared by the PCG solves: `iteration(stream)` enqueues one PCG iteration whose launches take every scalar
@@ -530,14 +540,7 @@ static int pcg_poll_loop(gs_plan* p, cudaStream_t st, PcgState* state, PcgState*
         finished = host_state->done || launched >= itermax;
     }
     if (gexec) cudaGraphExecDestroy(gexec);
-    const PcgState& s = *host_state;
-    if (n_iter_out) *n_iter_out = s.iter;
-    if (resid_out) *resid_out = s.d0 > 0.0 ? sqrt(s.rr / s.d0) : 0.0;
-    if (s.d0 > 0.0 && s.rr > s.eps2 * s.d0) {
-        gs_set_error("PCG stopped at iter_max = %d with |r|/|r0| = %.3e > eps = %.1e", itermax, sqrt(s.rr / s.d0), eps);
-        return GS_E_NOTCONVERGED;
-    }
-    return GS_OK;
+    return pcg_report(*host_state, eps, itermax, -1, n_iter_out, resid_out);
 }
 
 // spin 2: (E, B) system; spin 0: temperature (dl_BB, rhs_B, x_B unused)
@@ -566,12 +569,7 @@ static int cr_pcg_impl(gs_plan* p, int spin, const double* dl_EE, const double* 
     ActiveRings act(p);
     if ((rc = act.begin(inv_noise, st))) return rc;
 
-    PcgState h;
-    memset(&h, 0, sizeof(h));
-    h.eps2 = eps * eps;
-    h.itermax = itermax;
-    *w->host_state = h;
-    GS_CHECK_CUDA(cudaMemcpyAsync(w->state, w->host_state, sizeof(PcgState), cudaMemcpyHostToDevice, st));
+    if ((rc = pcg_state_reset(w->state, w->host_state, eps, itermax, st))) return rc;
     if (warm_start) {  // r0 = b - Q x0
         if ((rc = apply_noise_op(p, x_E, x_B, bl, inv_noise, w->q[0], w->q[1], st, nullptr, spin))) return rc;
         add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->ic_l[0], w->lof, x_E, w->q[0], n);
@@ -657,12 +655,7 @@ extern "C" int gs_cr_pcg_pol_batch(gs_plan* p, int n_chain, const double* dl_EE,
         precond_kernel<<<lb, 256, 0, st>>>(dl_EE + k * (L + 1), bl, ninv_sum_over_4pi, L, w->ic_l[0], w->pre_l[0]);
         precond_kernel<<<lb, 256, 0, st>>>(dl_BB + k * (L + 1), bl, ninv_sum_over_4pi, L, w->ic_l[1], w->pre_l[1]);
         GS_CHECK_LAUNCH();
-        PcgState h;
-        memset(&h, 0, sizeof(h));
-        h.eps2 = eps * eps;
-        h.itermax = itermax;
-        *w->host_state = h;
-        GS_CHECK_CUDA(cudaMemcpyAsync(w->state, w->host_state, sizeof(PcgState), cudaMemcpyHostToDevice, st));
+        if ((rc = pcg_state_reset(w->state, w->host_state, eps, itermax, st))) return rc;
         zero2_kernel<<<SV_GRID, SV_NT, 0, st>>>(x_E + k * stride, x_B + k * stride, n);
         pcg_init_kernel<<<SV_GRID, SV_NT, 0, st>>>(*w, rhs_E + k * stride, rhs_B + k * stride, 0, n, 2);
         GS_CHECK_LAUNCH();
@@ -693,16 +686,10 @@ extern "C" int gs_cr_pcg_pol_batch(gs_plan* p, int n_chain, const double* dl_EE,
         GS_CHECK_CUDA(cudaStreamSynchronize(st));
         for (int k = 0; k < 2; ++k) done[k] = W[k].host_state->done != 0;
     }
-    int ret = GS_OK;
-    for (int k = 0; k < 2; ++k) {
-        const PcgState& sdone = *W[k].host_state;
-        if (n_iter_out) n_iter_out[k] = sdone.iter;
-        if (resid_out) resid_out[k] = sdone.d0 > 0.0 ? sqrt(sdone.rr / sdone.d0) : 0.0;
-        if (sdone.d0 > 0.0 && sdone.rr > sdone.eps2 * sdone.d0) {
-            gs_set_error("PCG (chain %d of the batch) stopped at iter_max = %d with |r|/|r0| = %.3e > eps = %.1e", k, itermax, sqrt(sdone.rr / sdone.d0), eps);
+    int ret = GS_OK;   // both chains are reported; GS_E_NOTCONVERGED if either stopped at iter_max
+    for (int k = 0; k < 2; ++k)
+        if (pcg_report(*W[k].host_state, eps, itermax, k, n_iter_out ? n_iter_out + k : nullptr, resid_out ? resid_out + k : nullptr))
             ret = GS_E_NOTCONVERGED;
-        }
-    }
     return ret;
 }
 
@@ -718,11 +705,11 @@ extern "C" int gs_cr_pcg_tt(gs_plan* p, const double* dl_TT, const double* bl, c
                        check_every, n_iter_out, resid_out, stream);
 }
 
-extern "C" int gs_cr_apply_q_tt(gs_plan* p, const double* dl_TT, const double* bl, const double* inv_noise, const double* x,
-                                double* y, void* stream)
+// gs_cr_apply_q_pol (spin 2) and gs_cr_apply_q_tt (spin 0: temperature in the E slots, the B arguments unused)
+static int apply_q_impl(gs_plan* p, int spin, const double* dl_E, const double* dl_B, const double* bl, const double* inv_noise,
+                        const double* x_E, const double* x_B, double* y_E, double* y_B, void* stream)
 {
-    if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
-    GS_REQUIRE(dl_TT && bl && inv_noise && x && y, "null pointer argument");
+    const int nc = spin ? 2 : 1;
     GS_CHECK_CUDA(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
     gs_pcg_ws* w = get_ws(p);
@@ -731,11 +718,61 @@ extern "C" int gs_cr_apply_q_tt(gs_plan* p, const double* dl_TT, const double* b
     ActiveRings act(p);
     if ((rc = act.begin(inv_noise, st))) return rc;
     const int L = p->d.lmax;
-    precond_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_TT, bl, 0.0, L, w->ic_l[0], w->pre_l[0]);   // only C^-1 is read
-    if ((rc = apply_noise_op(p, x, nullptr, bl, inv_noise, w->q[0], nullptr, st, nullptr, 0))) return rc;
-    add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->ic_l[0], w->lof, x, y, p->nreal_loc);
+    const double* dl[2] = {dl_E, dl_B};
+    const double* x[2] = {x_E, x_B};
+    double* y[2] = {y_E, y_B};
+    for (int c = 0; c < nc; ++c)
+        precond_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl[c], bl, 0.0, L, w->ic_l[c], w->pre_l[c]);   // only C^-1 is read
+    if ((rc = apply_noise_op(p, x_E, x_B, bl, inv_noise, w->q[0], spin ? w->q[1] : nullptr, st, nullptr, spin))) return rc;
+    for (int c = 0; c < nc; ++c) add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[c], w->ic_l[c], w->lof, x[c], y[c], p->nreal_loc);
     GS_CHECK_LAUNCH();
     return GS_OK;
+}
+
+// gs_cr_rhs_pol (spin 2) and gs_cr_rhs_tt (spin 0: the temperature maps in the Q slots, its coefficients in the E slots, the
+// U and B arguments unused).  The data term is computed from the maps when bdata_E is NULL.
+static int rhs_impl(gs_plan* p, int spin, const double* dl_E, const double* dl_B, const double* bl, const double* inv_noise,
+                    const double* sqrt_inv_noise, const double* bdata_E, const double* bdata_B, const double* d_Q, const double* d_U,
+                    const double* xi_Q, const double* xi_U, const double* xi_E, const double* xi_B, int fluct_iter, double* rhs_E,
+                    double* rhs_B, void* stream)
+{
+    const int nc = spin ? 2 : 1;
+    GS_CHECK_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    gs_pcg_ws* w = get_ws(p);
+    if (!w) return GS_E_NOMEM;
+    auto map2alm = [&](const double* mQ, const double* mU, const double* pixw, int iter, int adjoint, double* aE, double* aB) {
+        return spin ? gs_map2alm_spin2(p, mQ, mU, pixw, iter, adjoint, bl, aE, aB, GS_ALM_REAL, stream)
+                    : gs_map2alm_spin0(p, mQ, pixw, iter, adjoint, bl, aE, GS_ALM_REAL, stream);
+    };
+    int rc;
+    // fluctuation term 1: utils.adjoint_synthesis_hp (utils.py:79-111) = bl * (Npix/4pi) * map2alm(iter=3)
+    if ((rc = map2alm(xi_Q, xi_U, sqrt_inv_noise, fluct_iter, 0, rhs_E, rhs_B))) return rc;
+    const double resc = (double)p->d.npix / (4.0 * 3.14159265358979323846);
+    // fluctuation term 2 and data term; use r[] / p[] of the PCG workspace as scratch
+    const double* dl[2] = {dl_E, dl_B};
+    for (int c = 0; c < nc; ++c)
+        if ((rc = gs_plan_expand_per_l(p, dl[c], 4, w->r[c], st))) return rc;
+    const double* bd[2] = {bdata_E, bdata_B};
+    if (!bdata_E) {
+        if ((rc = map2alm(d_Q, d_U, inv_noise, 0, 1, w->p[0], w->p[1]))) return rc;
+        bd[0] = w->p[0];
+        bd[1] = w->p[1];
+    }
+    // rhs = resc * rhs + sqrt(C^-1) xi + bdata
+    const double* xi[2] = {xi_E, xi_B};
+    double* rhs[2] = {rhs_E, rhs_B};
+    for (int c = 0; c < nc; ++c) rhs_combine_kernel<<<SV_GRID, SV_NT, 0, st>>>(rhs[c], w->r[c], xi[c], bd[c], resc, p->nreal_loc);
+    GS_CHECK_LAUNCH();
+    return GS_OK;
+}
+
+extern "C" int gs_cr_apply_q_tt(gs_plan* p, const double* dl_TT, const double* bl, const double* inv_noise, const double* x,
+                                double* y, void* stream)
+{
+    if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
+    GS_REQUIRE(dl_TT && bl && inv_noise && x && y, "null pointer argument");
+    return apply_q_impl(p, 0, dl_TT, nullptr, bl, inv_noise, x, nullptr, y, nullptr, stream);
 }
 
 // Right-hand side of the temperature system (CenteredGibbs.py:145-147, NonCenteredGibbs.py:61-63; RNG order xi_alm, xi_pix):
@@ -749,22 +786,8 @@ extern "C" int gs_cr_rhs_tt(gs_plan* p, const double* dl_TT, const double* bl, c
     GS_REQUIRE(dl_TT && bl && inv_noise && sqrt_inv_noise && xi_alm && xi_pix && rhs, "null pointer argument");
     GS_REQUIRE(bdata || d, "need either the precomputed data term or the data map");
     GS_REQUIRE(fluct_iter >= 0, "fluct_iter must be >= 0");
-    GS_CHECK_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    gs_pcg_ws* w = get_ws(p);
-    if (!w) return GS_E_NOMEM;
-    int rc;
-    if ((rc = gs_map2alm_spin0(p, xi_pix, sqrt_inv_noise, fluct_iter, 0, bl, rhs, GS_ALM_REAL, stream))) return rc;
-    const double resc = (double)p->d.npix / (4.0 * 3.14159265358979323846);
-    if ((rc = gs_plan_expand_per_l(p, dl_TT, 4, w->r[0], st))) return rc;
-    const double* bd = bdata;
-    if (!bd) {
-        if ((rc = gs_map2alm_spin0(p, d, inv_noise, 0, 1, bl, w->p[0], GS_ALM_REAL, stream))) return rc;
-        bd = w->p[0];
-    }
-    rhs_combine_kernel<<<SV_GRID, SV_NT, 0, st>>>(rhs, w->r[0], xi_alm, bd, resc, p->nreal_loc);
-    GS_CHECK_LAUNCH();
-    return GS_OK;
+    return rhs_impl(p, 0, dl_TT, nullptr, bl, inv_noise, sqrt_inv_noise, bdata, nullptr, d, nullptr, xi_pix, nullptr, xi_alm, nullptr,
+                    fluct_iter, rhs, nullptr, stream);
 }
 
 // y = Q x = C^-1 x + B A^T N^-1 A B x   (qcinv opfilt_pp.fwd_op; CenteredGibbs.py:629, 651-656)
@@ -774,22 +797,7 @@ extern "C" int gs_cr_apply_q_pol(gs_plan* p, const double* dl_EE, const double* 
 {
     if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
     GS_REQUIRE(dl_EE && dl_BB && bl && inv_noise && x_E && x_B && y_E && y_B, "null pointer argument");
-    GS_CHECK_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    gs_pcg_ws* w = get_ws(p);
-    if (!w) return GS_E_NOMEM;
-    const int64_t n = p->nreal_loc;
-    int rc;
-    ActiveRings act(p);
-    if ((rc = act.begin(inv_noise, st))) return rc;
-    const int L = p->d.lmax;
-    precond_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_EE, bl, 0.0, L, w->ic_l[0], w->pre_l[0]);   // only C^-1 is read
-    precond_kernel<<<(L + 256) / 256, 256, 0, st>>>(dl_BB, bl, 0.0, L, w->ic_l[1], w->pre_l[1]);
-    if ((rc = apply_noise_op(p, x_E, x_B, bl, inv_noise, w->q[0], w->q[1], st, nullptr))) return rc;
-    add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[0], w->ic_l[0], w->lof, x_E, y_E, n);
-    add_cinv_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->q[1], w->ic_l[1], w->lof, x_B, y_B, n);
-    GS_CHECK_LAUNCH();
-    return GS_OK;
+    return apply_q_impl(p, 2, dl_EE, dl_BB, bl, inv_noise, x_E, x_B, y_E, y_B, stream);
 }
 
 // Right-hand side of the masked-sky system (CenteredGibbs.py:469-483, RNG order xi_Q, xi_U, xi_E, xi_B):
@@ -807,32 +815,9 @@ extern "C" int gs_cr_rhs_pol(gs_plan* p, const double* dl_EE, const double* dl_B
                "null pointer argument");
     GS_REQUIRE((bdata_E && bdata_B) || (d_Q && d_U), "need either the precomputed data term or the data maps");
     GS_REQUIRE(fluct_iter >= 0, "fluct_iter must be >= 0");
-    GS_CHECK_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    gs_pcg_ws* w = get_ws(p);
-    if (!w) return GS_E_NOMEM;
-    const int64_t n = p->nreal_loc;
-    int rc;
-    // fluctuation term 1: utils.adjoint_synthesis_hp (utils.py:79-111) = bl * (Npix/4pi) * map2alm(iter=3)
-    if ((rc = gs_map2alm_spin2(p, xi_Q, xi_U, sqrt_inv_noise, fluct_iter, 0, bl, rhs_E, rhs_B, GS_ALM_REAL, stream))) return rc;
-    const double resc = (double)p->d.npix / (4.0 * 3.14159265358979323846);
-    // fluctuation term 2 and data term; use r[] / p[] of the PCG workspace as scratch
-    if ((rc = gs_plan_expand_per_l(p, dl_EE, 4, w->r[0], st))) return rc;
-    if ((rc = gs_plan_expand_per_l(p, dl_BB, 4, w->r[1], st))) return rc;
-    const double* bdE = bdata_E;
-    const double* bdB = bdata_B;
-    if (!bdE) {
-        if ((rc = gs_map2alm_spin2(p, d_Q, d_U, inv_noise, 0, 1, bl, w->p[0], w->p[1], GS_ALM_REAL, stream))) return rc;
-        bdE = w->p[0];
-        bdB = w->p[1];
-    }
-    // rhs = resc * rhs + sqrt(C^-1) xi + bdata
-    rhs_combine_kernel<<<SV_GRID, SV_NT, 0, st>>>(rhs_E, w->r[0], xi_E, bdE, resc, n);
-    rhs_combine_kernel<<<SV_GRID, SV_NT, 0, st>>>(rhs_B, w->r[1], xi_B, bdB, resc, n);
-    GS_CHECK_LAUNCH();
-    return GS_OK;
+    return rhs_impl(p, 2, dl_EE, dl_BB, bl, inv_noise, sqrt_inv_noise, bdata_E, bdata_B, d_Q, d_U, xi_Q, xi_U, xi_E, xi_B, fluct_iter,
+                    rhs_E, rhs_B, stream);
 }
-
 
 // ------------------------------------------------------------------ joint T/E/B system on a cut sky
 // qcinv's joint T+P filter (opfilt_tp upstream; not vendored, restated here): the (T, E, B) coefficients of every (l, m) are
@@ -1101,13 +1086,12 @@ static TebWs* get_ws_teb(gs_plan* p)
     return w;
 }
 
-static void teb_ws_free(gs_plan* p)
+void gs_pcg_ws_free(gs_plan* p)
 {
-    TebWs* w = (TebWs*)p->pcg_ws_teb;
-    if (!w) return;
-    if (w->host_state) cudaFreeHost(w->host_state);
-    delete w;
-    p->pcg_ws_teb = nullptr;
+    delete (gs_pcg_ws*)p->pcg_ws;
+    delete[] (gs_pcg_ws*)p->pcg_ws_batch;
+    delete (TebWs*)p->pcg_ws_teb;
+    p->pcg_ws = p->pcg_ws_batch = p->pcg_ws_teb = nullptr;
 }
 
 // Two weight maps, one set of plan-wide ring flags: the Legendre and ring launchers read act_ring / act_pairs / act_slot0 /
@@ -1204,12 +1188,7 @@ extern "C" int gs_cr_pcg_teb(gs_plan* p, const double* dl_TT, const double* dl_T
     TebRings tr(p);
     if ((rc = tr.begin(inv_noise_T, inv_noise_P, st))) return rc;
 
-    PcgState h;
-    memset(&h, 0, sizeof(h));
-    h.eps2 = eps * eps;
-    h.itermax = itermax;
-    *w->host_state = h;
-    GS_CHECK_CUDA(cudaMemcpyAsync(w->state, w->host_state, sizeof(PcgState), cudaMemcpyHostToDevice, st));
+    if ((rc = pcg_state_reset(w->state, w->host_state, eps, itermax, st))) return rc;
     if (warm_start) {  // r0 = b - Q x0
         if ((rc = teb_noise_op(p, tr, x_T, x_E, x_B, bl, inv_noise_T, inv_noise_P, w->q[0], w->q[1], w->q[2], st, nullptr))) return rc;
     } else {
@@ -1367,6 +1346,45 @@ extern "C" int gs_profile_matvec_teb(gs_plan* p, const double* bl, const double*
 long long g_gs_launches = 0;
 extern "C" long long gs_launch_count(void) { return g_gs_launches; }
 
+// Times the stages of one PCG mat-vec with CUDA events on `st`, averaged over nrep: ms_out[0] Legendre synthesis, then the ring
+// stage (split_ring: ring synthesis and ring analysis with N^-1 as two stages; otherwise the fused ring stage), then Legendre
+// analysis + finish.  n_chain right-hand sides at x / y + c stride (doubles) per launch; the times are for the whole batch.
+static int profile_matvec(gs_plan* p, int n_chain, int64_t stride, bool split_ring, const double* x_E, const double* x_B,
+                          const double* bl, const double* inv_noise, double* y_E, double* y_B, int nrep, float* ms_out,
+                          cudaStream_t st, const char* who)
+{
+    const int ns = split_ring ? 4 : 3;
+    cudaEvent_t ev[5];
+    for (int i = 0; i <= ns; ++i) GS_CHECK_CUDA(cudaEventCreate(&ev[i]));
+    double acc[4] = {0, 0, 0, 0};
+    int rc;
+    {
+        ActiveRings act(p);   // as in the PCG: rings without weight are skipped unless gs_set_ring_skip(0)
+        rc = act.begin(inv_noise, st);
+        for (int r = 0; r < nrep && rc == GS_OK; ++r) {
+            int e = 0;
+            cudaEventRecord(ev[e++], st);
+            rc = gs_leg_synth(p, 2, x_E, x_B, GS_ALM_REAL, bl, st, nullptr, nullptr, n_chain, stride);
+            cudaEventRecord(ev[e++], st);
+            if (split_ring) {
+                if (!rc) rc = gs_ring_synth(p, 2, p->mapQ_tmp, p->mapU_tmp, st);
+                cudaEventRecord(ev[e++], st);
+                if (!rc) rc = gs_ring_anal(p, 2, p->mapQ_tmp, p->mapU_tmp, inv_noise, st);
+            } else if (!rc) {
+                rc = gs_ring_apply(p, 2, inv_noise, st, nullptr, n_chain);
+            }
+            cudaEventRecord(ev[e++], st);
+            if (!rc) rc = gs_leg_anal(p, 2, y_E, y_B, GS_ALM_REAL, bl, 1.0, 0, st, nullptr, n_chain, stride);
+            cudaEventRecord(ev[e], st);
+            if (cudaEventSynchronize(ev[e]) != cudaSuccess) { gs_set_error("%s: %s", who, cudaGetErrorString(cudaGetLastError())); rc = GS_E_CUDA; break; }
+            for (int i = 0; i < ns; ++i) { float ms = 0; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); acc[i] += ms; }
+        }
+    }
+    for (int i = 0; i < ns; ++i) ms_out[i] = (float)(acc[i] / nrep);
+    for (int i = 0; i <= ns; ++i) cudaEventDestroy(ev[i]);
+    return rc;
+}
+
 // Times the four kernels of one PCG mat-vec (Legendre synthesis, ring synthesis, ring analysis with
 // fused N^-1, Legendre analysis + finish) with CUDA events on the launching stream; ms_out[0..3]
 // receive the average duration of each stage over nrep repetitions.
@@ -1377,30 +1395,10 @@ extern "C" int gs_profile_matvec(gs_plan* p, const double* x_E, const double* x_
     if (!p) { gs_set_error("null plan"); return GS_E_BADARG; }
     GS_REQUIRE(x_E && x_B && bl && inv_noise && y_E && y_B && ms_out && nrep >= 1, "bad arguments");
     GS_CHECK_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaEvent_t ev[5];
-    for (int i = 0; i < 5; ++i) GS_CHECK_CUDA(cudaEventCreate(&ev[i]));
-    double acc[4] = {0, 0, 0, 0};
-    int rc = GS_OK;
-    ActiveRings act(p);   // as in the PCG: rings without weight are skipped unless gs_set_ring_skip(0)
-    if ((rc = act.begin(inv_noise, st))) { for (int i = 0; i < 5; ++i) cudaEventDestroy(ev[i]); return rc; }
-    for (int r = 0; r < nrep && rc == GS_OK; ++r) {
-        cudaEventRecord(ev[0], st);
-        rc = gs_leg_synth(p, 2, x_E, x_B, GS_ALM_REAL, bl, st);
-        cudaEventRecord(ev[1], st);
-        // fused ring stage (the PCG's own path): reported as stage 1, stage 2 = 0
-        if (!rc) rc = g_gs_ring_fused ? gs_ring_apply(p, 2, inv_noise, st) : gs_ring_synth(p, 2, p->mapQ_tmp, p->mapU_tmp, st);
-        cudaEventRecord(ev[2], st);
-        if (!rc && !g_gs_ring_fused) rc = gs_ring_anal(p, 2, p->mapQ_tmp, p->mapU_tmp, inv_noise, st);
-        cudaEventRecord(ev[3], st);
-        if (!rc) rc = gs_leg_anal(p, 2, y_E, y_B, GS_ALM_REAL, bl, 1.0, 0, st);
-        cudaEventRecord(ev[4], st);
-        if (cudaEventSynchronize(ev[4]) != cudaSuccess) { gs_set_error("gs_profile_matvec: %s", cudaGetErrorString(cudaGetLastError())); rc = GS_E_CUDA; break; }
-        for (int i = 0; i < 4; ++i) { float ms = 0; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); acc[i] += ms; }
-    }
-    for (int i = 0; i < 4; ++i) ms_out[i] = (float)(acc[i] / nrep);
-    if (g_gs_ring_fused) ms_out[2] = 0.0f;
-    for (int i = 0; i < 5; ++i) cudaEventDestroy(ev[i]);
+    const int rc = profile_matvec(p, 1, 0, !g_gs_ring_fused, x_E, x_B, bl, inv_noise, y_E, y_B, nrep, ms_out, (cudaStream_t)stream,
+                                  __func__);
+    // fused ring stage (the PCG's own path): reported as stage 1, stage 2 = 0
+    if (g_gs_ring_fused) { ms_out[3] = ms_out[2]; ms_out[2] = 0.0f; }
     return rc;
 }
 
@@ -1415,29 +1413,7 @@ extern "C" int gs_profile_matvec_batch(gs_plan* p, int n_chain, const double* x_
     GS_CHECK_CUDA(cudaSetDevice(p->device));
     int rc;
     if (n_chain > 1 && (rc = gs_plan_reserve_chains(p, n_chain))) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaEvent_t ev[4];
-    for (int i = 0; i < 4; ++i) GS_CHECK_CUDA(cudaEventCreate(&ev[i]));
-    double acc[3] = {0, 0, 0};
-    rc = GS_OK;
-    {
-        ActiveRings act(p);
-        rc = act.begin(inv_noise, st);
-        for (int r = 0; r < nrep && rc == GS_OK; ++r) {
-            cudaEventRecord(ev[0], st);
-            rc = gs_leg_synth(p, 2, x_E, x_B, GS_ALM_REAL, bl, st, nullptr, nullptr, n_chain, stride);
-            cudaEventRecord(ev[1], st);
-            if (!rc) rc = gs_ring_apply(p, 2, inv_noise, st, nullptr, n_chain);
-            cudaEventRecord(ev[2], st);
-            if (!rc) rc = gs_leg_anal(p, 2, y_E, y_B, GS_ALM_REAL, bl, 1.0, 0, st, nullptr, n_chain, stride);
-            cudaEventRecord(ev[3], st);
-            if (cudaEventSynchronize(ev[3]) != cudaSuccess) { gs_set_error("gs_profile_matvec_batch: %s", cudaGetErrorString(cudaGetLastError())); rc = GS_E_CUDA; break; }
-            for (int i = 0; i < 3; ++i) { float ms = 0; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); acc[i] += ms; }
-        }
-    }
-    for (int i = 0; i < 3; ++i) ms_out[i] = (float)(acc[i] / nrep);
-    for (int i = 0; i < 4; ++i) cudaEventDestroy(ev[i]);
-    return rc;
+    return profile_matvec(p, n_chain, stride, false, x_E, x_B, bl, inv_noise, y_E, y_B, nrep, ms_out, (cudaStream_t)stream, __func__);
 }
 
 // Times the three vector kernels of one PCG iteration (q += C^-1 p with <p,q>; x, r update with <r,r>, <r,Mr>; p = M r + beta p)

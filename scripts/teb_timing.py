@@ -187,7 +187,7 @@ def main():
                              cr.ninvP_sum_over_4pi, _dev.ptr(rhs[1]), _dev.ptr(rhs[2]), _dev.ptr(xe), _dev.ptr(xb), 0, cr.pcg_accuracy,
                              cr.pcg_itermax, 8, C.byref(nit), C.byref(res), _dev.stream())
         torch.cuda.synchronize()
-        if rc not in (0, -3):
+        if rc not in (0, _lib.GS_E_NOTCONVERGED):
             _lib.check(rc)
         if k:
             eb_ms.append((time.perf_counter() - t0) * 1e3)

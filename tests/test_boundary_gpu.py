@@ -119,8 +119,8 @@ def test_remove_monopole_dipole_contributions():
 
 
 def test_plan_create_solve_destroy_cycles():
-    """ADVICE r1: the PCG workspace lives in the plan and dies with it (no pointer-keyed cache): create, solve, destroy,
-    create at the same or another size, solve again."""
+    """ADVICE r1: the PCG workspaces live in the plan and die with it (no pointer-keyed cache): create, solve (E/B, a two-chain
+    E/B batch, joint T/E/B), destroy, create at the same or another size, solve again."""
     from gibbssampler_b200 import _lib, _dev
     L = _lib.lib()
     th, _ = O.pix_angles(NSIDE)
@@ -132,22 +132,38 @@ def test_plan_create_solve_destroy_cycles():
         npix, nre = 12 * nside ** 2, (lmax + 1) ** 2
         g = np.random.default_rng(7)
         ell = np.arange(lmax + 1)
-        dl = _dev.f64(np.where(ell >= 2, 1.0 + 0.1 * ell, 0.0))
+        dl_np = np.where(ell >= 2, 1.0 + 0.1 * ell, 0.0)
+        dl, dl_te = _dev.f64(dl_np), _dev.f64(0.3 * dl_np)
+        dl2 = _dev.f64(np.stack([dl_np, 0.5 * dl_np]))   # [chain][l]
         bl = _dev.f64(O.gauss_beam(np.radians(8.0), lmax))
         invn = _dev.f64(np.full(npix, 20.0))
-        rhs_e, rhs_b = _dev.f64(g.standard_normal(nre)), _dev.f64(g.standard_normal(nre))
-        for a in (rhs_e, rhs_b):
-            a[[0, 1, lmax + 1, lmax + 2]] = 0
+        ninv = float(invn.sum().item()) / (4 * np.pi)
+        rhs = _dev.f64(g.standard_normal((3, nre)))   # E, B, T
+        rhs[:, [0, 1, lmax + 1, lmax + 2]] = 0
+        rhs_e, rhs_b, rhs_t = rhs
         xe, xb = torch.empty_like(rhs_e), torch.empty_like(rhs_b)
         nit, res = C.c_int(0), C.c_double(0)
-        rc = L.gs_cr_pcg_pol(h, _dev.ptr(dl), _dev.ptr(dl), _dev.ptr(bl), _dev.ptr(invn), float(invn.sum().item()) / (4 * np.pi),
+        rc = L.gs_cr_pcg_pol(h, _dev.ptr(dl), _dev.ptr(dl), _dev.ptr(bl), _dev.ptr(invn), ninv,
                              _dev.ptr(rhs_e), _dev.ptr(rhs_b), _dev.ptr(xe), _dev.ptr(xb), 0, 1e-10, 500, 8, C.byref(nit), C.byref(res),
                              _dev.stream())
         assert rc == 0 and res.value <= 1e-10
+        rhs2 = torch.stack([rhs[[0, 1]], rhs[[1, 0]]])   # [chain][E, B][nre]
+        x2 = torch.empty_like(rhs2)
+        nit2, res2 = (C.c_int * 2)(), (C.c_double * 2)()
+        rc = L.gs_cr_pcg_pol_batch(h, 2, _dev.ptr(dl2), _dev.ptr(dl2), _dev.ptr(bl), _dev.ptr(invn), ninv, _dev.ptr(rhs2[0, 0]),
+                                   _dev.ptr(rhs2[0, 1]), _dev.ptr(x2[0, 0]), _dev.ptr(x2[0, 1]), 2 * nre, 1e-10, 500, 8, nit2, res2,
+                                   _dev.stream())
+        assert rc == 0 and max(res2) <= 1e-10
+        x3 = torch.empty_like(rhs)   # T, E, B
+        rc = L.gs_cr_pcg_teb(h, _dev.ptr(dl), _dev.ptr(dl_te), _dev.ptr(dl), _dev.ptr(dl), _dev.ptr(bl), _dev.ptr(invn), _dev.ptr(invn),
+                             ninv, ninv, *[_dev.ptr(r) for r in (rhs_t, rhs_e, rhs_b)], *[_dev.ptr(v) for v in x3], 0, 1e-10, 500, 8,
+                             C.byref(nit), C.byref(res), _dev.stream())
+        assert rc == 0 and res.value <= 1e-10
         torch.cuda.synchronize()
-        sols.append((nside, xe.cpu().numpy().copy()))
+        sols.append([a.cpu().numpy().copy() for a in (xe, x2, x3)])
         _lib.check(L.gs_plan_destroy(h))
-    assert np.array_equal(sols[0][1], sols[2][1]) and np.array_equal(sols[2][1], sols[3][1])
+    for k in range(3):
+        assert np.array_equal(sols[0][k], sols[2][k]) and np.array_equal(sols[2][k], sols[3][k])
 
 
 def test_non_shard_aware_samplers_refuse_sharded_plans():
