@@ -18,6 +18,7 @@ class CenteredClsSampler(ClsSampler):
 
     def sample(self, alms):
         out = self._invgamma_draw(f64(alms), self.bins)
+        self.last_sigma = {"TT": self._last_cl}
         return out if isinstance(alms, torch.Tensor) else out.cpu().numpy()
 
 
@@ -31,7 +32,9 @@ class PolarizedCenteredClsSampler(ClsSampler):
     def sample(self, alms):
         host = not isinstance(alms["EE"], torch.Tensor)
         ee = self.sample_one_pol(alms["EE"], "EE")
+        cl_ee = self._last_cl
         bb = self.sample_one_pol(alms["BB"], "BB")
+        self.last_sigma = {"EE": cl_ee, "BB": self._last_cl}
         if host:
             return {"EE": ee.cpu().numpy(), "BB": bb.cpu().numpy()}
         return {"EE": ee, "BB": bb}
@@ -259,10 +262,16 @@ class PolarizedCenteredConstrainedRealization(ConstrainedRealization):
 class CenteredGibbs(GibbsSampler):
     def __init__(self, pix_map, noise_temp, noise_pol, beam, nside, lmax, Npix, mask_path=None,
                  polarization=False, bins=None, n_iter=100000, rj_step=False, all_sph=False, gibbs_cr=False,
-                 overrelaxation=False, ula=False, *, mask=None, rng="philox", seed=None, verbose=False, plan=None):
+                 overrelaxation=False, ula=False, *, mask=None, rng="philox", seed=None, verbose=False, plan=None, keep_sigma=False):
         """`plan` = a gibbssampler_b200.sharded.ShardedPlan runs this single chain m-sharded over the GPUs of the
         plan's process group (BASELINE config #4); inputs are full-sky arrays as usual, sky maps returned by the
-        constrained sampler are local alm shards (plan.gather_alm reassembles them)."""
+        constrained sampler are local alm shards (plan.gather_alm reassembles them).
+        keep_sigma=True: run() also leaves sigma_history = {"TT"} or {"EE", "BB"}: (n_iter, lmax + 1) numpy arrays whose row i is
+        the empirical spectrum of the sky drawn in iteration i (the sky row i + 1 of the D history was drawn from), the input of
+        BlackwellRao.  Not available with a sharded plan (any world size), in run_fused or in multichain.run_chains."""
+        if keep_sigma and plan is not None:
+            raise _lib.GibbsB200Error("keep_sigma is not available with a sharded plan: the chain's spectra are not recorded there")
+        self.keep_sigma = bool(keep_sigma)
         super().__init__(pix_map, noise_temp, beam, nside, lmax, polarization=polarization, bins=bins, n_iter=n_iter,
                          rj_step=rj_step, gibbs_cr=gibbs_cr, verbose=verbose)
         shared = _dev.Rng(rng, seed)
@@ -290,6 +299,8 @@ class CenteredGibbs(GibbsSampler):
         hold the mean.  Philox draws only (numpy-stream parity is what run() is for)."""
         import time
         cr = self.constrained_sampler
+        if self.keep_sigma:
+            raise _lib.GibbsB200Error("run_fused does not record the sky spectra: use run() for a chain built with keep_sigma=True")
         if not self.polarization or cr.masked or cr.d_E is None or cr.plan.world > 1 or cr.rng.mode != "philox":
             raise _lib.GibbsB200Error("run_fused: polarised full-sky chain with harmonic data (pix_map['EE'/'BB']) and Philox draws only")
         bins = {k: torch.as_tensor(np.asarray(self.bins[k]), dtype=torch.int32, device=cr.dev) for k in ("EE", "BB")}

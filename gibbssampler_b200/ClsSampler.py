@@ -45,6 +45,7 @@ class ClsSampler():
         edges = np.asarray(bins, dtype=np.int64)
         nb = len(edges) - 1
         cl = self._alm2cl_real(alms_real_d)
+        self._last_cl = cl       # the empirical spectrum of this draw (GibbsSampler's keep_sigma records it)
         out = torch.empty(nb, dtype=torch.float64, device=self.dev)
         inject = None
         if self.rng.mode == "numpy":

@@ -9,7 +9,24 @@ from . import _dev, utils
 from ._dev import f64
 
 
+class SigmaRecorder():
+    """Empirical spectra sigma^i of the sky samples of a run (the input of BlackwellRao): one (n_iter, lmax + 1) device buffer
+    per spectrum, filled by device-to-device copies as the chain runs (no synchronisation) and copied to the host once."""
+
+    def __init__(self, keys, n_iter, lmax):
+        self.buf = {k: torch.empty((n_iter, lmax + 1), dtype=torch.float64, device=_dev.device()) for k in keys}
+
+    def record(self, i, sigma):
+        for k, b in self.buf.items():
+            b[i].copy_(sigma[k])
+
+    def result(self):
+        return {k: b.cpu().numpy() for k, b in self.buf.items()}
+
+
 class GibbsSampler():
+    keep_sigma = False   # CenteredGibbs(keep_sigma=True): run() leaves the empirical spectra of its sky samples in sigma_history
+
     def __init__(self, pix_map, noise, beam_fwhm_deg, nside, lmax, polarization=False, bins=None, n_iter=10000,
                  gibbs_cr=False, rj_step=False, ula=False, *, verbose=False):
         self.noise = noise
@@ -62,6 +79,7 @@ class GibbsSampler():
             skymap, accept = self.constrained_sampler.sample(dls_unbinned)
         h_dls["EE"].append(_dev.to_host(binned_dls["EE"]))
         h_dls["BB"].append(_dev.to_host(binned_dls["BB"]))
+        rec = SigmaRecorder(("EE", "BB"), self.n_iter, self.lmax) if self.keep_sigma else None
         for i in range(self.n_iter):
             if self.verbose and i % 100 == 0:
                 print("Default Gibbs" if not self.ula else "ULA")
@@ -77,6 +95,8 @@ class GibbsSampler():
 
             start_time = time.perf_counter()
             binned_dls = self.cls_sampler.sample(dict(skymap))
+            if rec is not None:
+                rec.record(i, self.cls_sampler.last_sigma)
             dls_unbinned = {"EE": self._unfold(binned_dls, "EE"), "BB": self._unfold(binned_dls, "BB")}
             torch.cuda.synchronize()
             h_duration_cls_sampling.append(time.perf_counter() - start_time)
@@ -84,6 +104,8 @@ class GibbsSampler():
             h_dls["BB"].append(_dev.to_host(binned_dls["BB"]))
         if self.verbose and (self.rj_step == True or self.ula == True):
             print("Acception rate constrained realization:", np.mean(h_accept_cr))
+        if rec is not None:
+            self.sigma_history = rec.result()
         h_dls["EE"] = np.array(h_dls["EE"])
         h_dls["BB"] = np.array(h_dls["BB"])
         return h_dls, np.array(h_accept_cr), np.array(h_duration_cr), np.array(h_duration_cls_sampling)
@@ -100,6 +122,7 @@ class GibbsSampler():
         cls, var_cls_full = self._tt_state(binned_dls)
         skymap, accept = self.constrained_sampler.sample(cls, var_cls_full, None, metropolis_step=False)
         h_dls.append(_dev.to_host(binned_dls))
+        rec = SigmaRecorder(("TT",), self.n_iter, self.lmax) if self.keep_sigma else None
         for i in range(self.n_iter):
             if self.verbose:
                 print("Default Gibbs")
@@ -107,11 +130,15 @@ class GibbsSampler():
             start_time = time.perf_counter()
             skymap, accept = self.constrained_sampler.sample(cls, var_cls_full, skymap, metropolis_step=False, use_gibbs=False)
             binned_dls = self.cls_sampler.sample(skymap)
+            if rec is not None:
+                rec.record(i, self.cls_sampler.last_sigma)
             cls, var_cls_full = self._tt_state(binned_dls)
             torch.cuda.synchronize()
             h_accept_cr.append(accept)
             h_dls.append(_dev.to_host(binned_dls))
             h_time_seconds.append(time.perf_counter() - start_time)
+        if rec is not None:
+            self.sigma_history = rec.result()
         return np.array(h_dls), np.array(h_accept_cr), h_time_seconds
 
     def run(self, dls_init):

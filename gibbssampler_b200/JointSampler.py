@@ -234,6 +234,7 @@ class JointClsSampler():
             return self._sample_binned(alms, inject, gamma_inject)
         L = _lib.lib()
         ch = self.empirical(alms)
+        self.last_sigma = ch
         self.rng.counter += 2          # shared generator counter (see ClsSampler._invgamma_draw): one index per draw kernel
         self._call = self.rng.counter - 1
         tt, te, ee = (torch.empty(self.lmax + 1, dtype=torch.float64, device=self.dev) for _ in range(3))
@@ -258,6 +259,7 @@ class JointClsSampler():
         if gi is not None and gi.numel() != nb:
             raise ValueError("gamma_inject must have %d entries, got %d" % (nb, gi.numel()))
         ch = self.empirical(alms)
+        self.last_sigma = ch
         self.rng.counter += 2          # the same two call indices as the per-l draw
         self._call = self.rng.counter - 1
         tt, te, ee = (torch.empty(nt, dtype=torch.float64, device=self.dev) for _ in range(3))
@@ -276,8 +278,11 @@ class JointGibbs():
     constrained realization sees D unfolded to L+1 multipoles (utils.unfold_bins)."""
 
     def __init__(self, pix_map, noise_temp, noise_pol, beam_fwhm_deg, nside, lmax, n_iter=1000, *, mask=None, mask_pol=None,
-                 bins=None, rng="philox", seed=None):
+                 bins=None, rng="philox", seed=None, keep_sigma=False):
+        """keep_sigma=True: run() also leaves sigma_history = {"TT", "TE", "EE", "BB"}: (n_iter, lmax + 1) numpy arrays whose row i
+        is the empirical (cross-)spectrum of the sky drawn in iteration i, the input of BlackwellRao."""
         self.lmax, self.nside, self.n_iter = int(lmax), int(nside), int(n_iter)
+        self.keep_sigma = bool(keep_sigma)
         bl = _dev.gauss_beam(np.radians(beam_fwhm_deg), self.lmax)
         shared = _dev.Rng(rng, seed)
         self.cls_sampler = JointClsSampler(lmax, bins=bins, rng=shared)     # first: bad bins fail before the plan is built
@@ -300,9 +305,15 @@ class JointGibbs():
                 if dls[k].numel() != want:
                     raise ValueError("dls_init[%r] must hold %d binned values, got %d" % (k, want, dls[k].numel()))
         h = {k: [_dev.to_host(dls[k])] for k in keys}
-        for _ in range(self.n_iter):
+        from .GibbsSampler import SigmaRecorder
+        rec = SigmaRecorder(("TT", "TE", "EE", "BB"), self.n_iter, self.lmax) if self.keep_sigma else None
+        for i in range(self.n_iter):
             sky, _ = self.constrained_sampler.sample(self._unfold(dls))
             dls = self.cls_sampler.sample(sky)
+            if rec is not None:
+                rec.record(i, self.cls_sampler.last_sigma)
             for k in keys:
                 h[k].append(_dev.to_host(dls[k]))
+        if rec is not None:
+            self.sigma_history = rec.result()
         return {k: np.array(v) for k, v in h.items()}

@@ -15,6 +15,9 @@ GS_ALM_REAL = 1
 
 GS_E_NOTCONVERGED = -3   # a PCG solve stopped at its iteration limit (include/gibbs_b200.h)
 
+GS_BR_IG = 0             # Blackwell-Rao spectrum groups (include/gibbs_b200.h): inverse-gamma spectrum
+GS_BR_IW = 1             # (TT, TE; TE, EE) inverse-Wishart block
+
 _lib = None
 
 _vp = C.c_void_p
@@ -92,6 +95,11 @@ SIGNATURES = {
     "gs_alm2cl_cross": (_i, [_vp, _vp, _i, _vp, _vp]),
     "gs_cls_invwishart": (_i, [_vp, _vp, _vp, _i, _vp, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
     "gs_cls_invwishart_binned": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
+    "gs_br_sample_features": (_i, [_i, _vp, _vp, _vp, _i64, _i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
+    "gs_br_model_features": (_i, [_i, _vp, _vp, _vp, _i64, _i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
+    "gs_br_logmeanexp_scratch": (_i64, [_i64, _i64]),
+    "gs_br_logmeanexp": (_i, [_vp, _vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
+    "gs_br_marginal": (_i, [_i, _vp, _i64, _i, _vp, _i, _i, _vp, _i64, _i, _vp, _vp]),
     "gs_nccl_unique_id": (_i, [C.c_char_p]),
     "gs_plan_create_sharded": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _i, C.c_char_p]),
     "gs_local_group_create": (_i, [C.POINTER(_vp), _i]),

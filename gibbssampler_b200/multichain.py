@@ -33,6 +33,8 @@ def run_chains(gibbs, dls_init):
     dls_init: one binned {"EE", "BB"} start per chain.  Chains are paired (0, 1), (2, 3), ...; an odd last chain runs alone.
     Returns one (h_dls, accept, t_cr, t_cls) tuple per chain, as the chain's own run()."""
     assert len(gibbs) == len(dls_init) and len(gibbs) >= 1
+    if any(getattr(g, "keep_sigma", False) for g in gibbs):
+        raise ValueError("run_chains does not record the sky spectra: run chains built with keep_sigma=True through their own run()")
     n_iter = gibbs[0].n_iter
     assert all(g.n_iter == n_iter and g.polarization for g in gibbs)
     K = len(gibbs)

@@ -397,6 +397,55 @@ int gs_cls_invwishart_binned(const double* cl_tt, const double* cl_te, const dou
                              const int* bins, int nbins, const double* inject, uint64_t seed, uint64_t call,
                              double* dl_tt, double* dl_te, double* dl_ee, void* stream);
 
+/* ---- Blackwell-Rao estimator of the spectrum posterior (Wandelt, Larson & Lakshminarayanan 2004; Chu et al. 2005) ----------
+ * The reference has no BR code.  From the empirical spectra sigma^i of the N sky samples of a chain,
+ *   log L(theta_k) = log( (1/N) sum_i exp( sum_b log p(D_b^k | sigma^i) ) ),  D in D units, p = the chain's C_l conditional:
+ *   GS_BR_IG (one spectrum, edges of gs_cls_invgamma): alpha_b = sum_{l in b} (2l+1)/2 - 1,
+ *     beta_b^i = sum_{l in b} (2l+1) l (l+1) sigma_l^i / 4pi (the arithmetic of gs_cls_invgamma's beta_out),
+ *     log p = alpha log beta - lgamma(alpha) - (alpha+1) log D_b - beta / D_b;
+ *   GS_BR_IW (the (TT, TE; TE, EE) block of gs_cls_invwishart_binned): nu_b = sum (2l+1) - 3,
+ *     Psi_b^i = sum (2l+1) l (l+1)/2pi Chat_l^i, log p = (nu/2) log|Psi| - nu log 2 - log Gamma_2(nu/2) - (nu+3)/2 log|D|
+ *     - tr(Psi D^-1)/2, log Gamma_2(a) = log(pi)/2 + lgamma(a) + lgamma(a - 1/2).
+ * Written x_ik = c_i + sum_j S_ji W_jk + e_k, S is a (K, N) feature-major matrix (IG bin: one row beta_b; IW bin: three rows
+ * Psi00, Psi01, Psi11), W a (K, M) one (IG: -1/D_b; IW: -(D^-1)00/2, -(D^-1)01, -(D^-1)11/2); c and e carry the rest.
+ * Every bin passed to these calls is evaluated: callers pass the edges of the bins they want (the chains' bins 0 and 1 are
+ * fixed at D = 0 and are never evaluated).  bins = nbins + 1 int32 device edges; each thread checks its own bin
+ * (0 <= first < last <= ncl) and writes NaN for a broken one instead of reading out of range. */
+#define GS_BR_IG 0
+#define GS_BR_IW 1
+/* Sample features of one spectrum group: sigma (IG) or sigma = TT, sigma_te, sigma_ee (IW), each (nsamp, ncl) row-major
+ * (row i = empirical C_l of sample i, ncl = lmax + 1).  Writes rows 0 .. f nbins - 1 of S (f = 1 for IG, 3 for IW; row r at
+ * S + r nsamp: pass S offset to the group's first row) and c[i] = (accumulate ? c[i] : 0) + sum_b t_b^i, b ascending, with
+ * t_b = alpha_b log beta_b (IG) or (nu_b / 2) log|Psi_b| (IW).  scratch: nbins * nsamp doubles.  GS_E_BADARG for null
+ * pointers, a bad kind, nsamp < 1 or nbins outside [1, min(ncl, 65535)]. */
+int gs_br_sample_features(int kind, const double* sigma, const double* sigma_te, const double* sigma_ee, int64_t nsamp, int ncl,
+                          const int* bins, int nbins, double* S, double* c, int accumulate, double* scratch, void* stream);
+/* Model features of one group: dl (IG) or dl = TT, dl_te, dl_ee (IW), each (nmod, nbins) row-major binned D of the group's
+ * bins.  Writes rows 0 .. f nbins - 1 of W (row r at W + r nmod) and e[k] = (accumulate ? e[k] : 0) + sum_b u_b^k with
+ * u_b = -lgamma(alpha) - (alpha+1) log D_b (IG) or -nu log 2 - log Gamma_2(nu/2) - (nu+3)/2 log|D_b| (IW).  A model with
+ * D_b <= 0, or an IW block that is not positive definite, gets W = 0 and e = -inf (its estimate is exactly -inf).
+ * scratch: nbins * nmod doubles.  GS_E_BADARG as gs_br_sample_features. */
+int gs_br_model_features(int kind, const double* dl, const double* dl_te, const double* dl_ee, int64_t nmod, int ncl,
+                         const int* bins, int nbins, double* W, double* e, int accumulate, double* scratch, void* stream);
+/* Fused GEMM + log-mean-exp: logl_out[k] = log((1/N) sum_i exp(x_ik)), x = c + S^T W + e (S: (K, nsamp), W: (K, nmod)), and
+ * neff_out[k] (nullable) = (sum w_i)^2 / sum w_i^2, w_i = exp(x_ik - max_i x_ik): 0 and -inf for a model with e = -inf, NaN
+ * for e = NaN.  Never forms the nsamp x nmod matrix.  The sample axis is split over
+ *   P = min(ceil(nsamp / 256), ceil(2368 / ceil(nmod / 64)))
+ * CTA columns; scratch: 3 * nmod * P doubles (the per-split partials, merged in a fixed order), as gs_br_logmeanexp_scratch
+ * returns.  The split depends on
+ * (nsamp, nmod) only, so repeated calls are bit-identical.  GS_E_BADARG for null pointers or nsamp, nmod, K < 1. */
+/* Doubles of scratch gs_br_logmeanexp needs for (nsamp, nmod): 3 nmod P (-1 for nsamp or nmod < 1). */
+int64_t gs_br_logmeanexp_scratch(int64_t nsamp, int64_t nmod);
+int gs_br_logmeanexp(const double* S, const double* c, int64_t nsamp, const double* W, const double* e, int64_t nmod, int K,
+                     double* scratch, double* logl_out, double* neff_out, void* stream);
+/* Per-bin marginals out[b][g] = log((1/N) sum_i p(grid_b[g] | sigma_b^i)) of one group, p = IG(alpha_b, beta_b^i) for GS_BR_IG
+ * (comp = 0; S = the group's nbins rows) and, for GS_BR_IW, the marginal of diagonal entry comp (0 = TT, 2 = EE) of the
+ * inverse-Wishart, IG((nu_b - 1)/2, Psi_b,comp / 2) (S = the group's 3 nbins rows).  grid_b = grid + b grid_ld (grid_ld = 0:
+ * one grid for all bins), ngrid points; a point <= 0 gives -inf.  out: (nbins, ngrid).  GS_E_BADARG for null pointers, a
+ * bad kind / comp, nsamp or ngrid < 1, grid_ld < 0 or nbins outside [1, min(ncl, 65535)]. */
+int gs_br_marginal(int kind, const double* S, int64_t nsamp, int ncl, const int* bins, int nbins, int comp, const double* grid,
+                   int64_t grid_ld, int ngrid, double* out, void* stream);
+
 /* ---- whole chain in one call (SURVEY.md 8b gs_gibbs_step_centered; BASELINE config #1) -----------------------------------
  * GibbsSampler.run_polarization (GibbsSampler.py:118-180) for the full-sky isotropic-noise centred sampler: every iteration is
  * PolarizedCenteredConstrainedRealization.sample_no_mask (CenteredGibbs.py:317-353) + PolarizedCenteredClsSampler.sample
