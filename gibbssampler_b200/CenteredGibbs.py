@@ -62,7 +62,7 @@ class PolarizedCenteredConstrainedRealization(ConstrainedRealization):
         self.pcg_itermax = 4000
         self.pcg_check_every = 8
         self.fluct_iter = 3                                            # utils.adjoint_synthesis_hp uses iter=3 (utils.py:89)
-        self.dls_to_cls_array = np.array([2 * np.pi / (l * (l + 1)) if l != 0 else 0 for l in range(lmax + 1)])
+        self.dls_to_cls_array = utils.dls_to_cls_array(lmax)
         self.alpha = alpha
         self.bl_fwhm = bl_fwhm
         self.tau = 0.02

@@ -2,7 +2,7 @@
 import numpy as np
 import torch
 
-from . import _dev, _lib
+from . import _dev, _lib, utils
 from ._dev import f64, ptr, stream
 from ._lib import check, GS_ALM_REAL
 from .sht import Plan
@@ -76,7 +76,7 @@ class MHClsSampler(ClsSampler):
         self.n_iter = n_iter
         self.proposal_variances = proposal_variances
         self.polarization = polarization
-        self.dls_to_cls_array = np.array([2 * np.pi / (l * (l + 1)) if l != 0 else 0 for l in range(lmax + 1)])
+        self.dls_to_cls_array = utils.dls_to_cls_array(lmax)
 
     def dls_to_cls(self, dls_):
         return dls_ * self.dls_to_cls_array

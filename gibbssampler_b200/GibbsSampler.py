@@ -53,7 +53,7 @@ class GibbsSampler():
                 self.bins = {"TT": bins, "EE": bins, "TE": bins, "BB": bins}
         else:
             self.bins = bins
-        self.dls_to_cls_array = np.array([2 * np.pi / (l * (l + 1)) if l != 0 else 0 for l in range(lmax + 1)])
+        self.dls_to_cls_array = utils.dls_to_cls_array(lmax)
 
     def dls_to_cls(self, dls_):
         return dls_[:] * self.dls_to_cls_array

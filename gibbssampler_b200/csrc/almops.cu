@@ -3,33 +3,11 @@
 #include <algorithm>
 
 #include "gs_internal.h"
+#include "spectra.cuh"
 
 #define EW_NT 256
 
 static inline int ew_blocks(int64_t n) { return (int)std::min<int64_t>((n + EW_NT - 1) / EW_NT, 148 * 16); }
-
-// (l, m) of healpy index id for lmax L:  id = m(2L+1-m)/2 + l,  m <= l <= L.
-__device__ __forceinline__ void lm_of_index(int64_t id, int L, int& l, int& m)
-{
-    // largest m with m(2L+1-m)/2 + m <= id  <=>  first element of column m is (m,m)
-    const double b = 2.0 * L + 3.0;
-    int mm = (int)floor((b - sqrt(b * b - 8.0 * (double)id)) * 0.5);
-    if (mm < 0) mm = 0;
-    if (mm > L) mm = L;
-    while (mm > 0 && (int64_t)mm * (2 * L + 1 - mm) / 2 + mm > id) --mm;
-    while (mm < L && (int64_t)(mm + 1) * (2 * L + 1 - (mm + 1)) / 2 + (mm + 1) <= id) ++mm;
-    m = mm;
-    l = (int)(id - (int64_t)mm * (2 * L + 1 - mm) / 2);
-}
-
-// l of entry i of the real layout ((L+1)^2 doubles)
-__device__ __forceinline__ int l_of_real_index(int64_t i, int L)
-{
-    if (i <= L) return (int)i;
-    int l, m;
-    lm_of_index((i + L + 1) >> 1, L, l, m);
-    return l;
-}
 
 // ---- utils.real_to_complex / complex_to_real (utils.py:49-76, variance_expension.pyx:65-100)
 __global__ void real_to_complex_kernel(const double* __restrict__ r, double2* __restrict__ c, int L, int64_t nalm)
@@ -59,26 +37,12 @@ __global__ void complex_to_real_kernel(const double2* __restrict__ c, double* __
     }
 }
 
-// ---- per-l array -> real layout.  mode 0: copy x_l (GibbsSampler.compute_bl_map, GibbsSampler.py:64-74,
-// config.generate_var_cl config.py:75-84); mode 1: D_l -> C_l = D_l 2 pi / (l(l+1)), l = 0 copied
-// (utils.generate_var_cl_cython utils.py:114-137, variance_expension.pyx:8-33); mode 2: 1/C_l where C_l != 0
-// else 0; mode 3: sqrt(C_l); mode 4: sqrt(1/C_l) where C_l != 0 else 0.
-__device__ __forceinline__ double per_l_value(const double* x, int l, int mode)
-{
-    double v = x[l];
-    if (mode == 0) return v;
-    if (l != 0) v = v * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
-    if (mode == 1) return v;
-    if (mode == 3) return sqrt(v);
-    const double inv = (v != 0.0) ? 1.0 / v : 0.0;
-    return mode == 2 ? inv : sqrt(inv);
-}
-
+// ---- per-l array -> real layout (per_l_value modes 0-4)
 __global__ void expand_per_l_kernel(const double* __restrict__ x, double* __restrict__ out, int L, int mode)
 {
     const int64_t nre = (int64_t)(L + 1) * (L + 1);
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < nre; i += (int64_t)gridDim.x * blockDim.x)
-        out[i] = per_l_value(x, l_of_real_index(i, L), mode);
+        out[i] = per_l_value(x, l_of_real(i, L), mode);
 }
 
 // ---- utils.unfold_bins (utils.py:150-162): np.repeat(binned, diff(bins))
@@ -86,10 +50,8 @@ __global__ void unfold_bins_kernel(const double* __restrict__ binned, const int*
                                    double* __restrict__ out, int nout)
 {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nout; i += gridDim.x * blockDim.x) {
-        const int l = bins[0] + i;  // output position i corresponds to multipole bins[0] + i
-        int lo = 0, hi = nbins - 1;
-        while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (bins[mid] <= l) lo = mid; else hi = mid - 1; }
-        out[i] = binned[lo];
+        // output position i corresponds to multipole bins[0] + i
+        out[i] = binned[bin_of(bins, nbins, bins[0] + i)];
     }
 }
 
@@ -98,7 +60,7 @@ __global__ void almxfl_kernel(const double* __restrict__ in, double* __restrict_
                               int layout, int64_t n, const int* __restrict__ lof)
 {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        if (layout == GS_ALM_REAL) out[i] = in[i] * fl[lof ? lof[i] : l_of_real_index(i, L)];
+        if (layout == GS_ALM_REAL) out[i] = in[i] * fl[lof ? lof[i] : l_of_real(i, L)];
         else {
             int l, m;
             lm_of_index(i, L, l, m);
@@ -115,15 +77,13 @@ __global__ void alm2cl_kernel(const double* __restrict__ alm, int layout, int L,
     const int l = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (l > L) return;
     double s = 0.0;
-    for (int m = lane; m <= l; m += 32) {
-        const int64_t id = (int64_t)m * (2 * L + 1 - m) / 2 + l;
-        if (layout == GS_ALM_COMPLEX) {
-            const double2 v = reinterpret_cast<const double2*>(alm)[id];
+    if (layout == GS_ALM_COMPLEX)
+        for (int m = lane; m <= l; m += 32) {
+            const double2 v = reinterpret_cast<const double2*>(alm)[(int64_t)m * (2 * L + 1 - m) / 2 + l];
             s += (m ? 2.0 : 1.0) * (v.x * v.x + v.y * v.y);
-        } else if (m == 0) s += alm[l] * alm[l];
-        else { const int64_t o = 2 * id - (L + 1); s += alm[o] * alm[o] + alm[o + 1] * alm[o + 1]; }
-    }
-    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        }
+    else s = alm2cl_real_lane(alm, l, L, lane);
+    s = warp_sum(s);
     if (lane == 0) cl[l] = s / (2.0 * l + 1.0);
 }
 
@@ -136,8 +96,6 @@ __global__ void map_residual_kernel(const double* __restrict__ a, const double* 
 }
 
 // ------------------------------------------------------------------ C ABI
-#define STREAM(s) ((cudaStream_t)(s))
-
 extern "C" int gs_real_to_complex(const double* real_alm, double* complex_alm, int lmax, void* stream)
 {
     GS_REQUIRE(real_alm && complex_alm && lmax >= 0, "bad arguments");
@@ -238,7 +196,7 @@ extern "C" int gs_alm2map_spin2_fl2(gs_plan* p, const double* almE, const double
 static int map2alm_impl(gs_plan* p, int spin, const double* mapQ, const double* mapU, const double* pixw, int iter,
                         int adjoint, const double* fl, double* almE, double* almB, int layout, cudaStream_t st)
 {
-    const double scale = adjoint ? 1.0 : 4.0 * 3.14159265358979323846 / (double)p->d.npix;
+    const double scale = adjoint ? 1.0 : 4.0 * GS_PI / (double)p->d.npix;
     if (adjoint) iter = 0;
     const double* fl0 = iter > 0 ? nullptr : fl;
     int rc;
@@ -317,7 +275,7 @@ extern "C" int gs_map2alm_batch(gs_plan* p, int spin, int n_chain, const double*
                (layout == GS_ALM_COMPLEX || layout == GS_ALM_REAL), "bad arguments");
     if (n_chain > 1 && (rc = gs_plan_reserve_chains(p, 2))) return rc;
     cudaStream_t st = STREAM(stream);
-    const double scale = adjoint ? 1.0 : 4.0 * 3.14159265358979323846 / (double)p->d.npix;
+    const double scale = adjoint ? 1.0 : 4.0 * GS_PI / (double)p->d.npix;
     for (int c = 0; c < n_chain; c += 2) {
         const int nc = n_chain - c >= 2 ? 2 : 1;
         const double* q = mapQ + c * map_stride;

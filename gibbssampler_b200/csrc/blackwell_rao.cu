@@ -9,15 +9,13 @@
 #include <algorithm>
 
 #include "gs_internal.h"
+#include "spectra.cuh"
 
 #define BR_NT 256
 #define BR_BK 8                   // features per shared-memory stage of the GEMM
 #define BR_SPLIT_UNIT 256         // the sample axis is split over CTAs in multiples of this many samples
 #define BR_TARGET_CTAS (148 * 16) // CTAs the split aims at: 16 waves of one CTA per SM keep the last-wave tail small
 #define BR_SMALL_M 32             // up to this many models the narrow 8-model tile runs (one parameter-MCMC call is M = 1)
-#define BR_PI 3.14159265358979323846
-
-#define STREAM(s) ((cudaStream_t)(s))
 
 __device__ __forceinline__ bool br_bin(const int* __restrict__ bins, int b, int ncl, int& l0, int& l1)
 {
@@ -26,27 +24,11 @@ __device__ __forceinline__ bool br_bin(const int* __restrict__ bins, int b, int 
     return l0 >= 0 && l1 > l0 && l1 <= ncl;
 }
 
-// alpha_b = sum_{l in b} (2l+1)/2 - 1, summed as cls_invgamma_kernel does
-__device__ __forceinline__ double br_ig_alpha(int l0, int l1)
-{
-    double ex = 0.0;
-    for (int l = l0; l < l1; ++l) ex += (2.0 * l + 1.0) / 2.0;
-    return ex - 1.0;
-}
-
-// nu_b = sum_{l in b} (2l+1) - 3, as invwishart_binned_kernel
-__device__ __forceinline__ double br_iw_nu(int l0, int l1)
-{
-    double nu = -3.0;
-    for (int l = l0; l < l1; ++l) nu += 2.0 * l + 1.0;
-    return nu;
-}
-
 __device__ __forceinline__ double br_nan() { return __longlong_as_double(0x7ff8000000000000ll); }
 
 // ------------------------------------------------------------------ features
-// Thread (sample i, bin b).  IG: S row b = beta_b^i (the expression and order of cls_invgamma_kernel, so it equals its beta_out bit
-// for bit), t[b][i] = alpha_b log beta_b^i.  IW: S rows 3b..3b+2 = (Psi00, Psi01, Psi11) of invwishart_binned_kernel,
+// Thread (sample i, bin b).  IG: S row b = beta_b^i (ig_bin_stats, as cls_invgamma_kernel, so it equals its beta_out bit for bit),
+// t[b][i] = alpha_b log beta_b^i.  IW: S rows 3b..3b+2 = (Psi00, Psi01, Psi11) (iw_bin_stats, as invwishart_binned_kernel),
 // t[b][i] = (nu_b / 2) log|Psi_b^i|.  A bin whose device edges are broken (empty, negative, past ncl) comes out NaN.
 __global__ void br_sample_features_kernel(int kind, const double* __restrict__ sig, const double* __restrict__ sig_te,
                                           const double* __restrict__ sig_ee, int64_t n, int ncl, const int* __restrict__ bins,
@@ -59,23 +41,16 @@ __global__ void br_sample_features_kernel(int kind, const double* __restrict__ s
     const bool ok = br_bin(bins, b, ncl, l0, l1);
     if (kind == GS_BR_IG) {
         if (!ok) { S[b * n + i] = br_nan(); t[b * n + i] = br_nan(); return; }
-        const double* cl_hat = sig + i * ncl;
-        double beta = 0.0;
-        for (int l = l0; l < l1; ++l) beta += (2.0 * l + 1.0) * (double)l * (double)(l + 1) * (cl_hat[l] / (4.0 * 3.14159265358979323846));
+        double beta, alpha = ig_bin_stats(sig + i * ncl, l0, l1, beta);
         S[b * n + i] = beta;
-        t[b * n + i] = br_ig_alpha(l0, l1) * log(beta);
+        t[b * n + i] = alpha * log(beta);
         return;
     }
     double* s = S + (int64_t)3 * b * n + i;
     if (!ok) { s[0] = br_nan(); s[n] = br_nan(); s[2 * n] = br_nan(); t[b * n + i] = br_nan(); return; }
-    const double *tt = sig + i * ncl, *te = sig_te + i * ncl, *ee = sig_ee + i * ncl;
-    double p00 = 0.0, p01 = 0.0, p11 = 0.0;
-    for (int l = l0; l < l1; ++l) {
-        const double f = 2.0 * l + 1.0, w = f * ((double)l * (double)(l + 1) / (2.0 * 3.14159265358979323846));
-        p00 += w * tt[l]; p01 += w * te[l]; p11 += w * ee[l];
-    }
-    s[0] = p00; s[n] = p01; s[2 * n] = p11;
-    t[b * n + i] = 0.5 * br_iw_nu(l0, l1) * log(p00 * p11 - p01 * p01);
+    double psi[3], nu = iw_bin_stats(sig + i * ncl, sig_te + i * ncl, sig_ee + i * ncl, l0, l1, psi);
+    s[0] = psi[0]; s[n] = psi[1]; s[2 * n] = psi[2];
+    t[b * n + i] = 0.5 * nu * log(psi[0] * psi[2] - psi[1] * psi[1]);
 }
 
 // Thread (model k, bin b).  IG: W row b = -1/D_b, t = -lgamma(alpha) - (alpha+1) log D_b.  IW: W rows = (-(D^-1)00 / 2, -(D^-1)01,
@@ -92,7 +67,7 @@ __global__ void br_model_features_kernel(int kind, const double* __restrict__ d,
     const bool ok = br_bin(bins, b, ncl, l0, l1);
     const int64_t j = k * nbins + b;
     if (kind == GS_BR_IG) {
-        const double D = d[j], alpha = ok ? br_ig_alpha(l0, l1) : 0.0;
+        const double D = d[j], alpha = ok ? ig_bin_alpha(l0, l1) : 0.0;
         const bool valid = D > 0.0;
         W[b * m + k] = !ok ? br_nan() : valid ? -1.0 / D : 0.0;
         t[b * m + k] = !ok ? br_nan() : valid ? -lgamma(alpha) - (alpha + 1.0) * log(D) : -INFINITY;
@@ -100,12 +75,12 @@ __global__ void br_model_features_kernel(int kind, const double* __restrict__ d,
     }
     double* w = W + (int64_t)3 * b * m + k;
     if (!ok) { w[0] = br_nan(); w[m] = br_nan(); w[2 * m] = br_nan(); t[b * m + k] = br_nan(); return; }
-    const double tt = d[j], te = d_te[j], ee = d_ee[j], det = tt * ee - te * te, nu = br_iw_nu(l0, l1);
+    const double tt = d[j], te = d_te[j], ee = d_ee[j], det = tt * ee - te * te, nu = iw_bin_nu(l0, l1);
     if (!(tt > 0.0 && det > 0.0)) { w[0] = 0.0; w[m] = 0.0; w[2 * m] = 0.0; t[b * m + k] = -INFINITY; return; }
     w[0] = -0.5 * (ee / det);
     w[m] = te / det;
     w[2 * m] = -0.5 * (tt / det);
-    const double lg2 = 0.5 * log(BR_PI) + lgamma(0.5 * nu) + lgamma(0.5 * nu - 0.5);
+    const double lg2 = 0.5 * log(GS_PI) + lgamma(0.5 * nu) + lgamma(0.5 * nu - 0.5);
     t[b * m + k] = -nu * log(2.0) - lg2 - 0.5 * (nu + 3.0) * log(det);
 }
 
@@ -403,9 +378,9 @@ __global__ void __launch_bounds__(BR_NT) br_marginal_kernel(int kind, const doub
     const double* row = S + (int64_t)b * n;
     if (ok) {
         if (kind == GS_BR_IG) {
-            alpha = br_ig_alpha(l0, l1);
+            alpha = ig_bin_alpha(l0, l1);
         } else {
-            alpha = 0.5 * (br_iw_nu(l0, l1) - 1.0);
+            alpha = 0.5 * (iw_bin_nu(l0, l1) - 1.0);
             scale = 0.5;
             row = S + ((int64_t)3 * b + comp) * n;
         }

@@ -14,6 +14,7 @@
 
 #include "gs_internal.h"
 #include "rng.cuh"
+#include "spectra.cuh"
 
 struct ChainDev {
     int L, nbE, nbB;
@@ -39,13 +40,7 @@ __global__ void gstep_binof_kernel(const int* __restrict__ bins, int nb, int L, 
 {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l > L) return;
-    int b = -1;
-    if (l >= bins[0] && l < bins[nb]) {
-        int lo = 0, hi = nb - 1;
-        while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (bins[mid] <= l) lo = mid; else hi = mid - 1; }
-        b = lo;
-    }
-    binof[l] = b;
+    binof[l] = l >= bins[0] && l < bins[nb] ? bin_of(bins, nb, l) : -1;
 }
 
 // constrained realization: diagonal solve + draw for E and B (CenteredGibbs.py:317-353); D_l of this iteration = history row `it`
@@ -59,14 +54,11 @@ __global__ void __launch_bounds__(256) gstep_cr_kernel(ChainDev C)
         const int l = l_of_real(i, L);
         const double b = C.bl[l];
         double n0, n1;
-        // stream ids: tag 0x43 ("C"onstrained realization) in the top byte, then the iteration: disjoint from every other consumer
-        box_muller(ph((uint64_t)i, (0x43ull << 56) | it), n0, n1);
+        box_muller(ph((uint64_t)i, RNG_CR | it), n0, n1);
 #pragma unroll
         for (int pol = 0; pol < 2; ++pol) {
             const int bin = (pol ? C.binofB : C.binofE)[l];
-            double c = bin >= 0 ? (pol ? C.histB + it * C.nbB : C.histE + it * C.nbE)[bin] : 0.0;
-            if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
-            const double ic = c != 0.0 ? 1.0 / c : 0.0;
+            const double ic = safe_rcp(dl_to_cl(bin >= 0 ? (pol ? C.histB + it * C.nbB : C.histE + it * C.nbE)[bin] : 0.0, l));
             const double sigma = 1.0 / (C.w * b * b + ic);
             const double d = (pol ? C.dB : C.dE)[i];
             (pol ? C.almB : C.almE)[i] = sigma * (b * (C.w * d)) + (pol ? n1 : n0) * sqrt(sigma);
@@ -80,17 +72,7 @@ __global__ void __launch_bounds__(256) gstep_cl_kernel(ChainDev C)
     const int L = C.L, wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (wid >= 2 * (L + 1)) return;
     const int pol = wid > L, l = pol ? wid - (L + 1) : wid;
-    const double* a = pol ? C.almB : C.almE;
-    double s = 0.0;
-    for (int m = lane; m <= l; m += 32) {
-        if (m == 0) { const double v = a[l]; s += v * v; }
-        else {
-            const int64_t id = (int64_t)m * (2 * L + 1 - m) / 2 + l, off = 2 * id - (L + 1);
-            const double x = a[off], y = a[off + 1];
-            s += x * x + y * y;
-        }
-    }
-    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    const double s = warp_sum(alm2cl_real_lane(pol ? C.almB : C.almE, l, L, lane));
     if (lane == 0) (pol ? C.clB : C.clE)[l] = s / (2.0 * l + 1.0);
 }
 
@@ -102,16 +84,9 @@ __global__ void __launch_bounds__(128) gstep_cls_kernel(ChainDev C)
     if (t < C.nbE + C.nbB) {
         const int pol = t >= C.nbE, b = pol ? t - C.nbE : t;
         const int* bins = pol ? C.binsB : C.binsE;
-        const double* cl = pol ? C.clB : C.clE;
-        double beta = 0.0, ex = 0.0;
-        for (int l = bins[b]; l < bins[b + 1]; ++l) {
-            beta += (2.0 * l + 1.0) * (double)l * (double)(l + 1) * (cl[l] / (4.0 * 3.14159265358979323846));
-            ex += (2.0 * l + 1.0) / 2.0;
-        }
-        double alpha = ex - 1.0;
+        double beta, alpha = ig_bin_stats(pol ? C.clB : C.clE, bins[b], bins[b + 1], beta);
         if (b == 0) alpha = 1.0;
-        // tag 0x47 ("G"amma), iteration, spectrum, bin
-        const double g = alpha > 0.0 ? gamma_mt(alpha, Philox(C.seed), (0x47ull << 56) | (it << 21) | ((uint64_t)pol << 20) | (uint64_t)b) : 1.0;
+        const double g = alpha > 0.0 ? gamma_mt(alpha, Philox(C.seed), RNG_GAMMA | (it << 21) | ((uint64_t)pol << 20) | (uint64_t)b) : 1.0;
         (pol ? C.histB + (it + 1) * C.nbB : C.histE + (it + 1) * C.nbE)[b] = (b < 2) ? 0.0 : beta / g;
     }
 }
@@ -149,7 +124,7 @@ extern "C" int gs_gibbs_run_centered_fullsky(int lmax, int64_t npix, double nois
     int* binof = reinterpret_cast<int*>(scratch + nd);
     C.binofE = binof; C.binofB = binof + (L + 1);
     C.bl = bl; C.dE = d_E; C.dB = d_B;
-    C.w = (double)npix / (noise_pol * 4.0 * 3.14159265358979323846);
+    C.w = (double)npix / (noise_pol * 4.0 * GS_PI);
     C.histE = hist_EE; C.histB = hist_BB;
     C.seed = seed;
     int rc = GS_OK;

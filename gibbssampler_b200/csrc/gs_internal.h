@@ -18,6 +18,8 @@ void gs_set_error(const char* fmt, ...);
         }                                                                                    \
     } while (0)
 #define GS_CHECK_LAUNCH() GS_CHECK_CUDA(cudaGetLastError())
+// the opaque stream argument of the C ABI
+#define STREAM(s) ((cudaStream_t)(s))
 #define GS_REQUIRE(cond, msg)                                \
     do {                                                     \
         if (!(cond)) {                                       \

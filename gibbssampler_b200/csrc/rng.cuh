@@ -1,5 +1,5 @@
-// Device helpers shared by sampler.cu and teb.cu: Philox4x32-10 counter RNG, Box-Muller normals,
-// Marsaglia-Tsang gamma variates, and the multipole of a real-layout index.
+// Device random numbers of the samplers: Philox4x32-10 counter RNG, its stream domains, Box-Muller normals and
+// Marsaglia-Tsang gamma variates.
 #pragma once
 #include <math.h>
 #include <stdint.h>
@@ -40,6 +40,15 @@ __device__ __forceinline__ void box_muller(uint4 r, double& n0, double& n1)
     n1 = rad * s;
 }
 
+// Stream domains: the top byte of a Philox stream id names its consumer, so no consumer walks into another one's streams however
+// long a chain runs (the counters of gs_randn / gs_randu stay below 2^56).  Each consumer keeps its own id layout, and changing one
+// changes every chain history:
+//   RNG_CR       normals of the fused chain (gibbs_step.cu): RNG_CR | it
+//   RNG_GAMMA    gs_cls_invgamma: ((call << 20) + b) & RNG_ID_MASK; the fused chain, on its own seed word: (it << 21) | (pol << 20) | b
+//   RNG_WISHART  inverse-Wishart draws (teb.cu): ((call << 22) + 4 k) & RNG_ID_MASK, then + 0 / 1 / 2
+constexpr uint64_t RNG_CR = 0x43ull << 56, RNG_GAMMA = 0x47ull << 56, RNG_WISHART = 0x57ull << 56;
+constexpr uint64_t RNG_ID_MASK = 0x00ffffffffffffffull;
+
 // ------------------------------------------------------------------ inverse-gamma C_l draw
 // Marsaglia-Tsang Gamma(a,1), a > 0, one thread per draw with its own Philox stream
 __device__ inline double gamma_mt(double a, const Philox& ph, uint64_t stream)
@@ -64,18 +73,3 @@ __device__ inline double gamma_mt(double a, const Philox& ph, uint64_t stream)
     }
     return boost * d;
 }
-
-// l of real-layout index (same mapping as almops.cu)
-__device__ __forceinline__ int l_of_real(int64_t i, int L)
-{
-    if (i <= L) return (int)i;
-    const int64_t id = (i + L + 1) >> 1;
-    const double b = 2.0 * L + 3.0;
-    int mm = (int)floor((b - sqrt(b * b - 8.0 * (double)id)) * 0.5);
-    if (mm < 0) mm = 0;
-    if (mm > L) mm = L;
-    while (mm > 0 && (int64_t)mm * (2 * L + 1 - mm) / 2 + mm > id) --mm;
-    while (mm < L && (int64_t)(mm + 1) * (2 * L + 1 - (mm + 1)) / 2 + (mm + 1) <= id) ++mm;
-    return (int)(id - (int64_t)mm * (2 * L + 1 - mm) / 2);
-}
-

@@ -7,6 +7,7 @@
 
 #include "gs_internal.h"
 #include "rng.cuh"
+#include "spectra.cuh"
 
 #define SM_NT 256
 #define SM_GRID (148 * 4)
@@ -98,11 +99,10 @@ __global__ void cr_direct_kernel(const double* __restrict__ dl, const double* __
     const int64_t n = (int64_t)(L + 1) * (L + 1);
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const int l = l_of_real(i, L);
-        double c = dl[l];
-        if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
+        const double c = dl_to_cl(dl[l], l);
         const double b = bl[l];
         if (mode == 0) {
-            const double ic = c != 0.0 ? 1.0 / c : 0.0;
+            const double ic = safe_rcp(c);
             const double sigma = 1.0 / (w * b * b + ic);
             out[i] = sigma * (b * (w * d_alm[i])) + xi[i] * sqrt(sigma);
         } else {
@@ -124,12 +124,11 @@ __global__ void cr_direct_pix_kernel(const double* __restrict__ dl, const double
     const int64_t n = (int64_t)(L + 1) * (L + 1);
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const int l = l_of_real(i, L);
-        double c = dl[l];
-        if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
+        const double c = dl_to_cl(dl[l], l);
         const double b = bl[l];
         double v;
         if (l < l_cut) {
-            const double ic = c != 0.0 ? 1.0 / c : 0.0;
+            const double ic = safe_rcp(c);
             v = (bsum[i] + xi[i] * sqrt(ic)) / (ic + w * b * b);
         } else {
             v = (sqrt(c) * bsum[i] + xi[i]) / (1.0 + c * w * b * b);
@@ -141,8 +140,7 @@ __global__ void cr_direct_pix_kernel(const double* __restrict__ dl, const double
 
 // ------------------------------------------------------------------ inverse-gamma C_l draw
 // PolarizedCenteredClsSampler.sample_one_pol / CenteredClsSampler.sample (CenteredGibbs.py:24-79):
-//   beta_l = (2l+1) l (l+1) Chat_l / (4 pi); per bin: beta = sum beta_l, alpha = sum (2l+1)/2 - 1;
-//   alpha[0] := 1; D_bin = beta / Gamma(alpha, 1); D[:2] := 0.
+//   alpha, beta of each bin from ig_bin_stats; alpha[0] := 1; D_bin = beta / Gamma(alpha, 1); D[:2] := 0.
 // gamma_inject (nullable): Gamma(alpha,1) variates drawn by the caller (parity with numpy's stream).
 __global__ void cls_invgamma_kernel(const double* __restrict__ cl_hat, const int* __restrict__ bins, int nbins,
                                     const double* __restrict__ gamma_inject, uint64_t seed, uint64_t call,
@@ -150,21 +148,13 @@ __global__ void cls_invgamma_kernel(const double* __restrict__ cl_hat, const int
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= nbins) return;
-    double beta = 0.0, ex = 0.0;
-    for (int l = bins[b]; l < bins[b + 1]; ++l) {
-        beta += (2.0 * l + 1.0) * (double)l * (double)(l + 1) * (cl_hat[l] / (4.0 * 3.14159265358979323846));
-        ex += (2.0 * l + 1.0) / 2.0;
-    }
-    double alpha = ex - 1.0;
+    double beta, alpha = ig_bin_stats(cl_hat, bins[b], bins[b + 1], beta);
     if (b == 0) alpha = 1.0;
     if (alpha_out) alpha_out[b] = alpha;
     if (beta_out) beta_out[b] = beta;
     double g;
     if (gamma_inject) g = gamma_inject[b];
-    // Philox stream ids carry the consumer in the top byte: the running counters of gs_randn / gs_randu stay below 2^56, "G"amma
-    // draws sit at 0x47 << 56, the inverse-Wishart draws of teb.cu at 0x57 << 56, the fused chain of gibbs_step.cu at 0x43 / 0x47 with
-    // its own seed word: no consumer can walk into another one's streams however long the chain runs
-    else g = alpha > 0.0 ? gamma_mt(alpha, Philox(seed), (0x47ull << 56) | (((call << 20) + (uint64_t)b) & 0x00ffffffffffffffull)) : 1.0;
+    else g = alpha > 0.0 ? gamma_mt(alpha, Philox(seed), RNG_GAMMA | (((call << 20) + (uint64_t)b) & RNG_ID_MASK)) : 1.0;
     out[b] = (b < 2) ? 0.0 : beta / g;
 }
 
@@ -197,7 +187,6 @@ __global__ void truncnorm_logpdf_kernel(const double* __restrict__ x, const doub
 }
 
 // ------------------------------------------------------------------ C ABI
-#define STREAM(s) ((cudaStream_t)(s))
 static inline int nblk(int64_t n) { return (int)std::min<int64_t>((n + SM_NT - 1) / SM_NT, SM_GRID); }
 
 extern "C" int gs_randn(double* out, int64_t n, uint64_t seed, uint64_t stream_id, void* stream)
@@ -332,8 +321,7 @@ __device__ __forceinline__ double binned_value(const double* cur, const double* 
                                                int l, bool use_prop, int b0, int b1)
 {
     if (l < bins[0] || l >= bins[nbins]) return 0.0;
-    int lo = 0, hi = nbins - 1;
-    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (bins[mid] <= l) lo = mid; else hi = mid - 1; }
+    const int lo = bin_of(bins, nbins, l);
     return (use_prop && lo >= b0 && lo < b1) ? prop[lo] : cur[lo];
 }
 
@@ -348,7 +336,7 @@ __global__ void mwg_filters_kernel(const double* cur_E, const double* cur_B, con
     if (l > L) return;
     double dE = binned_value(cur_E, prop_E, bins_E, nb_E, l, pol == 0, b0, b1);
     double dB = binned_value(cur_B, prop_B, bins_B, nb_B, l, pol == 1, b0, b1);
-    const double f = l ? 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1)) : 1.0;
+    const double f = l ? 2.0 * GS_PI / ((double)l * (double)(l + 1)) : 1.0;
     flE[l] = bl[l] * (l < l_cut ? 1.0 : sqrt(dE * f));
     flB[l] = bl[l] * (l < l_cut ? 1.0 : sqrt(dB * f));
 }
@@ -418,7 +406,7 @@ __global__ void mwg_dfl_kernel(const double* cur_E, const double* cur_B, const d
 {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l > L) return;
-    const double f = l ? 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1)) : 1.0;
+    const double f = l ? 2.0 * GS_PI / ((double)l * (double)(l + 1)) : 1.0;
     const double cE = binned_value(cur_E, prop_E, bins_E, nb_E, l, false, 0, 0);
     const double cB = binned_value(cur_B, prop_B, bins_B, nb_B, l, false, 0, 0);
     const double pE = binned_value(cur_E, prop_E, bins_E, nb_E, l, true, eb0, eb1);
@@ -706,9 +694,8 @@ __global__ void aux_s_kernel(const double* __restrict__ badj, const double* __re
     const double sq = sqrt(1.0 - alpha * alpha);
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const int l = l_of_real(i, L);
-        double c = dl[l];
-        if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
-        const double ic = c != 0.0 ? 1.0 / c : 0.0;
+        const double c = dl_to_cl(dl[l], l);
+        const double ic = safe_rcp(c);
         const double var = 1.0 / (mu_over_w * bl[l] * bl[l] + ic);
         const double mean = var * badj[i];
         double s = mean + sq * xi[i] * sqrt(var);
@@ -723,8 +710,7 @@ __global__ void pncp_factor_kernel(const double* __restrict__ dl, int L, int l_c
 {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l > L) return;
-    double c = dl[l];
-    if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
+    const double c = dl_to_cl(dl[l], l);
     double f = 1.0;
     if (l >= l_cut) f = mode ? sqrt(c) : (c != 0.0 ? sqrt(1.0 / c) : 0.0);
     out[l] = f;
@@ -763,9 +749,8 @@ __global__ void mala_sigma_kernel(const double* __restrict__ dl, const double* _
     const int64_t n = (int64_t)(L + 1) * (L + 1);
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const int l = l_of_real(i, L);
-        double c = dl[l];
-        if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
-        const double ic = c != 0.0 ? 1.0 / c : 0.0;
+        const double c = dl_to_cl(dl[l], l);
+        const double ic = safe_rcp(c);
         out[i] = 1.0 / (w * bl[l] * bl[l] + ic);
     }
 }
@@ -860,10 +845,9 @@ ula_nomask_kernel(const double* __restrict__ dl, const double* __restrict__ bl, 
     const int64_t n = (int64_t)(L + 1) * (L + 1);
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const int l = l_of_real(i, L);
-        double c = dl[l];
-        if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
+        const double c = dl_to_cl(dl[l], l);
         const double b = bl[l];
-        const double ic = c != 0.0 ? 1.0 / c : 0.0;
+        const double ic = safe_rcp(c);
         const double sigma = 1.0 / (w * b * b + ic);
         const double mean = sigma * (b * (w * d_alm[i]));
         const double so = s_old[i];

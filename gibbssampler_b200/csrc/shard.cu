@@ -22,6 +22,7 @@
 #include <algorithm>
 
 #include "gs_internal.h"
+#include "spectra.cuh"
 
 // ---------------------------------------------------------------- NCCL, resolved lazily
 namespace {
@@ -387,22 +388,11 @@ int gs_shard_allreduce(gs_plan* p, double* buf, int n, cudaStream_t st)
 }
 
 // ---------------------------------------------------------------- per-l helpers on the local real layout
-__device__ __forceinline__ double per_l_value_sh(const double* x, int l, int mode)
-{
-    double v = x[l];
-    if (mode == 0) return v;
-    if (l != 0) v = v * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
-    if (mode == 1) return v;
-    if (mode == 3) return sqrt(v);
-    const double inv = (v != 0.0) ? 1.0 / v : 0.0;
-    return mode == 2 ? inv : sqrt(inv);
-}
-
 __global__ void expand_per_l_shard_kernel(const double* __restrict__ x, const int* __restrict__ lof, double* __restrict__ out,
                                           int64_t n, int mode)
 {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        out[i] = per_l_value_sh(x, lof[i], mode);
+        out[i] = per_l_value(x, lof[i], mode);
 }
 
 int gs_plan_expand_per_l(gs_plan* p, const double* x, int mode, double* out, cudaStream_t st)

@@ -16,7 +16,7 @@
 #include <algorithm>
 
 #include "gs_internal.h"
-#include "rng.cuh"
+#include "spectra.cuh"
 
 #define SV_NT 256
 #define SV_GRID (148 * 4)
@@ -90,12 +90,9 @@ __global__ void precond_kernel(const double* __restrict__ dl, const double* __re
 {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l > L) return;
-    double c = dl[l];
-    if (l) c = c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
-    const double ic = c != 0.0 ? 1.0 / c : 0.0;
-    const double d = ic + bl[l] * bl[l] * ninv;
+    const double ic = safe_rcp(dl_to_cl(dl[l], l));
     invc_l[l] = ic;
-    pre_l[l] = d != 0.0 ? 1.0 / d : 0.0;
+    pre_l[l] = safe_rcp(ic + bl[l] * bl[l] * ninv);
 }
 
 __device__ __forceinline__ void pick(int64_t i, int64_t n, int& c, int64_t& j)
@@ -748,7 +745,7 @@ static int rhs_impl(gs_plan* p, int spin, const double* dl_E, const double* dl_B
     int rc;
     // fluctuation term 1: utils.adjoint_synthesis_hp (utils.py:79-111) = bl * (Npix/4pi) * map2alm(iter=3)
     if ((rc = map2alm(xi_Q, xi_U, sqrt_inv_noise, fluct_iter, 0, rhs_E, rhs_B))) return rc;
-    const double resc = (double)p->d.npix / (4.0 * 3.14159265358979323846);
+    const double resc = (double)p->d.npix / (4.0 * GS_PI);
     // fluctuation term 2 and data term; use r[] / p[] of the PCG workspace as scratch
     const double* dl[2] = {dl_E, dl_B};
     for (int c = 0; c < nc; ++c)
@@ -840,8 +837,6 @@ struct TebWs {
     PcgState* host_state;          // pinned, two slots
 };
 
-__device__ __forceinline__ double safe_rcp(double v) { return v != 0.0 ? 1.0 / v : 0.0; }
-
 // inverse of the symmetric 2x2 [[a, b], [b, d]] (safe_inv convention above)
 __device__ __forceinline__ void inv2x2(double a, double b, double d, double& i11, double& i12, double& i22)
 {
@@ -849,13 +844,6 @@ __device__ __forceinline__ void inv2x2(double a, double b, double d, double& i11
     const double det = a * d - b * b;
     const double id = safe_rcp(det);
     i11 = d * id; i12 = -b * id; i22 = a * id;
-}
-
-// C_l (l = 0: D_0 as it is, the convention of generate_var_cl / precond_kernel)
-__device__ __forceinline__ double dl_to_cl(const double* dl, int l)
-{
-    const double c = dl[l];
-    return l ? c * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1)) : c;
 }
 
 // One thread per l: C_l^-1 and the diag_cl preconditioner M_l = (C_l^-1 + diag(b_l^2 nT, b_l^2 nP, b_l^2 nP))^-1,
@@ -867,8 +855,8 @@ __global__ void teb_tables_kernel(const double* __restrict__ dlTT, const double*
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l > L) return;
     double i11, i12, i22;
-    inv2x2(dl_to_cl(dlTT, l), dl_to_cl(dlTE, l), dl_to_cl(dlEE, l), i11, i12, i22);
-    const double ibb = safe_rcp(dl_to_cl(dlBB, l));
+    inv2x2(dl_to_cl(dlTT[l], l), dl_to_cl(dlTE[l], l), dl_to_cl(dlEE[l], l), i11, i12, i22);
+    const double ibb = safe_rcp(dl_to_cl(dlBB[l], l));
     const double b2 = bl[l] * bl[l];
     double m11, m12, m22;
     inv2x2(i11 + b2 * nT, i12, i22 + b2 * nP, m11, m12, m22);
@@ -1049,7 +1037,7 @@ __global__ void teb_rhs_combine_kernel(const unsigned short* __restrict__ lof, c
 {
     for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
         const int l = lof[j];
-        const double a = dl_to_cl(dlTT, l), b = dl_to_cl(dlTE, l), d = dl_to_cl(dlEE, l), e = dl_to_cl(dlBB, l);
+        const double a = dl_to_cl(dlTT[l], l), b = dl_to_cl(dlTE[l], l), d = dl_to_cl(dlEE[l], l), e = dl_to_cl(dlBB[l], l);
         double fTT, fTE, fEE;
         if (b == 0.0) {
             fTT = a != 0.0 ? sqrt(1.0 / a) : 0.0;
@@ -1264,7 +1252,7 @@ extern "C" int gs_cr_rhs_teb(gs_plan* p, const double* dl_TT, const double* dl_T
         if ((rc = gs_map2alm_spin2(p, d_Q, d_U, inv_noise_P, 0, 1, bl, w->r[1], w->r[2], GS_ALM_REAL, stream))) return rc;
         for (int c = 0; c < 3; ++c) bd[c] = w->r[c];
     }
-    const double resc = (double)p->d.npix / (4.0 * 3.14159265358979323846);
+    const double resc = (double)p->d.npix / (4.0 * GS_PI);
     teb_rhs_combine_kernel<<<SV_GRID, SV_NT, 0, st>>>(w->lof, dl_TT, dl_TE, dl_EE, dl_BB, xi_T, xi_E, xi_B, bd[0], bd[1], bd[2], resc,
                                                       rhs_T, rhs_E, rhs_B, p->nreal_loc);
     GS_CHECK_LAUNCH();

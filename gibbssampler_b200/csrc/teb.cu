@@ -12,10 +12,10 @@
 
 #include "gs_internal.h"
 #include "rng.cuh"
+#include "spectra.cuh"
 
 #define TB_NT 256
 static inline int tb_blocks(int64_t n) { return (int)std::max<int64_t>(1, std::min<int64_t>((n + TB_NT - 1) / TB_NT, 148 * 16)); }
-#define STREAM(s) ((cudaStream_t)(s))
 
 // ---- variance_expension.pyx:36-61: (L+1,3,3) D_l -> ((L+1)^2,3,3) C_l over the real alm layout.
 // The reference indexes cls_[idx] instead of cls_[l] at :51 and raises IndexError (SURVEY.md 8c); the
@@ -27,9 +27,7 @@ __global__ void expand_var_cl_3x3_kernel(const double* __restrict__ dls, int L, 
         const int64_t i = t / 9;
         const int e = (int)(t - i * 9);
         const int l = l_of_real(i, L);
-        double v = dls[l * 9 + e];
-        if (l) v = v * 2.0 * 3.14159265358979323846 / ((double)l * (double)(l + 1));
-        out[t] = v;
+        out[t] = dl_to_cl(dls[l * 9 + e], l);
     }
 }
 
@@ -94,13 +92,7 @@ __global__ void alm2cl_cross_kernel(const double* __restrict__ x, const double* 
 {
     const int l = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (l > L) return;
-    double s = 0.0;
-    for (int m = lane; m <= l; m += 32) {
-        const int64_t id = (int64_t)m * (2 * L + 1 - m) / 2 + l;
-        if (m == 0) s += x[l] * y[l];
-        else { const int64_t o = 2 * id - (L + 1); s += x[o] * y[o] + x[o + 1] * y[o + 1]; }
-    }
-    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    const double s = warp_sum(alm2cl_cross_real_lane(x, y, l, L, lane));
     if (lane == 0) cl[l] = s / (2.0 * l + 1.0);
 }
 
@@ -109,7 +101,7 @@ __global__ void alm2cl_cross_kernel(const double* __restrict__ x, const double* 
 //   Psi^-1 = G G^T,  A = [[sqrt(chi2_nu), 0], [N(0,1), sqrt(chi2_{nu-1})]],  X^-1 = (G A)(G A)^T.
 // Draw k (a multipole or a bin) takes row k of inject ((chi2_nu, chi2_{nu-1}, normal) supplied by the caller, parity with a numpy
 // stream) or, without inject, Philox / Marsaglia-Tsang on the streams base, base + 1, base + 2 with
-// base = (0x57 << 56) | ((call << 22) + 4 k): the "W"ishart domain (see sampler.cu).
+// base = RNG_WISHART | ((call << 22) + 4 k) (rng.cuh).
 __device__ __forceinline__ void invwishart_2x2_draw(double p00, double p01, double p11, double nu, const double* __restrict__ inject, int k,
                                                     uint64_t seed, uint64_t call, double& x00, double& x01, double& x11)
 {
@@ -120,7 +112,7 @@ __device__ __forceinline__ void invwishart_2x2_draw(double p00, double p01, doub
     if (inject) { c1 = inject[3 * k]; c2 = inject[3 * k + 1]; z = inject[3 * k + 2]; }
     else {
         const Philox ph(seed);
-        const uint64_t base = (0x57ull << 56) | (((call << 22) + 4ull * (uint64_t)k) & 0x00ffffffffffffffull);
+        const uint64_t base = RNG_WISHART | (((call << 22) + 4ull * (uint64_t)k) & RNG_ID_MASK);
         c1 = 2.0 * gamma_mt(0.5 * nu, ph, base);
         c2 = 2.0 * gamma_mt(0.5 * (nu - 1.0), ph, base + 1);
         double z2;
@@ -171,14 +163,9 @@ __global__ void invwishart_binned_kernel(const double* __restrict__ tt, const do
         o_tt[b] = v; o_te[b] = v; o_ee[b] = v;
         return;
     }
-    double p00 = 0.0, p01 = 0.0, p11 = 0.0, nu = -3.0;
-    for (int l = l0; l < l1; ++l) {
-        const double f = 2.0 * l + 1.0, w = f * ((double)l * (double)(l + 1) / (2.0 * 3.14159265358979323846));
-        p00 += w * tt[l]; p01 += w * te[l]; p11 += w * ee[l];
-        nu += f;
-    }
+    double psi[3], nu = iw_bin_stats(tt, te, ee, l0, l1, psi);
     double x00, x01, x11;
-    invwishart_2x2_draw(p00, p01, p11, nu, inject, b, seed, call, x00, x01, x11);
+    invwishart_2x2_draw(psi[0], psi[1], psi[2], nu, inject, b, seed, call, x00, x01, x11);
     o_tt[b] = x00; o_te[b] = x01; o_ee[b] = x11;
 }
 

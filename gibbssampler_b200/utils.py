@@ -48,6 +48,11 @@ def generate_var_cl(cls_):
     return expand_per_l(cls_, 1)
 
 
+def dls_to_cls_array(lmax):
+    """Per-l factor that turns D_l into C_l: 2 pi / (l (l+1)), and 0 at l = 0."""
+    return np.array([2 * np.pi / (l * (l + 1)) if l != 0 else 0 for l in range(lmax + 1)])
+
+
 def unfold_bins(binned_cls_, bins):
     """utils.unfold_bins (utils.py:150-162): np.repeat(binned, diff(bins))."""
     b = f64(binned_cls_)
