@@ -8,7 +8,10 @@ it) and p(D | sigma) the C_l conditional the chain draws from, in D units: the b
 TT, EE and BB, and the (TT, TE; TE, EE) inverse-Wishart of gs_cls_invwishart_binned plus the inverse-gamma BB of the joint
 sampler.  Every conditional corresponds to a flat prior on D_b, so the estimate is the normalised posterior density and
 equals the likelihood up to a constant.  The sum over samples runs on the device as one fused FP64 GEMM + log-mean-exp
-(gs_br_logmeanexp, include/gibbs_b200.h): the N x M matrix of log-densities is never formed."""
+(gs_br_logmeanexp, include/gibbs_b200.h): the N x M matrix of log-densities is never formed.
+
+GaussianizedBlackwellRao (Rudjord et al. 2009) joins the one-dimensional BR marginals, which converge where the multivariate sum
+does not, by a Gaussian copula fitted to the chain; its mixture-CDF transform is gs_gbr_transform."""
 import numpy as np
 import torch
 
@@ -46,6 +49,13 @@ class BlackwellRao:
     Inputs may be numpy arrays or CUDA tensors; results come back as numpy arrays or CUDA tensors like the input of each call."""
 
     def __init__(self, sigma, bins, *, burn_in=0):
+        chains, burn_in = self._validate(sigma, bins, burn_in)
+        self.sigma = {k: torch.cat([f64(c[k])[burn_in:] for c in chains]).contiguous() for k in self.keys}
+        self._feat = {}
+        self._features(None)     # the full set of bins, built once
+
+    def _validate(self, sigma, bins, burn_in):
+        """host checks of sigma, bins and burn_in; sets keys, edges, groups, nbins, ncl, lmax and n -> (chains, burn_in)"""
         chains = [sigma] if isinstance(sigma, dict) else list(sigma)
         if not chains or not all(isinstance(c, dict) and c for c in chains):
             raise ValueError("sigma must be a non-empty dict of spectra or a list of such dicts")
@@ -87,10 +97,8 @@ class BlackwellRao:
             self.edges = {k: _edges(bins[k] if isinstance(bins, dict) else bins, ncl, k) for k in self.keys}
             self.groups = [(GS_BR_IG, (k,)) for k in self.keys]
         self.nbins = {k: len(e) - 1 for k, e in self.edges.items()}
-        self.sigma = {k: torch.cat([f64(c[k])[burn_in:] for c in chains]).contiguous() for k in self.keys}
-        self.n = int(self.sigma[self.keys[0]].shape[0])
-        self._feat = {}
-        self._features(None)     # the full set of bins, built once
+        self.n = sum(int(c[self.keys[0]].shape[0]) - burn_in for c in chains)
+        return chains, burn_in
 
     @classmethod
     def from_sampler(cls, gibbs, burn_in=0):
@@ -155,11 +163,12 @@ class BlackwellRao:
         return f
 
     # ------------------------------------------------------------------ estimator
-    def _dls(self, dls):
-        if set(dls) != set(self.keys):
-            raise ValueError("dls must hold the keys %s, got %s" % (sorted(self.keys), sorted(dls)))
+    def _dls(self, dls, keys=None):
+        keys = self.keys if keys is None else keys
+        if set(dls) != set(keys):
+            raise ValueError("dls must hold the keys %s, got %s" % (sorted(keys), sorted(dls)))
         out, m, one = {}, None, None
-        for k in self.keys:
+        for k in keys:
             d = f64(dls[k])
             if d.dim() not in (1, 2) or d.shape[-1] != self.nbins[k]:
                 raise ValueError("dls[%r] must have shape (%d,) or (M, %d), got %s" % (k, self.nbins[k], self.nbins[k], tuple(d.shape)))
@@ -210,6 +219,51 @@ class BlackwellRao:
         """doubles of scratch gs_br_logmeanexp needs (the library owns the split of the sample axis)"""
         return int(_lib.lib().gs_br_logmeanexp_scratch(self.n, M))
 
+    def _group_of(self, key):
+        """-> (group index, kind, comp) of a TT, EE or BB key; TE has no marginal"""
+        if key not in self.keys:
+            raise ValueError("no spectrum %r (have %s)" % (key, sorted(self.keys)))
+        if key == "TE":
+            raise ValueError("the TE marginal is not available (only TT, EE and BB)")
+        gi = next(i for i, (_, keys) in enumerate(self.groups) if key in keys)
+        kind, keys = self.groups[gi]
+        return gi, kind, 0 if kind == GS_BR_IG else keys.index(key)
+
+    def _transform(self, key, d, lrange=None):
+        """gs_gbr_transform of the (M, nbins of the selection) D of one key on the bins lrange selects -> (x, logm), CUDA tensors"""
+        gi, kind, comp = self._group_of(key)
+        f = self._features(lrange)
+        b0, b1 = f["sel"][gi]
+        M, nb = d.shape[0], b1 - b0
+        x = torch.empty((M, nb), dtype=torch.float64, device=d.device)
+        logm = torch.empty_like(x)
+        L = _lib.lib()
+        scratch = torch.empty(int(L.gs_gbr_transform_scratch(self.n, M, nb)), dtype=torch.float64, device=d.device)
+        check(L.gs_gbr_transform(kind, ptr(f["S"][sum(f["rows"][:gi])]), self.n, self.ncl, ptr(f["edges"][gi]), nb, comp,
+                                 ptr(d.contiguous()), M, ptr(x), ptr(logm), ptr(scratch), stream()))
+        return x, logm
+
+    def cdf(self, key, grid):
+        """Per-bin BR marginal CDF P(D_b <= g | d) = (1/N) sum_i Q(alpha, beta_i / g) on a grid laid out as for marginal(): grid (G,)
+        or (nbins, G) -> (nbins, G), rows of the bins 0 and 1 NaN.  Computed by gs_gbr_transform as Phi(x), so both tails keep
+        their relative accuracy."""
+        self._group_of(key)
+        host = _is_host(grid)
+        g = f64(grid)
+        nb = self.nbins[key]
+        if g.dim() == 1:
+            d = g[:, None].expand(g.shape[0], nb - 2)
+        elif g.dim() == 2 and g.shape[0] == nb:
+            d = g[2:].T
+        else:
+            raise ValueError("grid must have shape (G,) or (%d, G), got %s" % (nb, tuple(g.shape)))
+        if d.shape[0] < 1:
+            raise ValueError("grid is empty")
+        x, _ = self._transform(key, d.contiguous())
+        out = torch.full((nb, d.shape[0]), float("nan"), dtype=torch.float64, device=g.device)
+        out[2:] = torch.special.ndtr(x).T
+        return out.cpu().numpy() if host else out
+
     def marginal(self, key, grid):
         """Per-bin BR marginal log p(D_b = g | d) on a grid: grid (G,) for every bin or (nbins, G) per bin; -> (nbins, G), rows of
         the bins 0 and 1 NaN.  IG spectra use their inverse-gamma; TT and EE of the joint block the marginal of a diagonal entry of
@@ -238,4 +292,147 @@ class BlackwellRao:
         out = torch.full((nb, G), float("nan"), dtype=torch.float64, device=g.device)
         check(_lib.lib().gs_br_marginal(kind, ptr(f["S"][r0]), self.n, self.ncl, ptr(f["edges"][gi]), nb - 2, comp, ptr(g), ld, G,
                                         ptr(out[2]), stream()))
+        return out.cpu().numpy() if host else out
+
+
+def _history_rows(h, keys, chain):
+    """the (n_iter + 1, nbins) D history of each key of one chain: a dict (polarised and joint samplers) or an array (TT)"""
+    if isinstance(h, tuple):                  # CenteredGibbs.run() returns (history, ...)
+        h = h[0]
+    if not isinstance(h, dict):
+        if keys != ("TT",):
+            raise ValueError("dls of chain %d must be a dict of D histories with the keys %s" % (chain, sorted(keys)))
+        h = {"TT": h}
+    missing = [k for k in keys if k not in h]
+    if missing:
+        raise ValueError("dls of chain %d has no history for %s" % (chain, missing))
+    return {k: h[k] for k in keys}
+
+
+class GaussianizedBlackwellRao:
+    """GaussianizedBlackwellRao(sigma, dls, bins, *, burn_in=0): the Gaussianized Blackwell-Rao likelihood of Rudjord et al. (2009).
+
+    Each bin b is mapped through its own BR marginal, x_b = Phi^-1(F_b(D_b)) with F_b(D) = (1/N) sum_i F_IG(D; alpha_b, beta_b^i), and
+    the bins are joined by a Gaussian copula fitted to the chain's own D samples:
+        log L(D) = log N(x; mu, Sigma) + sum_b [log p_b(D_b) - log phi(x_b)],
+    p_b the BR marginal density (so dx_b / dD_b = p_b / phi(x_b)).  Unlike BlackwellRao.logpdf it needs only the one-dimensional
+    marginals to converge, so it stays usable when the multivariate BR sum rests on a handful of samples (many bins).
+
+    sigma, bins, burn_in: as BlackwellRao (its validation, bins and sample features are used as they are).  dls: the D histories
+    run() returned, in the same layout as sigma (a dict, a list of dicts, or a TT array per chain); a history has n_iter + 1 rows.
+    Row alignment: sigma row i is the sky that D row i + 1 was drawn from, so after burn_in, mu and Sigma come from the D rows
+    burn_in + 1 ... n_iter of every chain.  Spectra: TT, EE, BB of CenteredGibbs; TT, EE, BB of JointGibbs, TT and EE through the
+    inverse-Wishart diagonal marginal, so TE is marginalised (a "TE" model entry raises ValueError).  The transform runs on the
+    device (gs_gbr_transform); mu and Sigma are FP64, and the Cholesky factor of every lrange selection's sub-matrix is kept."""
+
+    def __init__(self, sigma, dls, bins, *, burn_in=0):
+        # every check runs on the host before anything reaches the device
+        br = self.br = BlackwellRao.__new__(BlackwellRao)
+        chains, burn_in = br._validate(sigma, bins, burn_in)
+        self.keys = ("TT", "EE", "BB") if br.joint else br.keys
+        hists = [dls] if isinstance(dls, (dict, tuple, np.ndarray, torch.Tensor)) else list(dls)
+        if len(hists) != len(chains):
+            raise ValueError("dls holds %d chains, sigma %d" % (len(hists), len(chains)))
+        hists = [_history_rows(h, self.keys, i) for i, h in enumerate(hists)]
+        for i, (s, h) in enumerate(zip(chains, hists)):
+            n_iter = int(s[br.keys[0]].shape[0])
+            for k in self.keys:
+                shape = tuple(np.shape(h[k]))
+                if shape != (n_iter + 1, br.nbins[k]):
+                    raise ValueError("dls[%r] of chain %d has shape %s, expected (%d, %d): the D history of a chain of %d iterations"
+                                     % (k, i, shape, n_iter + 1, br.nbins[k], n_iter))
+        # the Gaussianized chain, bins 2 .. nbins - 1 of every key in key order
+        self._cols, c0 = {}, 0
+        for k in self.keys:
+            self._cols[k] = c0
+            c0 += br.nbins[k] - 2
+        B, n = c0, br.n
+        if n < B + 1:
+            raise ValueError("%d samples after burn_in for %d bins: the copula covariance needs at least %d" % (n, B, B + 1))
+        br.sigma = {k: torch.cat([f64(c[k])[burn_in:] for c in chains]).contiguous() for k in br.keys}
+        br._feat = {}
+        X = torch.empty((n, B), dtype=torch.float64, device=br.sigma[br.keys[0]].device)
+        for k in self.keys:
+            d = torch.cat([f64(h[k])[burn_in + 1:] for h in hists])[:, 2:].contiguous()
+            X[:, self._cols[k]:self._cols[k] + d.shape[1]] = self.br._transform(k, d)[0]
+        bad = int((~torch.isfinite(X)).sum())
+        if bad:
+            raise ValueError("%d of the chain's %d Gaussianized values are not finite" % (bad, X.numel()))
+        self.mean = X.mean(0)
+        Xc = X - self.mean
+        self.cov = (Xc.T @ Xc) / (n - 1)
+        self.nbins = B
+        self._chol = {}
+        self._factor(None)
+
+    @classmethod
+    def from_sampler(cls, gibbs, history, burn_in=0):
+        """The likelihood of a chain run with keep_sigma=True (CenteredGibbs or JointGibbs); history = what its run() returned."""
+        sig = getattr(gibbs, "sigma_history", None)
+        if sig is None:
+            raise ValueError("the sampler has no sigma_history: construct it with keep_sigma=True and call run()")
+        bins = gibbs.bins
+        if isinstance(bins, dict) and "TE" not in sig:
+            bins = {k: bins[k] for k in sig}
+        return cls(sig, history, bins, burn_in=burn_in)
+
+    def _factor(self, lrange):
+        """-> (selection, column index, Cholesky factor of the sub-matrix of Sigma) of the bins lrange selects"""
+        sel = self.br._selection(lrange)
+        if sel in self._chol:
+            return self._chol[sel]
+        idx = []
+        for k in self.keys:
+            gi = self.br._group_of(k)[0]
+            b0, b1 = sel[gi]
+            idx += [self._cols[k] + b - 2 for b in range(b0, b1)]
+        idx = torch.as_tensor(idx, dtype=torch.long, device=self.cov.device)
+        L, info = torch.linalg.cholesky_ex(self.cov[idx][:, idx])
+        if int(info):
+            raise ValueError("the copula covariance of %d bins is not positive definite (leading minor %d)" % (len(idx), int(info)))
+        self._chol[sel] = (sel, idx, L)
+        return self._chol[sel]
+
+    def gaussianize(self, key, dls):
+        """x = Phi^-1(F_b(D_b)) of one spectrum: dls (nbins,) or (M, nbins) -> the same shape, columns of the bins 0 and 1 NaN"""
+        if key not in self.keys:
+            raise ValueError("no spectrum %r (have %s)" % (key, sorted(self.keys)))
+        host = _is_host(dls)
+        d = f64(dls)
+        nb = self.br.nbins[key]
+        if d.dim() not in (1, 2) or d.shape[-1] != nb or d.numel() == 0:
+            raise ValueError("dls must have shape (%d,) or (M, %d), got %s" % (nb, nb, tuple(d.shape)))
+        d2 = d.reshape(-1, nb)
+        out = torch.full(d2.shape, float("nan"), dtype=torch.float64, device=d.device)
+        out[:, 2:] = self.br._transform(key, d2[:, 2:].contiguous())[0]
+        out = out.reshape(d.shape)
+        return out.cpu().numpy() if host else out
+
+    def logpdf(self, dls, *, lrange=None):
+        """Gaussianized BR log-likelihood of each model, in the layout of BlackwellRao.logpdf (keys TT / EE / BB, (nbins,) or
+        (M, nbins), bins 0 and 1 ignored, lrange selecting whole bins).  A model with some D_b <= 0, or one so far out that F_b or
+        1 - F_b is 0 in FP64, gets -inf; broken input (NaN) gives NaN."""
+        if "TE" in dls and self.br.joint:
+            raise ValueError("TE is marginalised in the Gaussianized BR likelihood: pass TT, EE and BB only")
+        self.br._selection(lrange)          # a cut bin raises before any device work
+        host = _is_host(next(iter(dls.values())))
+        d, M, one = self.br._dls(dls, self.keys)
+        sel, idx, L = self._factor(lrange)
+        xs, lms = [], []
+        for k in self.keys:
+            b0, b1 = sel[self.br._group_of(k)[0]]
+            if b1 == b0:
+                continue
+            x, lm = self.br._transform(k, d[k][:, b0:b1], lrange)
+            xs.append(x)
+            lms.append(lm)
+        x, lm = torch.cat(xs, 1), torch.cat(lms, 1)
+        z = torch.linalg.solve_triangular(L, (x - self.mean[idx]).T, upper=False)
+        out = -0.5 * (z * z).sum(0) - torch.log(torch.diagonal(L)).sum() + (lm + 0.5 * x * x).sum(1)
+        finite = torch.isfinite(x).all(1) & torch.isfinite(lm).all(1)
+        nan = torch.isnan(x).any(1) | torch.isnan(lm).any(1)
+        out = torch.where(finite, out, torch.full_like(out, -float("inf")))
+        out = torch.where(nan, torch.full_like(out, float("nan")), out)
+        if one:
+            out = out[0]
         return out.cpu().numpy() if host else out

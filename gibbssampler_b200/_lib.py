@@ -100,6 +100,8 @@ SIGNATURES = {
     "gs_br_logmeanexp_scratch": (_i64, [_i64, _i64]),
     "gs_br_logmeanexp": (_i, [_vp, _vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "gs_br_marginal": (_i, [_i, _vp, _i64, _i, _vp, _i, _i, _vp, _i64, _i, _vp, _vp]),
+    "gs_gbr_transform_scratch": (_i64, [_i64, _i64, _i]),
+    "gs_gbr_transform": (_i, [_i, _vp, _i64, _i, _vp, _i, _i, _vp, _i64, _vp, _vp, _vp, _vp]),
     "gs_nccl_unique_id": (_i, [C.c_char_p]),
     "gs_plan_create_sharded": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _i, C.c_char_p]),
     "gs_local_group_create": (_i, [C.POINTER(_vp), _i]),

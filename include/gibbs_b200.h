@@ -445,6 +445,19 @@ int gs_br_logmeanexp(const double* S, const double* c, int64_t nsamp, const doub
  * bad kind / comp, nsamp or ngrid < 1, grid_ld < 0 or nbins outside [1, min(ncl, 65535)]. */
 int gs_br_marginal(int kind, const double* S, int64_t nsamp, int ncl, const int* bins, int nbins, int comp, const double* grid,
                    int64_t grid_ld, int ngrid, double* out, void* stream);
+/* Gaussianized BR transform (Rudjord et al. 2009) of one group, with the bins, kind, comp and S of gs_br_marginal: for the BR
+ * marginal of bin b, the mixture (1/N) sum_i IG(alpha_b, beta_b^i), and dl (nmod, nbins) row-major binned D,
+ *   x_out[k][b] = Phi^-1(F_b(D_kb)),  F_b(D) = (1/N) sum_i Q(alpha_b, beta_b^i / D),   logm_out[k][b] = log p_b(D_kb)
+ * (Q, P: the regularized upper and lower incomplete gammas; logm is the quantity gs_br_marginal returns).  Sum Q and sum P are
+ * kept apart, each sample computing its smaller tail directly (series, continued fraction or Temme's uniform expansion), and
+ * x = Phi^-1(F) for F <= 1/2, else -Phi^-1(1 - F).  Broken edges: NaN; D <= 0 (or NaN), or F or 1 - F = 0 in FP64: x = -inf / +inf
+ * and logm = -inf.  The sample axis is split over P CTA columns as a function of (nsamp, nmod, nbins) only and the partials merged
+ * in a fixed order, so repeated calls are bit-identical; scratch: 4 * nmod * nbins * P doubles, as gs_gbr_transform_scratch
+ * returns (-1 for nsamp or nmod < 1 or nbins outside [1, 65535]).  GS_E_BADARG for null pointers, a bad kind / comp, nsamp or
+ * nmod < 1 or nbins outside [1, min(ncl, 65535)]. */
+int64_t gs_gbr_transform_scratch(int64_t nsamp, int64_t nmod, int nbins);
+int gs_gbr_transform(int kind, const double* S, int64_t nsamp, int ncl, const int* bins, int nbins, int comp, const double* dl,
+                     int64_t nmod, double* x_out, double* logm_out, double* scratch, void* stream);
 
 /* ---- whole chain in one call (SURVEY.md 8b gs_gibbs_step_centered; BASELINE config #1) -----------------------------------
  * GibbsSampler.run_polarization (GibbsSampler.py:118-180) for the full-sky isotropic-noise centred sampler: every iteration is
