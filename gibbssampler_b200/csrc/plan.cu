@@ -221,7 +221,10 @@ static int plan_create_impl(gs_plan** out, int nside, int lmax, int device, int 
 {
     if (!out) { gs_set_error("gs_plan_create: null output"); return GS_E_BADARG; }
     *out = nullptr;
-    GS_REQUIRE(nside >= 1 && nside <= 8192, "nside out of range [1, 8192]");
+    // the ring stage takes a ring whole or as four sub-transforms of n/4 points (ringfft.cu, gs_ring_setup).  A belt ring's
+    // quarter has nside points; unless that is a power of two it runs as a Bluestein transform of next_pow2(2 nside - 1)
+    // points, and one CTA holds at most 4096: nside <= 2048.  Refused here, before any table is built on the device.
+    GS_REQUIRE(nside >= 1 && nside <= GS_NSIDE_MAX, "nside out of range [1, 2048]: rings longer than 8192 pixels need a deeper ring split");
     GS_REQUIRE(lmax >= 2 && lmax <= 4 * nside, "lmax must satisfy 2 <= lmax <= 4 nside");
     GS_REQUIRE(world >= 1 && rank >= 0 && rank < world, "need 0 <= rank < world");
     GS_REQUIRE(world <= 2 * nside && world <= (lmax + 2) / 2, "more ranks than ring pairs or m pairs");

@@ -1048,7 +1048,13 @@ int gs_ring_setup(gs_plan* p)
         const int v = atoi(e);
         if (v >= 4 && v < Mcap && (v & (v - 1)) == 0) Mcap = v;
     }
-    auto is_split = [&](int ring) { return ring_M(rn[ring]) > Mcap; };
+    // A Bluestein sub-transform of the split path takes its chirp-spectrum product inside the last radix-16 pass of
+    // fft_dif<true>, so it needs M >= 16.  The quarter of a 12-pixel ring would have M = 8 (only reachable with
+    // GS_RING_MCAP <= 16): such a ring stays on the direct path.
+    auto is_split = [&](int ring) {
+        const int q = rn[ring] / 4;
+        return ring_M(rn[ring]) > Mcap && ((q & (q - 1)) == 0 || ring_M(q) >= 16);
+    };
     std::map<int, int> n2bs;
     std::vector<BluesteinDesc> descs;
     int64_t off = 0;
@@ -1065,7 +1071,8 @@ int gs_ring_setup(gs_plan* p)
         if (!is_split(r)) need_len(rn[r], maxMd);
         else {
             if (ring_M(rn[r] / 4) > Mcap) {
-                gs_set_error("ring FFT: nside %d / lmax %d needs a deeper ring split than this build provides", nside, L);
+                gs_set_error("ring FFT: nside %d needs a deeper ring split than this build provides (nside <= %d)", nside,
+                             Mcap / 2);
                 return GS_E_BADARG;
             }
             need_len(rn[r] / 4, maxMs);

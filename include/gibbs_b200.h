@@ -43,6 +43,10 @@ extern "C" {
 #define GS_ALM_COMPLEX 0
 #define GS_ALM_REAL 1
 
+/* Largest NSIDE a plan accepts: the ring stage transforms a ring in one CTA or as four sub-transforms, and rings longer
+ * than 4 * 2048 pixels would need a deeper split. */
+#define GS_NSIDE_MAX 2048
+
 typedef struct gs_plan gs_plan;
 
 /* ---- library / plan ------------------------------------------------------------------ */
@@ -51,7 +55,8 @@ int gs_version(void);
 
 /* Builds ring geometry, FP64 recurrence tables and ring-FFT tables for (nside, lmax) on CUDA
  * device `device` (-1 = current).  Replaces the implicit healpy/libsharp geometry + plan that
- * hp.alm2map / hp.map2alm rebuild on every call.  Synchronous. */
+ * hp.alm2map / hp.map2alm rebuild on every call.  Accepts 1 <= nside <= GS_NSIDE_MAX (2048) and
+ * 2 <= lmax <= 4 nside; anything else returns GS_E_BADARG before any device work.  Synchronous. */
 int gs_plan_create(gs_plan** plan, int nside, int lmax, int device);
 int gs_plan_destroy(gs_plan* plan);
 /* Chain batches (SURVEY.md 8b: gs_plan_create(nside, lmax, n_chain, ...); BASELINE config #5 "batched over chains"): sizes the
